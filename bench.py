@@ -22,6 +22,10 @@ on the launching stream, L2 flushed between steps, max over ranks.  `e2e`: the s
 pinned host buffers, host<->device copies inside the timed region.  `parity`: max-abs / RMS of the GPU poses,
 rotation matrices and FK joints against the CPU arm on the clips that arm computes (fails loudly above tolerance).
 
+`--dump-outputs DIR` writes, after the timed steps, what the timed path computed in its last step as DIR/<name>.npy
+(float32; rank 0's clips; a fixed, seeded sample of the clips when the arrays exceed 64 MB).  The inputs depend only on
+the arguments, so two builds can be compared output for output.
+
 `--impl reference` (and the `cpu_baseline` leg) time the reference's OWN PyTorch modules on the host cores when
 oracle/_ref (snapshot made by oracle/build_ref.py) or /root/reference is present (kind "reference"), else the
 oracle restatement (kind "port"); FK has no in-repo reference code (third-party smplx) and always uses the oracle's
@@ -70,6 +74,26 @@ def _emit(line):
     out = _JSON_OUT or sys.stdout
     out.write(json.dumps(line) + "\n")
     out.flush()
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes each array (clips along axis 0) as out_dir/<name>.npy in float32.  Above DUMP_LIMIT_BYTES in all, the
+    same seeded sample of clips is taken from every array."""
+    import numpy as np
+    arrays = {k: np.ascontiguousarray(np.asarray(v, dtype=np.float32)) for k, v in arrays.items()}
+    n = next(iter(arrays.values())).shape[0]
+    assert all(a.shape[0] == n for a in arrays.values()), {k: a.shape for k, a in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        keep = max(1, n * DUMP_LIMIT_BYTES // total)
+        idx = np.sort(np.random.RandomState(0).choice(n, keep, replace=False))
+        arrays = {k: a[idx] for k, a in arrays.items()}
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a)
 
 
 def _peaks():
@@ -249,18 +273,21 @@ def run_reference(args):
 
     def one_pass():
         if batch1:                                                # DataLoader(batch_size=1) loop of inference.py:43-52
-            for i in range(x.shape[0]):
-                arm.step(x[i:i + 1])
-        else:
-            arm.step(x)
+            return [arm.step(x[i:i + 1]) for i in range(x.shape[0])]
+        return [arm.step(x)]
 
     for _ in range(warm):
         one_pass()
     ts = []
     for _ in range(steps):
         t0 = time.perf_counter()
-        one_pass()
+        outs = one_pass()
         ts.append(time.perf_counter() - t0)
+    if args.dump_outputs:
+        import numpy as np
+        poses = np.concatenate([o[0] for o in outs])
+        joints = np.concatenate([o[2] for o in outs]).reshape(poses.shape[0], poses.shape[1], J, 3)
+        dump_outputs(args.dump_outputs, {"poses": poses, "joints": joints})
     sec = sum(ts) / len(ts)
     fps = x.shape[0] * x.shape[1] / sec
     threads = torch.get_num_threads()
@@ -418,6 +445,7 @@ def run_ours(args):
         # run, so that every N of a scaling series carries it next to the configs[2] headline
         a3 = copy.copy(args)
         a3.config, a3.steps, a3.warmup, a3.no_cpu, a3.no_hbm, a3.batch, a3.dtype = 3, min(args.steps, 5), 3, True, True, 0, None
+        a3.dump_outputs = None                                   # --dump-outputs writes the headline configs[2] results
         l3 = measure(a3, dev, world, rank, local)
         if rank == 0:
             line["configs3"] = {k: l3[k] for k in ("value", "unit", "ms_per_step", "scaling", "e2e", "clocks", "steps", "warmup") if k in l3}
@@ -563,6 +591,9 @@ def measure(args, dev, world, rank, local):
     ms_steps = sorted(a.elapsed_time(b) for a, b in ev)
     ms = (sum(ms_steps) + max(0.0, ev[-1][1].elapsed_time(t_end))) / args.steps
     g_ms = sum(a.elapsed_time(b) for a, b in gather_ms) / len(gather_ms) if gather_ms else 0.0
+    # the end-to-end loop below computes into the same buffers: keep the last timed step's results as they are now
+    last_step = {"poses": poses_local.cpu(), "joints": joints_local.view(n_local, T_out, J, 3).cpu()} \
+        if (rank == 0 and args.dump_outputs) else None
 
     # ---- end to end through the public API: pinned host input -> H2D -> forward + FK -> (gather) -> D2H of the results
     # The copies are pipelined the way a serving loop would: the H2D copy of micro-batch k+1 runs on a copy stream
@@ -719,6 +750,8 @@ def measure(args, dev, world, rank, local):
             line["roofline_hbm"] = _hbm_rooflines(dev, peaks, args.hbm_frames)
         if args.config == 1:
             line["rot6d132_head"] = _config1_rot6d(dev, IterativePoseRegressor, default_hparams, synth, A, x_dev, args)
+        if last_step is not None:
+            dump_outputs(args.dump_outputs, {k: v.numpy() for k, v in last_step.items()})
         return line
     return None
 
@@ -786,10 +819,12 @@ def run_ours_windows(args, dev, dtype):
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for _ in range(args.steps):
-        bulk_fn()
+        y_bulk = bulk_fn()
     e1.record()
     e1.synchronize()
     ms_bulk = e0.elapsed_time(e1) / args.steps
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"poses": y_bulk.cpu().numpy()})
     # batch 1 through the public API: device latency (events) and host-observed latency incl. D2H, (a) on the
     # throughput plan with CUDA-graph replay (19-25 launches), (b) on the latency plan (one persistent cooperative
     # kernel, fp32) -- the one a streaming caller selects with model.low_latency = True
@@ -879,7 +914,11 @@ def main():
     ap.add_argument("--hbm-frames", type=int, default=1 << 23)
     ap.add_argument("--port", action="store_true", help="CPU arm: use the oracle restatement even if the reference modules are present")
     ap.add_argument("--no-graph", action="store_true", help="launch kernels one by one instead of replaying a CUDA graph")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's results (poses, joints) as DIR/<name>.npy, float32, 64 MB at most")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     world = int(os.environ.get("WORLD_SIZE", "1"))
     args.with_c3 = args.config is None and not args.no_c3 and not args.batch and args.impl == "ours"
     if args.config is None:

@@ -32,6 +32,20 @@ def test_reference_arm_line(extra, config):
         assert d["latency_us"]["per_window_mean"] > 0
 
 
+def test_reference_arm_dumps_its_last_step(tmp_path, golden):
+    """--dump-outputs: float32 .npy files of the last timed step, identical from run to run (configs[0]: the dance
+    windows, whose poses the reference's own modules produced in tests/golden/dance.npz)."""
+    import numpy as np
+    dumps = []
+    for run in ("a", "b"):
+        _run("--config", "0", "--dump-outputs", str(tmp_path / run))
+        dumps.append({n: np.load(tmp_path / run / f"{n}.npy") for n in ("poses", "joints")})
+    a, b = dumps
+    assert a["poses"].dtype == np.float32 and a["poses"].shape == (231, 1, 66) and a["joints"].shape == (231, 1, 22, 3)
+    assert all(np.array_equal(a[n], b[n]) for n in a)
+    np.testing.assert_allclose(a["poses"], golden("dance.npz")["poses"], rtol=0, atol=2e-5)
+
+
 def test_non_zero_ranks_of_the_reference_arm_exit_quietly():
     env = dict(os.environ, RANK="1", WORLD_SIZE="2", LOCAL_RANK="1")
     out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--gpus", "2", "--steps", "1"],

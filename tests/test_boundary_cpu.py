@@ -1,5 +1,5 @@
 """Boundary checks that need no GPU: the product Graph against the reference-generated goldens, state_dict
-round trips with the REAL reference modules (skipped when neither /root/reference nor oracle/_ref is present),
+round trips in the reference's layout (pinned by what its own modules left in tests/golden/stgcn.npz),
 Lightning-style checkpoints, pickling, cache invalidation, the header-derived limits, and the independent FK
 cross-check of the oracle (scipy-composed homogeneous chain)."""
 import copy
@@ -15,8 +15,6 @@ from temporal_inverse_kinematics_b200 import _lib, engine, smpl_util
 from temporal_inverse_kinematics_b200.graph import Graph
 from temporal_inverse_kinematics_b200.pose_regressor import IKPoseTrainer, PoseRegressor, default_hparams
 from temporal_inverse_kinematics_b200.st_gcn import StgConfig, StgGcn18, StgLayerConfig
-
-needs_reference = pytest.mark.skipif(not ref_import.available(), reason="reference modules not present")
 
 
 def test_product_graph_bit_identical_to_reference(golden):
@@ -35,43 +33,43 @@ def test_product_graph_bit_identical_to_reference(golden):
     assert torch.equal(m.backbone.A, torch.tensor(g["coco|uniform|2|1"], dtype=torch.float32))
 
 
-@needs_reference
-def test_state_dict_round_trip_with_real_reference():
-    """pose_trainer.py:66-92: load_state_dict(strict=True) both ways against the reference's own PoseRegressor."""
-    ref = ref_import.load()
+def _reference_state(golden):
+    """The state dict the reference's own PoseRegressor loaded with strict=True when tests/golden/stgcn.npz was made
+    (oracle/make_golden.py); the stored checksum proves it is the same one."""
+    g = golden("stgcn.npz")
+    sd = synth.make_regressor_state(Graph("coco", "uniform", 2, 1).A, seed=0)
+    assert synth.state_checksum(sd) == float(g["state_checksum"]), "synthetic weight stream drifted"
+    return sd, g
+
+
+def test_state_dict_round_trip_with_real_reference(golden):
+    """pose_trainer.py:66-92: load_state_dict(strict=True) both ways in the reference's PoseRegressor layout.  The
+    reference's side is what its own modules left in tests/golden/stgcn.npz: the state dict it loaded and its poses."""
+    theirs, g = _reference_state(golden)
     torch.manual_seed(3)
-    theirs = ref.pose_trainer.PoseRegressor(ref_import.default_hparams()).eval()
     ours = PoseRegressor(default_hparams()).eval()
-    sd_t = theirs.state_dict()
-    assert list(sd_t.keys()) == list(ours.state_dict().keys())
-    assert all(sd_t[k].shape == v.shape and sd_t[k].dtype == v.dtype for k, v in ours.state_dict().items())
-    ours.load_state_dict(sd_t, strict=True)
+    assert list(theirs.keys()) == list(ours.state_dict().keys())
+    assert all(theirs[k].shape == v.shape and theirs[k].dtype == v.dtype for k, v in ours.state_dict().items())
+    ours.load_state_dict(theirs, strict=True)
     for k, v in ours.state_dict().items():
-        assert torch.equal(v, sd_t[k]), k
-    sd_o = synth.make_regressor_state(Graph("coco", "uniform", 2, 1).A, seed=5)
-    ours.load_state_dict(sd_o, strict=True)
-    theirs.load_state_dict(ours.state_dict(), strict=True)
-    # the reference, carrying OUR state dict, reproduces the oracle port (ties the three together)
-    x = synth.make_clips(2, 9, seed=8)
-    with torch.no_grad():
-        y = theirs(x)["poses"]
-    assert float((y - sp.regressor_forward(sd_o, x)["poses"]).abs().max()) < 1e-5
+        assert torch.equal(v, theirs[k]), k
+    # OUR state dict, run through the oracle port, reproduces the reference's own output (ties the three together)
+    n, t, seed = [int(v) for v in g["t9_shape"]]
+    y = sp.regressor_forward(ours.state_dict(), synth.make_clips(n, t, seed=seed))["poses"]
+    assert float(np.abs(y.numpy() - g["t9_poses"]).max()) < 1e-5
 
 
-@needs_reference
-def test_lightning_checkpoint_from_real_reference(tmp_path):
-    """inference.py:136: IKPoseTrainer.load_from_checkpoint on a checkpoint whose state_dict comes from the
-    reference's own LightningModule layout ('regressor.' prefix, pickled hparams)."""
-    ref = ref_import.load()
-    torch.manual_seed(4)
+def test_lightning_checkpoint_from_real_reference(tmp_path, golden):
+    """inference.py:136: IKPoseTrainer.load_from_checkpoint on a checkpoint in the reference's own LightningModule
+    layout ('regressor.' prefix, pickled hparams), carrying the state dict the reference's PoseRegressor loaded."""
+    sd, _ = _reference_state(golden)
     hp = ref_import.default_hparams()
-    reg = ref.pose_trainer.PoseRegressor(hp)
-    ckpt = {"state_dict": {"regressor." + k: v for k, v in reg.state_dict().items()}, "hparams": vars(hp), "epoch": 98}
+    ckpt = {"state_dict": {"regressor." + k: v for k, v in sd.items()}, "hparams": vars(hp), "epoch": 98}
     path = tmp_path / "checkpoint_epoch=98.ckpt"
     torch.save(ckpt, path)
     m = IKPoseTrainer.load_from_checkpoint(str(path))
     assert m.hparams.win_size == hp.win_size and m.hparams.graph_layout == "coco"
-    for k, v in reg.state_dict().items():
+    for k, v in sd.items():
         assert torch.equal(m.state_dict()["regressor." + k], v), k
     # hparams stored as a Namespace (old Lightning) work as well
     ckpt["hparams"] = hp

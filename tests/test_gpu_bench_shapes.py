@@ -85,6 +85,26 @@ def test_fp32_parity_config1_shapes():
         assert mx < TOL_F32, (name, mx)
 
 
+def test_bench_dump_outputs_are_the_timed_results(tmp_path):
+    """bench.py --dump-outputs writes the poses and FK joints of its last timed step; its first clips are
+    synth.make_clips(seed=1234), which the oracle solves here."""
+    import os
+    import subprocess
+    import sys
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    out = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--batch", "64", "--steps", "2", "--warmup", "1",
+                          "--no-cpu", "--no-hbm", "--dump-outputs", str(tmp_path)], capture_output=True, text=True, timeout=600)
+    assert out.returncode == 0, out.stderr[-2000:]
+    poses, joints = np.load(tmp_path / "poses.npy"), np.load(tmp_path / "joints.npy")
+    assert poses.dtype == joints.dtype == np.float32 and poses.shape == (64, 4, 66) and joints.shape == (64, 4, J, 3)
+    _, sd = _model("bf16")
+    rest, parents = synth.make_rest_skeleton(), synth.SMPLX_BODY_PARENTS
+    w_poses, _, w_joints = _cpu_solve(sd, synth.make_clips(64, 64, seed=1234), rest, parents)
+    for name, got, want in (("poses", poses, w_poses), ("joints", joints, w_joints)):
+        mx, rms = _errs(got, want)
+        assert mx < TOL_BF16[name][0] and rms < TOL_BF16[name][1], (name, mx, rms)
+
+
 @pytest.mark.parametrize("dtype", ["fp32", "bf16"])
 def test_rot6d_head_variant_config1(dtype):
     """configs[1]'s second head variant (SURVEY 0.3): the commented-out iterative 6-D head + rot6d -> rotmat ->
