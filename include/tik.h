@@ -81,6 +81,37 @@ int tik_fk_body(const float* pose_dev, int pose_is_rotmat, const float* rest_hos
                 int J, const float* transl_dev, float* joints_dev, float* local_R_dev, float* global_R_dev,
                 int64_t F, void* stream);
 
+/* ------------------------------------------------------------------ mesh skinning
+ * Replaces the vertex output of common/smpl_util.py:22-82 run_smpl_inference(return_mesh=True) -> smplx.lbs.lbs
+ * (third-party; restated from the published SMPL-X formulation, see oracle/lbs_port.py).  The 55 SMPL-X joints and
+ * their local / global rotations come from tik_fk_body (want local and global rotations, NO transl); tik_lbs adds the
+ * pose blend shapes, skins the vertices and applies transl to vertices and joints, as smplx does.
+ * Device arrays of a model, packed once by the caller (temporal_inverse_kinematics_b200/smpl_util.py SmplxBodyModel): */
+#define TIK_LBS_MAX_LANDMARKS 8
+typedef struct TikLbsModel {
+  int32_t V;                 /* vertices */
+  int32_t J;                 /* joints: 55 */
+  int32_t kmax;              /* columns of the sparse skinning table: most non-zero weights of any vertex */
+  int32_t n_landmarks;       /* joints J .. J+n_landmarks-1 are these vertices (smplx VertexJointSelector) */
+  int32_t landmark_vid[TIK_LBS_MAX_LANDMARKS];
+  const float* v_shaped_dev;     /* (V,3) fp32: v_template + shapedirs . betas */
+  const float* rest_joints_dev;  /* (J,3) fp32: J_regressor . v_shaped, the rest joints given to tik_fk_body */
+  const void* posedirs_dev;      /* (ceil(3V/128)*128, 512) in the call's dtype, K contiguous: row 3v+c, column
+                                    9(j-1)+3a+b = posedirs[v,c,9(j-1)+3a+b] of the model file, zero padded; 16-byte aligned */
+  const int32_t* skin_idx_dev;   /* (V,kmax) joint of each non-zero skinning weight (padding: joint 0) */
+  const float* skin_w_dev;       /* (V,kmax) that weight (padding: 0) */
+} TikLbsModel;
+/* bytes of device workspace tik_lbs needs for F frames in `dtype` */
+int tik_lbs_workspace_bytes(const TikLbsModel* model, int dtype, int64_t F, int64_t* bytes);
+/* joints_dev (F,fk_J,3), local_R_dev / global_R_dev (F,fk_J,3,3): tik_fk_body outputs for the pose, fk_J >= 55 (joints
+ * past 54 are ignored); transl_dev (F,3) or NULL.  verts_dev (F,V,3) fp32 out.  joints_out_dev (F,joints_out_J,3) or NULL:
+ * posed joints + transl, joints_out_J <= 55 (the first joints_out_J joints) or 55 + n_landmarks (then followed by the
+ * landmark vertices).  dtype TIK_F32: 3xTF32 pose blend (1e-4 parity path); TIK_BF16: bf16 operands, fp32 accumulate.
+ * Skinning arithmetic is fp32 in both.  workspace_dev 256-byte aligned.  CUDA-graph capturable; F = 0 is a no-op. */
+int tik_lbs(const TikLbsModel* model, int dtype, const float* joints_dev, const float* local_R_dev, const float* global_R_dev,
+            int fk_J, const float* transl_dev, int64_t F, void* workspace_dev, int64_t workspace_bytes, float* verts_dev,
+            float* joints_out_dev, int joints_out_J, void* stream);
+
 /* ------------------------------------------------------------------ ST-GCN primitives
  * dtype is TIK_F32 (SIMT fp32, 1e-4 parity path) or TIK_BF16 (tcgen05 tensor cores, fp32 accumulate). */
 

@@ -21,6 +21,7 @@ def _header_defines():
 _H = _header_defines()
 TIK_F32, TIK_BF16 = _H["TIK_F32"], _H["TIK_BF16"]
 MAX_BLOCKS, MAX_SLABS, MAX_JOINTS = _H["TIK_MAX_BLOCKS"], _H["TIK_MAX_SLABS"], _H["TIK_MAX_JOINTS"]
+LBS_MAX_LANDMARKS = _H["TIK_LBS_MAX_LANDMARKS"]
 ACT_NONE, ACT_RELU, ACT_LEAKY = 0, 1, 2
 RES_NONE, RES_IDENTITY, RES_STEM, RES_CONV = 0, 1, 2, 3
 OUT_NODE_MAJOR, OUT_TIME_MAJOR, OUT_ROWS_F32 = 0, 1, 2
@@ -72,6 +73,11 @@ class TikNet(C.Structure):
                 ("w1_dev", vp), ("b1_dev", vp), ("w2_dev", vp), ("b2_dev", vp), ("leaky_slope", f32)]
 
 
+class TikLbsModel(C.Structure):
+    _fields_ = [("V", i32), ("J", i32), ("kmax", i32), ("n_landmarks", i32), ("landmark_vid", i32 * LBS_MAX_LANDMARKS),
+                ("v_shaped_dev", vp), ("rest_joints_dev", vp), ("posedirs_dev", vp), ("skin_idx_dev", vp), ("skin_w_dev", vp)]
+
+
 _PROTOS = {
     "tik_version": (C.c_int, []),
     "tik_last_error": (C.c_char_p, []),
@@ -84,6 +90,8 @@ _PROTOS = {
     "tik_rotmat_to_quat": (C.c_int, [vp, vp, i64, vp]),
     "tik_quat_to_aa": (C.c_int, [vp, vp, i64, vp]),
     "tik_fk_body": (C.c_int, [vp, C.c_int, C.POINTER(f32), C.POINTER(i32), C.c_int, vp, vp, vp, vp, i64, vp]),
+    "tik_lbs_workspace_bytes": (C.c_int, [C.POINTER(TikLbsModel), C.c_int, i64, C.POINTER(i64)]),
+    "tik_lbs": (C.c_int, [C.POINTER(TikLbsModel), C.c_int, vp, vp, vp, C.c_int, vp, i64, vp, i64, vp, vp, C.c_int, vp]),
     "tik_stem_gcn": (C.c_int, [C.c_int, vp, vp, vp, vp, vp, vp, vp, vp, vp, C.c_int, i64, C.c_int, C.c_int, C.c_int,
                                C.c_int, C.c_int, C.c_int, vp]),
     "tik_aggregate": (C.c_int, [C.c_int, vp, vp, vp, i64, C.c_int, C.c_int, C.c_int, C.c_int, vp]),

@@ -10,7 +10,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libtik.so")
-SOURCES = ["geometry.cu", "fk.cu", "stem.cu", "stem_block.cu", "stgcn_simt.cu", "rowgemm_tf32.cu", "stgcn_umma.cu", "gcn_fused.cu", "tcn_halo.cu", "plan.cu", "latency.cu", "pack.cu"]
+SOURCES = ["geometry.cu", "fk.cu", "stem.cu", "stem_block.cu", "stgcn_simt.cu", "rowgemm_tf32.cu", "stgcn_umma.cu", "gcn_fused.cu", "tcn_halo.cu", "plan.cu", "latency.cu", "pack.cu", "lbs.cu"]
 HEADERS = ["tik_common.cuh", "umma_prepared.h", "umma_ptx.cuh", os.path.join("..", "..", "include", "tik.h")]
 
 

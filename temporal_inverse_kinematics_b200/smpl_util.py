@@ -1,12 +1,13 @@
-"""Body-model forward kinematics behind the reference's ``run_smpl_inference`` signature.
+"""Body-model forward kinematics and mesh skinning behind the reference's ``run_smpl_inference`` signature.
 
-Mirrors reference common/smpl_util.py:8-82.  The reference delegates to the third-party ``smplx``
-package and licensed SMPL-X model files; neither is available offline, so ``load_smplx_models`` builds
-*synthetic* body models (seeded kinematic tree + rest joints + linear joint shape directions) and the
-joints come from the warp-per-frame FK kernel in libtik.so.  Vertices (``return_mesh=True``) need the
-licensed mesh template and are out of scope.
+Mirrors reference common/smpl_util.py:8-82.  The reference delegates to the third-party ``smplx`` package and the
+licensed SMPL-X model files.  ``load_smplx_models`` reads ``SMPLX_{MALE,FEMALE,NEUTRAL}.npz`` when the directory holds
+them (``SmplxBodyModel``: joints and vertices, ``return_mesh=True``) and otherwise builds *synthetic* body models
+(seeded kinematic tree + rest joints + linear joint shape directions; joints only).  Joints come from the FK kernels in
+libtik.so, vertices from its linear-blend-skinning kernels (``lbs``).
 """
 import ctypes as C
+import os
 
 import numpy as np
 import torch
@@ -34,6 +35,10 @@ SMPLX_FULL_PARENTS = (SMPLX_BODY_PARENTS + [15, 15, 15]
                       + [21, 40, 41, 21, 43, 44, 21, 46, 47, 21, 49, 50, 21, 52, 53])
 SMPLX_LANDMARK_NAMES = ["nose", "right_eye", "left_eye", "right_ear", "left_ear"]      # smplx JOINT_NAMES[55:60]
 SMPLX_LANDMARK_PARENT = 15                                                              # head
+# smplx vertex_ids["smplx"] of those landmarks (nose, reye, leye, rear, lear): what VertexJointSelector appends after joint 54
+SMPLX_LANDMARK_VERTEX_IDS = [9120, 9929, 9448, 616, 6]
+SMPLX_NUM_JOINTS = 55
+SMPLX_NUM_BETAS = 10                                                                    # smplx.create default; the reference passes betas[:10]
 
 
 def fk_body(pose, rest_joints, parents, transl=None, want_local=False, want_global=False):
@@ -100,10 +105,179 @@ class SyntheticBodyModel:
         return self.rest_joints + self.joint_shapedirs @ np.asarray(betas, dtype=np.float32)[: self.joint_shapedirs.shape[2]]
 
 
+def read_smplx_npz(path):
+    """Model arrays of one SMPL-X ``.npz`` file.  Opened without pickle support and only these keys are read: real files
+    also carry object arrays, which are never loaded.  Shapes and the kinematic tree are checked (``ValueError``)."""
+    keys = ("v_template", "shapedirs", "posedirs", "J_regressor", "weights", "kintree_table", "f")
+    with np.load(path, allow_pickle=False) as z:
+        missing = [k for k in keys if k not in z.files]
+        if missing:
+            raise ValueError(f"{path}: missing {missing}")
+        a = {k: np.asarray(z[k]) for k in keys}
+    V, J = a["v_template"].shape[0], SMPLX_NUM_JOINTS
+    want = {"v_template": (V, 3), "posedirs": (V, 3, (J - 1) * 9), "J_regressor": (J, V), "weights": (V, J),
+            "kintree_table": (2, J)}
+    for k, shp in want.items():
+        if a[k].shape != shp:
+            raise ValueError(f"{path}: {k} has shape {a[k].shape}, expected {shp}")
+    if a["shapedirs"].ndim != 3 or a["shapedirs"].shape[:2] != (V, 3) or a["shapedirs"].shape[2] < SMPLX_NUM_BETAS:
+        raise ValueError(f"{path}: shapedirs has shape {a['shapedirs'].shape}, expected ({V}, 3, >={SMPLX_NUM_BETAS})")
+    if a["f"].ndim != 2 or a["f"].shape[1] != 3:
+        raise ValueError(f"{path}: f has shape {a['f'].shape}, expected (n, 3)")
+    if V < 1 or not np.array_equal(a["kintree_table"][0, 1:].astype(np.int64), SMPLX_FULL_PARENTS[1:J]):
+        raise ValueError(f"{path}: kintree_table is not the SMPL-X tree")      # the root's entry is ignored, as smplx does
+    return a
+
+
+class SmplxBodyModel:
+    """A body model read from an SMPL-X model file: the same surface as ``SyntheticBodyModel`` (``parents``,
+    ``joint_names``, ``skeleton``, ``rest(betas)``, ``faces``) plus the mesh, skinned on the GPU by ``lbs``.
+
+    skeleton='body': joints 0..21; skeleton='full': the 55 joints followed by the five face landmarks, which are the
+    posed mesh vertices ``landmark_vertex_ids`` (smplx's VertexJointSelector; checked against V for 'full' only)."""
+
+    def __init__(self, arrays, gender="neutral", batch_size=1, device="cuda", skeleton="body",
+                 landmark_vertex_ids=SMPLX_LANDMARK_VERTEX_IDS):
+        self.gender, self.batch_size, self.device = gender, batch_size, device
+        if skeleton == "body":
+            self.parents, self.joint_names = list(SMPLX_BODY_PARENTS), list(SMPLX_BODY_JOINT_NAMES)
+        elif skeleton == "full":
+            self.parents = list(SMPLX_FULL_PARENTS) + [SMPLX_LANDMARK_PARENT] * len(SMPLX_LANDMARK_NAMES)
+            self.joint_names = list(SMPLX_FULL_JOINT_NAMES) + list(SMPLX_LANDMARK_NAMES)
+        else:
+            raise ValueError("skeleton must be 'body' or 'full'")
+        self.skeleton = skeleton
+        self.v_template = np.asarray(arrays["v_template"], dtype=np.float64)
+        self.V = self.v_template.shape[0]
+        self.landmark_vertex_ids = [int(i) for i in landmark_vertex_ids]
+        if len(self.landmark_vertex_ids) != len(SMPLX_LANDMARK_NAMES) or (
+                skeleton == "full" and not all(0 <= i < self.V for i in self.landmark_vertex_ids)):
+            raise ValueError(f"landmark_vertex_ids must be {len(SMPLX_LANDMARK_NAMES)} vertex indices below V={self.V}")
+        self.shapedirs = np.asarray(arrays["shapedirs"], dtype=np.float64)[:, :, :SMPLX_NUM_BETAS]
+        self.posedirs = np.asarray(arrays["posedirs"], dtype=np.float32)
+        self.J_regressor = np.asarray(arrays["J_regressor"], dtype=np.float64)
+        self.weights = np.asarray(arrays["weights"], dtype=np.float32)
+        self.faces = np.asarray(arrays["f"])
+        # sparse skinning table: every non-zero weight of a row (exact zeros dropped, no threshold, no renormalisation)
+        nz = self.weights != 0
+        self.kmax = max(1, int(nz.sum(axis=1).max()))
+        self.skin_idx = np.zeros((self.V, self.kmax), dtype=np.int32)
+        self.skin_w = np.zeros((self.V, self.kmax), dtype=np.float32)
+        for v in range(self.V):
+            j = np.flatnonzero(nz[v])
+            self.skin_idx[v, :len(j)] = j
+            self.skin_w[v, :len(j)] = self.weights[v, j]
+        self._packed, self._shaped = {}, {}
+
+    def to(self, device):
+        self.device = device
+        return self
+
+    def shaped(self, betas=None):
+        """-> (v_shaped (V,3), rest joints (55,3)), float64: v_template + shapedirs[..., :10] . betas and its J_regressor."""
+        v = self.v_template
+        if betas is not None:
+            b = np.asarray(betas, dtype=np.float64).reshape(-1)
+            if b.shape[0] > SMPLX_NUM_BETAS:
+                raise ValueError(f"at most {SMPLX_NUM_BETAS} betas, got {b.shape[0]}")
+            v = v + self.shapedirs[:, :, :b.shape[0]] @ b
+        return v, self.J_regressor @ v
+
+    def rest(self, betas=None):
+        """Rest joints (55,3) fp32 for ``betas`` (None: the template)."""
+        return self.shaped(betas)[1].astype(np.float32)
+
+    def device_shape(self, betas, device):
+        """(v_shaped, rest joints) as CUDA fp32 tensors plus the rest joints on the host, cached per betas."""
+        key = (str(device), None if betas is None else np.asarray(betas, dtype=np.float32).reshape(-1).tobytes())
+        if key not in self._shaped:
+            if len(self._shaped) >= 16:
+                self._shaped.clear()
+            v, j = self.shaped(betas)
+            j32 = np.ascontiguousarray(j, dtype=np.float32)
+            self._shaped[key] = (torch.from_numpy(v.astype(np.float32)).to(device), torch.from_numpy(j32).to(device), j32)
+        return self._shaped[key]
+
+    def device_pack(self, dtype, device):
+        """posedirs as the (ceil(3V/128)*128, 512) K-contiguous operand in ``dtype`` and the sparse skinning table, on
+        ``device``; packed once per (dtype, device)."""
+        key = (dtype, str(device))
+        if key not in self._packed:
+            rows = -(-3 * self.V // 128) * 128
+            pd = np.zeros((rows, 512), dtype=np.float32)
+            pd[:3 * self.V, :self.posedirs.shape[2]] = self.posedirs.reshape(3 * self.V, -1)
+            t = torch.from_numpy(pd).to(device)
+            self._packed[key] = (t.to(torch.bfloat16) if dtype == "bf16" else t, torch.from_numpy(self.skin_idx).to(device),
+                                 torch.from_numpy(self.skin_w).to(device))
+        return self._packed[key]
+
+
 def load_smplx_models(smplx_dir, device, batch_size, skeleton="body"):
-    """Same signature as reference common/smpl_util.py:8-19; ``smplx_dir`` is unused (synthetic models).
-    skeleton='full' builds the 55-joint + landmark tree (hands, jaw, eyes; SURVEY.md 8f row 3)."""
-    return {g: SyntheticBodyModel(g, batch_size, device, skeleton=skeleton) for g in ("male", "female", "neutral")}
+    """Same signature as reference common/smpl_util.py:8-19.  With ``smplx_dir`` holding SMPLX_{MALE,FEMALE,NEUTRAL}.npz
+    (the reference's file names) the models are read from them (``SmplxBodyModel``, joints and vertices); with None or a
+    directory without them, synthetic models (joints only).  skeleton='full' gives the 55 joints + five face landmarks
+    (SURVEY.md 8f row 3)."""
+    genders = ("male", "female", "neutral")
+    if smplx_dir is not None:
+        paths = {g: os.path.join(smplx_dir, f"SMPLX_{g.upper()}.npz") for g in genders}
+        present = [g for g in genders if os.path.exists(paths[g])]
+        if present and len(present) < len(genders):
+            raise FileNotFoundError(f"{smplx_dir} holds only {[os.path.basename(paths[g]) for g in present]}")
+        if present:
+            return {g: SmplxBodyModel(read_smplx_npz(paths[g]), g, batch_size, device, skeleton=skeleton) for g in genders}
+    return {g: SyntheticBodyModel(g, batch_size, device, skeleton=skeleton) for g in genders}
+
+
+def lbs(pose, model, betas=None, transl=None, dtype="fp32"):
+    """SMPL-X forward of a ``SmplxBodyModel`` on the GPU (smplx.lbs.lbs + VertexJointSelector + transl).
+    pose (F, 22 | 55 | 60, 3) axis-angle CUDA tensor (22: body only, hands / jaw / eyes identity; 60: joints past 54
+    ignored); betas up to 10 values or None; transl (F,3) CUDA tensor or None; dtype 'fp32' (3xTF32 pose blend, 1e-4
+    parity) or 'bf16' (bf16 pose-blend operands).  Returns joints (F, len(model.parents), 3) and vertices (F, V, 3), fp32
+    CUDA tensors."""
+    if not (torch.is_tensor(pose) and pose.is_cuda):
+        raise RuntimeError("lbs: pose must be a CUDA tensor -- there is no CPU fallback")
+    if transl is not None and not (torch.is_tensor(transl) and transl.is_cuda):
+        raise RuntimeError("lbs: transl must be a CUDA tensor -- there is no CPU fallback")
+    if not isinstance(model, SmplxBodyModel):
+        raise TypeError("lbs needs a SmplxBodyModel (a model read from an SMPL-X file)")
+    if pose.dim() != 3 or pose.shape[1] not in (22, SMPLX_NUM_JOINTS, 60) or pose.shape[2] != 3:
+        raise ValueError(f"lbs: pose must be (F, 22 | 55 | 60, 3), got {tuple(pose.shape)}")
+    F = pose.shape[0]
+    if transl is not None and tuple(transl.shape) != (F, 3):
+        raise ValueError(f"lbs: transl must be ({F}, 3), got {tuple(transl.shape)}")
+    if dtype not in ("fp32", "bf16"):
+        raise ValueError(f"lbs: dtype must be 'fp32' or 'bf16', got {dtype!r}")
+    dev = pose.device
+    pose = pose.detach().float()
+    if pose.shape[1] == 22:                                      # full_pose_from_amass of a 66-column pose
+        pose = torch.cat([pose, pose.new_zeros(F, SMPLX_NUM_JOINTS - 22, 3)], dim=1)
+    pose = pose[:, :SMPLX_NUM_JOINTS].contiguous()
+    if transl is not None:
+        transl = transl.detach().float().contiguous()
+    v_shaped, rest_dev, rest_host = model.device_shape(betas, dev)
+    posedirs, skin_idx, skin_w = model.device_pack(dtype, dev)
+    Jo = len(model.parents)
+    joints = torch.empty((F, Jo, 3), dtype=torch.float32, device=dev)
+    verts = torch.empty((F, model.V, 3), dtype=torch.float32, device=dev)
+    if F == 0:
+        return joints, verts
+    fk_j, fk_loc, fk_glo = fk_body(pose, rest_host, SMPLX_FULL_PARENTS[:SMPLX_NUM_JOINTS], want_local=True, want_global=True)
+    m = L.TikLbsModel()
+    m.V, m.J, m.kmax = model.V, SMPLX_NUM_JOINTS, model.kmax
+    if model.skeleton == "full":
+        m.n_landmarks = len(model.landmark_vertex_ids)
+        for k, v in enumerate(model.landmark_vertex_ids):
+            m.landmark_vid[k] = v
+    m.v_shaped_dev, m.rest_joints_dev, m.posedirs_dev = v_shaped.data_ptr(), rest_dev.data_ptr(), posedirs.data_ptr()
+    m.skin_idx_dev, m.skin_w_dev = skin_idx.data_ptr(), skin_w.data_ptr()
+    dt = L.TIK_BF16 if dtype == "bf16" else L.TIK_F32
+    nbytes = L.i64()
+    with L.on_device(pose):
+        L.check(L.lib().tik_lbs_workspace_bytes(C.byref(m), dt, F, C.byref(nbytes)))
+        ws = torch.empty(max(1, nbytes.value), dtype=torch.uint8, device=dev)
+        L.check(L.lib().tik_lbs(C.byref(m), dt, L.ptr(fk_j), L.ptr(fk_loc), L.ptr(fk_glo), SMPLX_NUM_JOINTS, L.ptr(transl), F,
+                                L.ptr(ws), nbytes.value, L.ptr(verts), L.ptr(joints), Jo, L.stream_ptr(dev)))
+    return joints, verts
 
 
 def full_pose_from_amass(poses, n_joints):
@@ -123,21 +297,27 @@ def full_pose_from_amass(poses, n_joints):
 def run_smpl_inference(data, smplx_models, device, apply_trans=True, apply_root_rot=True, apply_shape=True,
                        return_mesh=False):
     """data: {'poses': (F, >=66) axis-angle, 'gender', ['trans' (F,3)], ['betas']} -> joints (F, J, 3) numpy
-    (J = 22 for body models, 60 for skeleton='full' models: 55 SMPL-X joints + 5 face landmarks).
+    (J = 22 for body models, 60 for skeleton='full' models: 55 SMPL-X joints + 5 face landmarks), or (joints, vertices
+    (F, V, 3)) with return_mesh=True, which needs a model read from an SMPL-X file (``SmplxBodyModel``).
     Reference common/smpl_util.py:22-82; the fixed-batch padding loop there is unnecessary here (one launch)."""
-    if return_mesh:
-        raise NotImplementedError("SMPL-X vertices need the licensed mesh template; only joints are produced")
     model = smplx_models[str(data["gender"])]
+    mesh = isinstance(model, SmplxBodyModel)
+    if return_mesh and not mesh:
+        raise NotImplementedError("vertices need an SMPL-X model file: load_smplx_models(dir) with SMPLX_*.npz in dir")
     J = len(model.parents)
-    if J == 22:
+    if J == 22 and not return_mesh:
         poses = torch.as_tensor(np.asarray(data["poses"], dtype=np.float32)[:, :66]).to(device).view(-1, 22, 3).contiguous()
-    else:                                                         # full skeleton: body + hands (+ identity jaw / eyes / landmarks)
-        poses = torch.as_tensor(full_pose_from_amass(data["poses"], J)).to(device)
+    else:                                                         # full skeleton / mesh: body + hands (+ identity jaw / eyes / landmarks)
+        poses = torch.as_tensor(full_pose_from_amass(data["poses"], SMPLX_NUM_JOINTS if mesh else J)).to(device)
     if not apply_root_rot:
         poses = poses.clone()
         poses[:, 0] = 0
     transl = torch.as_tensor(np.asarray(data["trans"], dtype=np.float32)).to(device) if apply_trans else None
-    rest = model.rest(np.asarray(data["betas"])[:10] if apply_shape else None)
+    betas = np.asarray(data["betas"])[:10] if apply_shape else None
+    if mesh and (return_mesh or J != 22):                         # landmark joints are mesh vertices
+        joints, verts = lbs(poses, model, betas, transl)
+        return (joints.cpu().numpy(), verts.cpu().numpy()) if return_mesh else joints.cpu().numpy()
+    rest = model.rest(betas)[:J]
     return fk_body(poses, rest, model.parents, transl).cpu().numpy()
 
 
