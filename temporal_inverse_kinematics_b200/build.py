@@ -25,8 +25,6 @@ STAMP = os.path.join(HERE, "build", "flavour.txt")
 
 
 def _flavour():
-    if os.environ.get("TIK_TEST_WAIT") == "1":
-        return "probe-testwait" if os.environ.get("TIK_PROBE") == "1" else "testwait"
     return "probe" if os.environ.get("TIK_PROBE") == "1" else "release"
 
 
@@ -54,8 +52,6 @@ def build(force=False, verbose=False):
         flags += ["-Xptxas", "-v"]
     if os.environ.get("TIK_PROBE") == "1":          # in-kernel clock64 probes for tools/umma_probe.py
         flags += ["-DTIK_PROBE"]
-    if os.environ.get("TIK_TEST_WAIT") == "1":      # experiment: spin on mbarrier.test_wait instead of try_wait
-        flags += ["-DTIK_TEST_WAIT"]
     variant = os.environ.get("TIK_BUILD_VARIANT")   # A/B library next to the product one: build/libtik_<name>.so with -D<NAME>
     obj_dir = os.path.join(HERE, "build", variant) if variant else os.path.join(HERE, "build")
     if variant:

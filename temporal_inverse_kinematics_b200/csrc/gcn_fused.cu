@@ -5,7 +5,7 @@
 // Replaces the aggregate kernel + channel GEMM pair (gconv_origin.py:56-65 with the einsum moved in front of the
 // conv, st_gcn_aaai18.py:178-179), i.e. two full activation passes through HBM per block.
 //
-// A tile is f <= 7 frames x 17 nodes of one clip (<= 119 rows, row r = v*f + t_local; f = gcn_fused_frames(T)), fetched
+// A tile is f <= 7 frames x 17 nodes of one clip (<= 119 rows, row r = v*f + t_local; f = gcn_fused_frames(T, Cin)), fetched
 // as ONE 4-D TMA box (64 channels, f frames, 17 nodes, 1 clip) per 64-channel slab of the node-major activations.
 //   MMA 1 (aggregation as a dense block-structured GEMM):   D1[128 x Cin] = Abd[128 x 128] . Xtile[128 x Cin]
 //          Abd[(w,t),(v,t')] = A^[v,w] * delta(t,t'), bf16, K-major, resident in shared memory;
@@ -36,7 +36,7 @@ constexpr int kGwMaxBufs = 16;                     // gcn_wide_kernel: 64-channe
 
 struct GcnFusedParams {
   CUtensorMap map_x, map_out, map_w;
-  int32_t n_clips, T, V, ttg, tiles_t;   // ttg = frames per tile (gcn_fused_frames(T) <= 7)
+  int32_t n_clips, T, V, ttg, tiles_t;   // ttg = frames per tile (gcn_fused_frames(T, cin) <= 7)
   int32_t xbufs;                          // input tiles in flight
   int32_t sbufs;                          // staging tiles (2: the store of tile i-1 may still be reading while tile i is staged)
   int32_t halves;                         // gcn_wide_kernel: CTAs per tile (output-channel split)
@@ -46,7 +46,7 @@ struct GcnFusedParams {
   const float* bias;                      // (V, COUT)
   const __nv_bfloat16* abd;               // (128, 128) row-major block-structured adjacency, copied to tensor memory
   int32_t relu;
-  int32_t rev, l2;                        // LaunchOpts: clips walked last to first; evict-first hint on the X loads
+  int32_t rev;                            // LaunchOpts: clips walked last to first
 };
 
 template <int CIN, int COUT>
@@ -135,7 +135,6 @@ __global__ void __launch_bounds__(kGfThreads, 1) gcn_fused_kernel(const __grid_c
       mbar_expect_tx(w_full, (uint32_t)(KC1 * COUT * 128));
       for (int kc = 0; kc < KC1; ++kc) tma_load_2d(s_w + (size_t)kc * COUT * 128, &p.map_w, w_full, kc * 64, 0);
       int b = 0; uint32_t phase = 0;
-      const uint64_t pol = p.l2 ? l2_policy_evict_first() : 0;
       for (int tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
         const int nf = tile / p.tiles_t, tt = tile - nf * p.tiles_t;
         const int n = p.rev ? p.n_clips - 1 - nf : nf;
@@ -143,7 +142,7 @@ __global__ void __launch_bounds__(kGfThreads, 1) gcn_fused_kernel(const __grid_c
         mbar_wait(&x_empty[b], phase ^ 1);
         mbar_expect_tx(&x_full[b], x_bytes);
         for (int kc = 0; kc < KC1; ++kc)
-          tma_load_4d(s_x + ((size_t)b * KC1 + kc) * kGfTile, &p.map_x, &x_full[b], kc * 64, t0, 0, n, pol);
+          tma_load_4d(s_x + ((size_t)b * KC1 + kc) * kGfTile, &p.map_x, &x_full[b], kc * 64, t0, 0, n);
         if (++b == p.xbufs) { b = 0; phase ^= 1; }
       }
     }
@@ -410,7 +409,6 @@ __global__ void __launch_bounds__(kGfThreads, 1) gcn_fused_pair_kernel(const __g
       mbar_expect_tx(w_full, (uint32_t)(COUT * 128));
       tma_load_2d(s_w, &p.map_w, w_full, 0, 0);
       int b = 0; uint32_t phase = 0;
-      const uint64_t pol = p.l2 ? l2_policy_evict_first() : 0;
       for (int it = 0; it < my_pairs; ++it) {
         mbar_wait(&x_empty[b], phase ^ 1);
         mbar_expect_tx(&x_full[b], 2 * x_bytes);
@@ -418,7 +416,7 @@ __global__ void __launch_bounds__(kGfThreads, 1) gcn_fused_pair_kernel(const __g
         for (int h = 0; h < 2; ++h) {
           int n, t0; bool valid;
           tile_of(it, h, n, t0, valid);
-          tma_load_4d(s_x + ((size_t)b * 2 + h) * kGfTile, &p.map_x, &x_full[b], 0, t0, 0, n, pol);
+          tma_load_4d(s_x + ((size_t)b * 2 + h) * kGfTile, &p.map_x, &x_full[b], 0, t0, 0, n);
         }
         if (++b == p.xbufs) { b = 0; phase ^= 1; }
       }
@@ -683,14 +681,13 @@ __global__ void __launch_bounds__(kGfThreads, 1) gcn_wide_kernel(const __grid_co
       tma_load_2d(s_abd, &p.map_w, abd_full, 0, 0);
       tma_load_2d(s_abd + kGfTile, &p.map_w, abd_full, 64, 0);
       int b = 0; uint32_t phase = 0;
-      const uint64_t pol = p.l2 ? l2_policy_evict_first() : 0;
       for (int it = 0; it < my_tiles; ++it) {
         int n, t0;
         tile_of(it, n, t0);
         for (int q = 0; q < NQ; ++q) {
           mbar_wait(&x_empty[b], phase ^ 1);
           mbar_expect_tx(&x_full[b], x_bytes);
-          tma_load_4d(s_x + (size_t)b * p.xslab, &p.map_x, &x_full[b], q * 64, t0, 0, n, pol);
+          tma_load_4d(s_x + (size_t)b * p.xslab, &p.map_x, &x_full[b], q * 64, t0, 0, n);
           if (++b == p.xbufs) { b = 0; phase ^= 1; }
         }
       }
@@ -873,29 +870,23 @@ struct GcnFusedPrepared {
 };
 constexpr int kGwCo = 128;                 // output channels per CTA of the wide kernel
 
-// Frames per tile: at most 7 (7 x 17 nodes = 119 of the 128 MMA rows), balanced over the ceil(T/7) tiles of a clip so
-// that the last tile re-does as few frames as possible (T=16: 3 tiles of 6, not 7+7+shifted 7; T=8: 2 tiles of 4).
-int gcn_fused_frames(int T) {
-  const int tiles = (T + 6) / 7;
-  return (T + tiles - 1) / tiles;
-}
-// the 256-channel kernel keeps tile rows on the accumulator columns: at most 5 frames (85 rows -> N = 96)
+// Frames per tile: at most 7 (7 x 17 nodes = 119 of the 128 MMA rows); the 256-channel kernel keeps tile rows on the
+// accumulator columns, at most 5 frames (85 rows -> N = 96).  Balanced over the tiles of a clip so that the last tile
+// re-does as few frames as possible (T=16: 3 tiles of 6, not 7+7+shifted 7; T=8: 2 tiles of 4).
 int gcn_fused_frames(int T, int cin) {
-  if (cin != 256) return gcn_fused_frames(T);
-  const int tiles = (T + 4) / 5;
+  const int max_frames = cin == 256 ? 5 : 7;
+  const int tiles = (T + max_frames - 1) / max_frames;
   return (T + tiles - 1) / tiles;
 }
 
 bool gcn_fused_supported(int cin, int cout, int V, int K) {
   if (K != 1 || V * 7 > 128 || V < 1) return false;
-  if (cin == 256 && cout == 256) return !getenv("TIK_NO_GCN_WIDE");          // gcn_wide_kernel
-  return (cin == 64 && (cout == 64 || cout == 128)) || (cin == 128 && (cout == 128 || cout == 256));
+  return (cin == 64 && (cout == 64 || cout == 128)) || (cin == 128 && (cout == 128 || cout == 256)) ||
+         (cin == 256 && cout == 256);                                          // gcn_wide_kernel
 }
 
 int gcn_fused_prepare(const void* x, const void* abd, const void* w, const float* bias, void* out, int64_t n_clips, int T, int V,
-                      int cin, int cout, int relu, GcnFusedPrepared** outp, int x_row, int out_row) {
-  if (x_row <= 0) x_row = cin;                             // channels per row of the tensors in memory: a launch may work on a
-  if (out_row <= 0) out_row = cout;                        // channel slice of wider activations
+                      int cin, int cout, int relu, GcnFusedPrepared** outp) {
   TIK_CHECK_ARG(gcn_fused_supported(cin, cout, V, 1), "fused gcn: unsupported shape cin=%d cout=%d V=%d", cin, cout, V);
   TIK_CHECK_ARG(x && abd && w && bias && out && n_clips > 0 && T > 0, "fused gcn: bad arguments");
   GcnFusedPrepared* g = new GcnFusedPrepared();
@@ -909,13 +900,13 @@ int gcn_fused_prepare(const void* x, const void* abd, const void* w, const float
   int rc = TIK_OK;
   {
     uint64_t dims[4] = {(uint64_t)cin, (uint64_t)T, (uint64_t)V, (uint64_t)n_clips};
-    uint64_t strides[3] = {(uint64_t)x_row * 2, (uint64_t)x_row * 2 * T, (uint64_t)x_row * 2 * T * V};
+    uint64_t strides[3] = {(uint64_t)cin * 2, (uint64_t)cin * 2 * T, (uint64_t)cin * 2 * T * V};
     uint32_t box[4] = {64, (uint32_t)p.ttg, (uint32_t)V, 1};
     rc = encode_bf16_map(&p.map_x, x, 4, dims, strides, box);
   }
   if (rc == TIK_OK) {
     uint64_t dims[4] = {(uint64_t)cout, (uint64_t)T, (uint64_t)V, (uint64_t)n_clips};
-    uint64_t strides[3] = {(uint64_t)out_row * 2, (uint64_t)out_row * 2 * T, (uint64_t)out_row * 2 * T * V};
+    uint64_t strides[3] = {(uint64_t)cout * 2, (uint64_t)cout * 2 * T, (uint64_t)cout * 2 * T * V};
     uint32_t box[4] = {64, (uint32_t)p.ttg, (uint32_t)V, 1};
     rc = encode_bf16_map(&p.map_out, out, 4, dims, strides, box);
   }
@@ -957,7 +948,7 @@ int gcn_fused_prepare(const void* x, const void* abd, const void* w, const float
   const int w_bytes = kc1 * cout * 128;
   const int bias_bytes = (V * (cout + 4) * 4 + 1023) / 1024 * 1024;
   // 64 -> 128 would need 576 TMEM columns to keep D1 double buffered as a pair; single-buffered it is slower (360 vs 324 us)
-  g->pair = cin == 64 && cout == 64 && !getenv("TIK_NO_GCN_PAIR");
+  g->pair = cin == 64 && cout == 64;
   const int stage_tiles = g->pair ? 2 : 1;                // input tiles per ring stage
   // two staging tiles when at least three input stages still fit beside them (measured: input depth matters more);
   // the pair kernel always stages both of its tiles
@@ -1032,7 +1023,7 @@ int gcn_fused_launch(GcnFusedPrepared* g, int64_t n_clips, cudaStream_t s) {
   TIK_CHECK_ARG(n_clips <= cap, "fused gcn: n_clips exceeds the prepared capacity");
   const int32_t saved = p.n_clips;
   p.n_clips = (int32_t)n_clips;            // tiles only over the valid clips (tensor maps keep the full capacity)
-  p.rev = launch_opts().rev; p.l2 = launch_opts().l2;
+  p.rev = launch_opts().rev;
   int sms = 148;
   { int dev = 0; if (cudaGetDevice(&dev) == cudaSuccess) cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev); }
   const int64_t tiles = n_clips * p.tiles_t;
@@ -1043,7 +1034,6 @@ int gcn_fused_launch(GcnFusedPrepared* g, int64_t n_clips, cudaStream_t s) {
     rc = gf_launch_wide(g, (unsigned)std::min<int64_t>(want, cap_ctas), s);
   } else if (g->pair && g->cout == 64) rc = gf_launch_pair<64>(g, grid, s);
   else if (g->pair && g->cout == 128) rc = gf_launch_pair<128>(g, grid, s);
-  else if (g->cin == 64 && g->cout == 64) rc = gf_launch_variant<64, 64>(g, grid, s);
   else if (g->cin == 64 && g->cout == 128) rc = gf_launch_variant<64, 128>(g, grid, s);
   else if (g->cin == 128 && g->cout == 128) rc = gf_launch_variant<128, 128>(g, grid, s);
   else rc = gf_launch_variant<128, 256>(g, grid, s);
@@ -1059,7 +1049,7 @@ extern "C" int tik_gcn_fused(const void* x_dev, const void* abd_dev, const void*
                              int64_t N, int T, int V, int Cin, int Cout, int relu, void* stream) {
   using namespace tik;
   GcnFusedPrepared* g = nullptr;
-  int rc = gcn_fused_prepare(x_dev, abd_dev, w_dev, bias_dev, out_dev, N, T, V, Cin, Cout, relu, &g, 0, 0);
+  int rc = gcn_fused_prepare(x_dev, abd_dev, w_dev, bias_dev, out_dev, N, T, V, Cin, Cout, relu, &g);
   if (rc != TIK_OK) return rc;
   rc = gcn_fused_launch(g, N, (cudaStream_t)stream);
   gcn_fused_free(g);

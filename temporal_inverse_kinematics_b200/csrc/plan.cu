@@ -26,20 +26,15 @@ bool pdl_enabled() {
 }
 
 LaunchOpts& launch_opts() {
-  static thread_local LaunchOpts o = {0, 0};
+  static thread_local LaunchOpts o = {0};
   return o;
 }
-// Serpentine tile order + evict-first activation loads (tik_common.cuh LaunchOpts): TIK_SERPENTINE / TIK_L2_HINT = 0 | 1.
+// Serpentine tile order (tik_common.cuh LaunchOpts): TIK_SERPENTINE = 0 | 1.
 // Measured on one box, three alternating rounds (tools/ab_env.sh, profiles/r2_ab_serpentine.log), sum of the 17 network
-// launches of a configs[2] step: serpentine 3653-3658 us vs 3672-3700 us (on by default); the evict-first hint costs
-// 3-4 % (3755-3816 us: it also evicts tiles that a second CTA is about to read) and stays off.
+// launches of a configs[2] step: serpentine 3653-3658 us vs 3672-3700 us (on by default).
 static int serpentine_enabled() {           // read per run (two getenv calls): tests and A/B tools flip it inside one process
   const char* e = getenv("TIK_SERPENTINE");
   return e ? atoi(e) : 1;
-}
-static int l2_hint_enabled() {
-  const char* e = getenv("TIK_L2_HINT");
-  return e ? atoi(e) : 0;
 }
 
 void set_error(const char* fmt, ...) {
@@ -67,7 +62,6 @@ struct Step {
   const TikBlock* blk = nullptr;
   bool out_is_feat = false;   // GEMM: writes the batch-level feature buffer at the chunk's offset
   bool out_is_poses = false;  // GEMM: writes the caller's poses pointer
-  bool agg_only = false;      // FUSED_GCN used as a pure aggregation pass (identity weights): counts as 'aggregate'
   int k_identity = 0;         // GEMM: K columns that only carry an identity residual (not algorithmic FLOPs)
   const float* w_big = nullptr;   // fp32 GEMM: the weights split into their TF32 parts once per plan (rowgemm_tf32.cu)
   const float* w_small = nullptr;
@@ -100,7 +94,7 @@ struct TikPlan {
 namespace tik {
 
 struct WsLayout {
-  int64_t off_x0, off_x1, off_agg, off_h, off_r0, off_feat, off_z, off_abd, off_w16, off_eye, off_zbias, off_wsplit, total_bytes;
+  int64_t off_x0, off_x1, off_agg, off_h, off_r0, off_feat, off_z, off_abd, off_w16, off_wsplit, total_bytes;
 };
 
 static int check_net(const TikNet* net, int dtype) {
@@ -162,8 +156,6 @@ static void ws_layout(const TikNet* net, int dtype, int64_t n, int64_t n_max, in
   L->off_z = off; off = align_up(off + z * n_max * es, 1024);
   L->off_abd = off; off = align_up(off + (int64_t)net->n_blocks * 128 * 128 * 2, 1024);
   L->off_w16 = off; off = align_up(off + stem_block_workspace_bytes(), 1024);
-  L->off_eye = off; off = align_up(off + 128 * 128 * 2, 1024);               // identity weights: aggregation-only passes
-  L->off_zbias = off; off = align_up(off + 32 * 128 * 4, 1024);             // zero bias table (V <= 32 rows)
   L->off_wsplit = off;                                                       // fp32 plans: every GEMM's weights as TF32 big / small parts
   if (dtype == TIK_F32) {
     int64_t w_elems = 0;
@@ -221,7 +213,7 @@ static int run_impl(TikPlan* P, const float* x, int64_t N, float* poses, void* f
     if (st) trace->push_back({st, n});
     return TIK_OK;
   };
-  const int serp = serpentine_enabled(), l2 = l2_hint_enabled();
+  const int serp = serpentine_enabled();
   for (int64_t b0 = 0; b0 < N; b0 += P->n_max) {
     const int64_t nb = std::min<int64_t>(P->n_max, N - b0);
     for (int64_t n0 = 0; n0 < nb; n0 += P->n_chunk) {
@@ -231,9 +223,9 @@ static int run_impl(TikPlan* P, const float* x, int64_t N, float* poses, void* f
       for (auto& st : P->chunk_steps) {
         int rc = mark(&st, n);
         if (rc != TIK_OK) return rc;
-        launch_opts() = {serp ? (k & 1) : 0, l2};          // consecutive kernels walk the clips in opposite directions
+        launch_opts() = {serp ? (k & 1) : 0};              // consecutive kernels walk the clips in opposite directions
         rc = run_step(P, st, xc, n, n0, nullptr, s, win, b0 + n0);
-        launch_opts() = {0, 0};
+        launch_opts() = {0};
         if (rc != TIK_OK) return rc;
         ++k;
       }
@@ -242,9 +234,9 @@ static int run_impl(TikPlan* P, const float* x, int64_t N, float* poses, void* f
     for (auto& st : P->batch_steps) {
       int rc = mark(&st, nb);
       if (rc != TIK_OK) return rc;
-      launch_opts() = {serp && nb <= P->n_chunk ? (k & 1) : 0, l2};   // several chunks: the features were not written in one sweep
+      launch_opts() = {serp && nb <= P->n_chunk ? (k & 1) : 0};   // several chunks: the features were not written in one sweep
       rc = run_step(P, st, nullptr, nb, 0, poses ? poses + b0 * (int64_t)P->T_out * net.head_out : nullptr, s);
-      launch_opts() = {0, 0};
+      launch_opts() = {0};
       if (rc != TIK_OK) return rc;
       ++k;
     }
@@ -362,37 +354,8 @@ int tik_stgcn_plan_create(const TikNet* net, int dtype, int64_t n_chunk, int64_t
       s.fused_flops_per_clip = 2.0 * V * t * (double)b.c_in * b.c_out;
       P->chunk_steps.push_back(s);
     } else {
-      const bool tc_agg = dtype == TIK_BF16 && K == 1 && b.c_in % 128 == 0 && gcn_fused_supported(128, 128, V, 1) &&
-                          !getenv("TIK_NO_FUSED_GCN") && !getenv("TIK_NO_TC_AGG");
-      if (tc_agg) {
-        // wide layers (256 channels): the fused kernel does not fit, but its aggregation half does -- run it per
-        // 128-channel slice with identity weights and a zero bias (Abd . X on the tensor pipe, bf16 out), then the
-        // channel GEMM below.  Replaces the SIMT aggregate kernel (172 -> ~100 us at B=4096).
-        const int f = gcn_fused_frames(t);
-        std::vector<float> a_host((size_t)V * V);
-        cudaError_t ce = cudaMemcpy(a_host.data(), b.agg_dev, a_host.size() * sizeof(float), cudaMemcpyDeviceToHost);
-        std::vector<__nv_bfloat16> abd_host(128 * 128, __float2bfloat16_rn(0.f)), eye_host(128 * 128, __float2bfloat16_rn(0.f));
-        for (int w = 0; w < V; ++w)
-          for (int v = 0; v < V; ++v)
-            for (int q = 0; q < f; ++q) abd_host[(size_t)(w * f + q) * 128 + (v * f + q)] = __float2bfloat16_rn(a_host[(size_t)v * V + w]);
-        for (int d = 0; d < 128; ++d) eye_host[(size_t)d * 128 + d] = __float2bfloat16_rn(1.f);
-        void* abd_dev = ws + L.off_abd + (int64_t)i * 128 * 128 * 2;
-        if (ce == cudaSuccess) ce = cudaMemcpy(abd_dev, abd_host.data(), abd_host.size() * 2, cudaMemcpyHostToDevice);
-        if (ce == cudaSuccess) ce = cudaMemcpy(ws + L.off_eye, eye_host.data(), eye_host.size() * 2, cudaMemcpyHostToDevice);
-        if (ce == cudaSuccess) ce = cudaMemset(ws + L.off_zbias, 0, 32 * 128 * 4);
-        if (ce != cudaSuccess) { set_error("plan: aggregation operands upload failed: %s", cudaGetErrorString(ce)); delete P; return TIK_ERR_CUDA; }
-        for (int c0 = 0; c0 < b.c_in; c0 += 128) {
-          Step s; s.kind = Step::FUSED_GCN; s.blk = &b; s.t = t; s.agg_only = true;
-          int rcf = gcn_fused_prepare(reinterpret_cast<uint8_t*>(xbuf[cur]) + (size_t)c0 * 2, abd_dev, ws + L.off_eye,
-                                      reinterpret_cast<const float*>(ws + L.off_zbias), reinterpret_cast<uint8_t*>(agg) + (size_t)c0 * 2,
-                                      n_chunk, t, V, 128, 128, 0, &s.fused, b.c_in, b.c_in);
-          if (rcf != TIK_OK) { delete P; return rcf; }
-          P->chunk_steps.push_back(s);
-        }
-      } else {
-        Step s; s.kind = Step::AGG; s.src = xbuf[cur]; s.dst = agg; s.t = t; s.c = b.c_in; s.blk = &b;
-        P->chunk_steps.push_back(s);
-      }
+      Step s; s.kind = Step::AGG; s.src = xbuf[cur]; s.dst = agg; s.t = t; s.c = b.c_in; s.blk = &b;
+      P->chunk_steps.push_back(s);
       Step g; g.kind = Step::GEMM; memset(&g.g, 0, sizeof(g.g));
       g.g.n_slabs = K;
       for (int k = 0; k < K; ++k)
@@ -534,8 +497,7 @@ int tik_stgcn_plan_profile(TikPlan* P, const float* x, int64_t N, float* poses, 
     TIK_CUDA(cudaEventElapsedTime(&ms, ev[i], ev[i + 1]));
     Step& st = *trace[i].first;
     const int64_t n = trace[i].second;
-    const int kind = st.agg_only ? (int)Step::AGG
-                     : (st.kind == Step::FUSED_GCN || st.kind == Step::STEM_BLOCK || st.kind == Step::TCN_HALO) ? (int)Step::GEMM : (int)st.kind;   // tensor-core family
+    const int kind = (st.kind == Step::FUSED_GCN || st.kind == Step::STEM_BLOCK || st.kind == Step::TCN_HALO) ? (int)Step::GEMM : (int)st.kind;   // tensor-core family
     ms_by_kind[kind] += ms;
     launches_by_kind[kind] += 1;
     if (getenv("TIK_PLAN_TRACE")) {

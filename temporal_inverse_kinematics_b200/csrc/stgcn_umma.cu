@@ -72,11 +72,9 @@ struct UmmaParams {
   int32_t res_kind; const void* res; const float* res_w; int32_t res_cin, res_t_mul, res_t_in;
   void* out; int32_t out_layout;
   int32_t ts;                      // weights stationary in tensor memory (rowgemm_ts_kernel)
-  int32_t two_cta;                 // CTA pairs sharing one weight stream (rowgemm_umma2_kernel)
-  int32_t mc;                      // clusters of two CTAs multicasting the weight stream (rowgemm_umma_mc_kernel)
   const __nv_bfloat16* w_gmem;     // ts: (c_out, ktot) row-major weights
   int32_t ktot;
-  int32_t rev, l2;                 // LaunchOpts: tiles walked last to first; evict-first hint on the activation loads
+  int32_t rev;                     // LaunchOpts: tiles walked last to first
   unsigned long long* dbg_times;   // probe hook: clock64 timeline of CTA 0 (tools/umma_probe.py)
   int32_t dbg_flags;               // probe hook: 1 skip epilogue body, 2 skip residual, 4 skip MMAs, 8 skip A loads
   int32_t dbg_shift_rows, dbg_base_offset_mode;   // experiment hook: A operand read at a row offset (tik_debug_set_umma_shift)
@@ -97,15 +95,8 @@ __device__ __forceinline__ float apply_act(float v, int act, float slope) {
 #define TIK_PROBE_ONLY(x) false
 #endif
 
-// CL = CTAs per cluster.  CL = 2 (rowgemm_umma_mc_kernel, BN = 256 with streamed weights): the two CTAs of a cluster work
-// on two row tiles of the SAME column tile in lock step and share one weight stream -- each loads half of every W chunk
-// and TMA-multicasts it into both CTAs' ring slots, so the L2 -> SM weight traffic halves (the 256-channel temporal convs and
-// the first head layer re-stream 0.5-2.2 MB of weights per tile: 3.0 GB in 268 us for the b6 temporal conv = 11 TB/s).
-// Opt-in experiment (TIK_MC=1): it turned out NOT to be the limiter, see umma_prepare.  A ring slot is free when BOTH CTAs'
-// MMAs have read it: tcgen05.commit multicasts its
-// arrival to both empty barriers (count CL).  An odd last row tile is computed (and stored, identically) by both CTAs.
-template <int BN, int ACT, int CL>
-__device__ __forceinline__ void rowgemm_umma_body(const UmmaParams& p) {
+template <int BN, int ACT>
+__global__ void __launch_bounds__(kUmmaThreads, 1) rowgemm_umma_kernel(const __grid_constant__ UmmaParams p) {
   constexpr int kBBytes = BN * kChunkK * 2;
   if (threadIdx.x == 0) TIK_T(0);
   extern __shared__ uint8_t smem_raw[];
@@ -127,19 +118,9 @@ __device__ __forceinline__ void rowgemm_umma_body(const UmmaParams& p) {
   const int stages = p.stages;
   const int chunk_bytes = kABytes + (p.w_resident ? 0 : kBBytes);
   const int stage_bytes = p.group * chunk_bytes;
-  const int64_t num_tiles = p.tiles_m * p.n_tiles_n;
-  // work items: tiles (CL = 1), or groups of CL row tiles of one column tile, one per CTA of the cluster
-  const int cl_rank = CL > 1 ? (int)cluster_ctarank() : 0;
-  const int g0 = CL > 1 ? (int)blockIdx.x / CL : (int)blockIdx.x, gstep = CL > 1 ? (int)gridDim.x / CL : (int)gridDim.x;
-  const int n_items = CL > 1 ? (int)(((p.tiles_m + CL - 1) / CL) * p.n_tiles_n) : (int)num_tiles;
-  auto tile_of = [&](int g) -> int {
-    if (CL == 1) return p.rev ? (int)num_tiles - 1 - g : g;
-    const int tn = g % p.n_tiles_n;
-    int64_t tm = (int64_t)(g / p.n_tiles_n) * CL + cl_rank;
-    if (tm >= p.tiles_m) tm = p.tiles_m - 1;              // odd tail: the same tile twice (identical stores)
-    return (int)(tm * p.n_tiles_n + tn);
-  };
-  constexpr uint16_t kClMask = (uint16_t)((1u << CL) - 1u);
+  const int num_tiles = (int)(p.tiles_m * p.n_tiles_n);
+  const int g0 = (int)blockIdx.x, gstep = (int)gridDim.x;
+  auto tile_of = [&](int g) -> int { return p.rev ? num_tiles - 1 - g : g; };
 
   if (warp == 0 && lane == 0) {
     for (int s = 0; s < p.n_slabs; ++s) tma_prefetch_desc(&p.map_a[s]);
@@ -147,7 +128,7 @@ __device__ __forceinline__ void rowgemm_umma_body(const UmmaParams& p) {
     if (p.tma_store) tma_prefetch_desc(&p.map_out);
   }
   if (warp == 1 && lane == 0) {
-    for (int i = 0; i < stages; ++i) { mbar_init(&full_bar[i], 1); mbar_init(&empty_bar[i], CL); }
+    for (int i = 0; i < stages; ++i) { mbar_init(&full_bar[i], 1); mbar_init(&empty_bar[i], 1); }
     for (int i = 0; i < 2; ++i) { mbar_init(&tmem_full[i], 1); mbar_init(&tmem_empty[i], kEpiWarps); }
     mbar_init(w_full, 1);
     for (int i = 0; i < 2; ++i) { mbar_init(&stage_full[i], kEpiWarps); mbar_init(&stage_empty[i], 1); }
@@ -159,7 +140,6 @@ __device__ __forceinline__ void rowgemm_umma_body(const UmmaParams& p) {
   tc_fence_before();
   __syncthreads();
   tc_fence_after();
-  if (CL > 1) cluster_sync_all();                           // the peer's barriers are initialised before anyone signals them
   const uint32_t tmem_base = *tmem_slot;
   pdl_launch_dependents();                                  // the next kernel may begin its own prologue
   pdl_wait();                                               // everything below reads what the previous kernel wrote
@@ -177,9 +157,8 @@ __device__ __forceinline__ void rowgemm_umma_body(const UmmaParams& p) {
     const uint32_t tx_bytes = (uint32_t)(p.a_box_bytes + (p.w_resident ? 0 : kBBytes));
     const bool skip_a = (p.dbg_flags & 8) != 0;
     const int group = p.group, total_chunks = p.total_chunks;
-    const uint64_t pol = p.l2 ? l2_policy_evict_first() : 0;
     int stage = 0; uint32_t phase = 0;
-    for (int g = g0; g < n_items; g += gstep) {
+    for (int g = g0; g < num_tiles; g += gstep) {
       const int tile = tile_of(g);
       const int tm = tile / p.n_tiles_n;
       const int n0 = (tile - tm * p.n_tiles_n) * BN;
@@ -204,11 +183,8 @@ __device__ __forceinline__ void rowgemm_umma_body(const UmmaParams& p) {
           if (p3) TIK_T(26);
           uint8_t* sa = ring + (size_t)stage * stage_bytes + (size_t)j * chunk_bytes;
           if (leader) {
-            if (!skip_a) tma_load_3d(sa, &p.map_a[s], &full_bar[stage], c * kChunkK, ts, nv0, pol);
-            if (!p.w_resident) {
-              if (CL > 1) tma_load_2d_mc(sa + kABytes + cl_rank * (kBBytes / CL), &p.map_w, &full_bar[stage], kw * kChunkK, n0 + cl_rank * (BN / CL), kClMask);
-              else tma_load_2d(sa + kABytes, &p.map_w, &full_bar[stage], kw * kChunkK, n0);
-            }
+            if (!skip_a) tma_load_3d(sa, &p.map_a[s], &full_bar[stage], c * kChunkK, ts, nv0);
+            if (!p.w_resident) tma_load_2d(sa + kABytes, &p.map_w, &full_bar[stage], kw * kChunkK, n0);
           }
           if (p3) TIK_T(27);
           __syncwarp();
@@ -234,7 +210,7 @@ __device__ __forceinline__ void rowgemm_umma_body(const UmmaParams& p) {
     int stage = 0; uint32_t phase = 0;
     int acc = 0; uint32_t acc_phase = 0;
     const int total_chunks = p.total_chunks, group = p.group;
-    for (int g = g0; g < n_items; g += gstep) {
+    for (int g = g0; g < num_tiles; g += gstep) {
       const int tile = tile_of(g);
       const bool m3 = TIK_PROBE_ONLY(leader && tile == (int)blockIdx.x + 3 * (int)gridDim.x);
       if (m3) TIK_T(16);
@@ -269,7 +245,7 @@ __device__ __forceinline__ void rowgemm_umma_body(const UmmaParams& p) {
         }
         if (leader) {
           if (m3 && kc < 2 * group) TIK_T(19 + 3 * (kc / group));
-          if (CL > 1) umma_commit_mc(&empty_bar[stage], kClMask); else umma_commit(&empty_bar[stage]);   // frees this ring slot (in every CTA of the cluster) once the MMAs have read it
+          umma_commit(&empty_bar[stage]);                  // frees this ring slot once the MMAs have read it
           if (m3 && kc < 2 * group) TIK_T(20 + 3 * (kc / group));
         }
         __syncwarp();
@@ -290,7 +266,7 @@ __device__ __forceinline__ void rowgemm_umma_body(const UmmaParams& p) {
       const int ntn = p.n_tiles_n, tiles_t = p.tiles_t;
       int sbuf = 0; uint32_t sphase = 0;
       int prev = -1;
-      for (int g = g0; g < n_items; g += gstep) {
+      for (int g = g0; g < num_tiles; g += gstep) {
       const int tile = tile_of(g);
         const int tm = tile / ntn;
         const int n0 = (tile - tm * ntn) * BN;
@@ -324,7 +300,7 @@ __device__ __forceinline__ void rowgemm_umma_body(const UmmaParams& p) {
     const int ntn = p.n_tiles_n, tiles_t = p.tiles_t;
     int acc = 0; uint32_t acc_phase = 0;
     int sbuf = 0; uint32_t sphase = 0;
-    for (int g = g0; g < n_items; g += gstep) {
+    for (int g = g0; g < num_tiles; g += gstep) {
       const int tile = tile_of(g);
       const int tm = tile / ntn;
       const int n0 = (tile - tm * ntn) * BN;
@@ -430,274 +406,6 @@ __device__ __forceinline__ void rowgemm_umma_body(const UmmaParams& p) {
     tmem_dealloc<2 * BN>(tmem_base);
   }
   if (threadIdx.x == 64) TIK_T(10);
-  if (CL > 1) cluster_sync_all();                           // no CTA leaves while its peer may still multicast into its ring / signal its barriers
-}
-
-template <int BN, int ACT>
-__global__ void __launch_bounds__(kUmmaThreads, 1) rowgemm_umma_kernel(const __grid_constant__ UmmaParams p) {
-  rowgemm_umma_body<BN, ACT, 1>(p);
-}
-template <int ACT>
-__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kUmmaThreads, 1) rowgemm_umma_mc_kernel(const __grid_constant__ UmmaParams p) {
-  rowgemm_umma_body<256, ACT, 2>(p);
-}
-
-// ------------------------------------------------------------------------------------------------ CTA-pair variant (cta_group::2)
-// The 256-channel layers (K up to 896, weights 448 KB) can keep their weights neither beside the ring nor in tensor
-// memory: every 128-row tile streams all of W from L2 again, and each MMA reads a 128 x 16 A slice plus a 256 x 16 B
-// slice (12 KB) from shared memory.  Here two CTAs of a cluster work on two row tiles with ONE weight stream: each CTA
-// loads its own A chunk and HALF of the W chunk (128 of the 256 output channels), and the leader CTA issues
-// tcgen05.mma.cta_group::2 with M = 256 -- the tensor cores of both SMs read their own A tile and both B halves, so a
-// CTA moves 16 + 16 KB per chunk through its ring instead of 16 + 32 and reads 8 KB instead of 12 per MMA.
-// Barriers: the ring's "full" barrier lives in the leader and counts the bytes of all four TMA loads of a stage
-// (cta_group::2 loads may signal the peer's barrier); "empty" and "accumulator full" are committed to both CTAs
-// (multicast commit); the peer's epilogue warps arrive remotely on the leader's "accumulator empty".
-// STATUS: experiment (TIK_2CTA=1).  Results match the one-CTA kernel; a cross-CTA hand-off costs about twice a local
-// one, and with the two K chunks per stage that fit beside the staging tile it is still 0-25 % slower.
-template <int ACT>
-__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kUmmaThreads, 1) rowgemm_umma2_kernel(const __grid_constant__ UmmaParams p) {
-  constexpr int BN = 256;
-  constexpr int kBHalf = (BN / 2) * kChunkK * 2;            // this CTA's half of a W chunk: 16 KB
-  extern __shared__ uint8_t smem_raw[];
-  uint8_t* smem = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);   // 1024-aligned; pointer arithmetic on the shared base keeps the address space (LDS / STS, not generic LD / ST)
-  uint8_t* ring = smem + p.off_ring;
-  float* s_bias = reinterpret_cast<float*>(smem + p.off_bias);
-  uint8_t* s_stage = smem + p.off_stage;
-  uint64_t* full_bar = reinterpret_cast<uint64_t*>(smem + p.off_bar);
-  uint64_t* empty_bar = full_bar + kMaxStages;
-  uint64_t* tmem_full = empty_bar + kMaxStages;             // [2]
-  uint64_t* tmem_empty = tmem_full + 2;                     // [2]
-  uint64_t* w_full = tmem_empty + 2;                        // unused
-  uint64_t* stage_full = w_full + 1;                        // [2]
-  uint64_t* stage_empty = stage_full + 2;                   // [2]
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(stage_empty + 2);
-
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const uint32_t rank = cluster_ctarank();
-  const int cluster_id = (int)blockIdx.x >> 1, n_clusters = (int)gridDim.x >> 1;
-  const int stages = p.stages;
-  const int group = p.group;                                // K chunks per ring stage (one cross-CTA hand-off per stage)
-  const int chunk_bytes = kABytes + kBHalf;
-  const int stage_bytes = group * chunk_bytes;
-  const int ntn = p.n_tiles_n;
-  const int pairs_m = (int)((p.tiles_m + 1) / 2);
-  const int n_pairs = pairs_m * ntn;
-
-  if (warp == 0 && lane == 0) {
-    for (int s = 0; s < p.n_slabs; ++s) tma_prefetch_desc(&p.map_a[s]);
-    tma_prefetch_desc(&p.map_w);
-    if (p.tma_store) tma_prefetch_desc(&p.map_out);
-  }
-  if (warp == 1 && lane == 0) {
-    for (int i = 0; i < stages; ++i) { mbar_init(&full_bar[i], 2); mbar_init(&empty_bar[i], 1); }
-    for (int i = 0; i < 2; ++i) { mbar_init(&tmem_full[i], 1); mbar_init(&tmem_empty[i], 2 * kEpiWarps); }
-    for (int i = 0; i < 2; ++i) { mbar_init(&stage_full[i], kEpiWarps); mbar_init(&stage_empty[i], 1); }
-    fence_barrier_init();
-  }
-  if (warp == 2) tmem_alloc_2sm<512>(tmem_slot);
-  for (int i = threadIdx.x; i < p.bias_rows * p.c_out; i += kUmmaThreads) s_bias[(i / p.c_out) * (p.c_out + 4) + (i % p.c_out)] = __ldg(p.bias + i);
-  tc_fence_before();
-  __syncthreads();
-  cluster_sync_all();                                       // the peer's barriers are initialised before anyone signals them
-  tc_fence_after();
-  const uint32_t tmem_base = *tmem_slot;
-
-  // pair index -> (row tile of this CTA, output-channel tile)
-  auto tile_of = [&](int pr, int& tm, int& n0) {
-    const int q = pr / ntn;
-    n0 = (pr - q * ntn) * BN;
-    tm = 2 * q + (int)rank;
-  };
-
-  if (warp == 0) {
-    // ===================== TMA producer (both CTAs): own A chunk + own half of the W chunk =====================
-    if (lane == 0) {
-      const uint32_t tx_pair = 2u * (uint32_t)(p.a_box_bytes + kBHalf);
-      const int total_chunks = p.total_chunks;
-      int stage = 0; uint32_t phase = 0;
-      for (int pr = cluster_id; pr < n_pairs; pr += n_clusters) {
-        int tm, n0;
-        tile_of(pr, tm, n0);
-        const int tile_nv = tm / p.tiles_t;
-        const int t0 = (tm - tile_nv * p.tiles_t) * p.tt;
-        const int nv0 = tile_nv * p.vv;
-        int kw = 0, j = 0;
-        uint32_t full_leader = 0;
-        for (int s = 0; s < p.n_slabs; ++s) {
-          const int ts = t0 * p.t_mul[s] + p.t_off[s];
-          for (int c = 0; c < p.chunks[s]; ++c, ++kw) {
-            if (j == 0) {
-              mbar_wait(&empty_bar[stage], phase ^ 1);
-              full_leader = mapa_u32(smem_u32(&full_bar[stage]), 0);
-              const int in_stage = min(group, total_chunks - kw);
-              if (rank == 0) mbar_expect_tx(&full_bar[stage], tx_pair * (uint32_t)in_stage);
-              else mbar_arrive_cluster(full_leader);
-            }
-            uint8_t* sa = ring + (size_t)stage * stage_bytes + (size_t)j * chunk_bytes;
-            tma_load_3d_2sm(sa, &p.map_a[s], full_leader, c * kChunkK, ts, nv0);
-            tma_load_2d_2sm(sa + kABytes, &p.map_w, full_leader, kw * kChunkK, n0 + (int)rank * (BN / 2));
-            if (++j == group || kw + 1 == total_chunks) {
-              j = 0;
-              if (++stage == stages) { stage = 0; phase ^= 1; }
-            }
-          }
-        }
-      }
-    }
-  } else if (warp == 1) {
-    // ===================== MMA issuer: leader CTA only =====================
-    if (rank == 0) {
-      constexpr uint32_t idesc = make_idesc_bf16(256, BN);
-      const bool leader = lane == 0;
-      const uint32_t ring_u32 = smem_u32(ring);
-      const uint64_t desc_hi = make_smem_desc_kmajor_sw128(0);
-      int stage = 0; uint32_t phase = 0;
-      int acc = 0; uint32_t acc_phase = 0;
-      const int total_chunks = p.total_chunks;
-      for (int pr = cluster_id; pr < n_pairs; pr += n_clusters) {
-        mbar_wait(&tmem_empty[acc], acc_phase ^ 1);          // both CTAs' epilogues have drained this accumulator
-        tc_fence_after();
-        const uint32_t tmem_d = tmem_base + (uint32_t)(acc * BN);
-        for (int kc = 0; kc < total_chunks; kc += group) {
-          mbar_wait(&full_bar[stage], phase);
-          tc_fence_after();
-          const int in_stage = min(group, total_chunks - kc);
-          for (int j = 0; j < in_stage; ++j) {
-            const uint32_t sa = ring_u32 + (uint32_t)stage * (uint32_t)stage_bytes + (uint32_t)j * (uint32_t)chunk_bytes;
-            const uint64_t da = desc_hi | (uint64_t)((sa >> 4) & 0x3FFF);
-            const uint64_t db = desc_hi | (uint64_t)(((sa + kABytes) >> 4) & 0x3FFF);
-            if (leader) {
-#pragma unroll
-              for (int k = 0; k < kChunkK / 16; ++k)
-                umma_bf16_2sm(tmem_d, da + (uint64_t)(2 * k), db + (uint64_t)(2 * k), idesc, (kc | j | k) != 0 ? 1u : 0u);
-            }
-          }
-          if (leader) umma_commit_2sm(&empty_bar[stage]);    // frees this ring stage in both CTAs
-          __syncwarp();
-          if (++stage == stages) { stage = 0; phase ^= 1; }
-        }
-        if (leader) umma_commit_2sm(&tmem_full[acc]);        // accumulator complete -> both epilogues
-        __syncwarp();
-        if (++acc == 2) { acc = 0; acc_phase ^= 1; }
-      }
-    }
-  } else if (warp == 2 + kEpiWarps) {
-    // ===================== TMA-store warp =====================
-    if (lane == 0 && p.tma_store) {
-      int sbuf = 0; uint32_t sphase = 0;
-      int prev = -1;
-      for (int pr = cluster_id; pr < n_pairs; pr += n_clusters) {
-        int tm, n0;
-        tile_of(pr, tm, n0);
-        const int tile_nv = tm / p.tiles_t, tile_t = tm - tile_nv * p.tiles_t;
-        mbar_wait(&stage_full[sbuf], sphase);
-        for (int c = 0; c < BN / 64; ++c)
-          tma_store_3d(&p.map_out, s_stage + ((size_t)sbuf * (BN / 64) + c) * kABytes, n0 + c * 64, tile_t * p.tt, tile_nv * p.vv);
-        tma_store_commit();
-        if (p.stage_bufs == 2) {
-          tma_store_wait_read1();
-          if (prev >= 0) mbar_arrive(&stage_empty[prev]);
-          prev = sbuf;
-          if (++sbuf == 2) { sbuf = 0; sphase ^= 1; }
-        } else {
-          tma_store_wait_read0();
-          mbar_arrive(&stage_empty[0]);
-          sphase ^= 1;
-        }
-      }
-      tma_store_wait0();
-    }
-  } else {
-    // ===================== epilogue (both CTAs, each its own 128 rows): as rowgemm_umma_kernel =====================
-    constexpr int CW = BN / 4;
-    const int lane_grp = warp & 3;
-    const int cq = (warp - 2) >> 2;
-    const int r = lane_grp * 32 + lane;
-    const int nv_l = r / p.tt, t_l = r - nv_l * p.tt;
-    int acc = 0; uint32_t acc_phase = 0;
-    int sbuf = 0; uint32_t sphase = 0;
-    for (int pr = cluster_id; pr < n_pairs; pr += n_clusters) {
-      int tm, n0;
-      tile_of(pr, tm, n0);
-      const int tile_nv = tm / p.tiles_t, tile_t = tm - tile_nv * p.tiles_t;
-      const int t = tile_t * p.tt + t_l;
-      const int nv = tile_nv * p.vv + nv_l;
-      const bool valid = (nv_l < p.vv) && (nv < (int)p.nv) && (t < p.t_out) && (tm < (int)p.tiles_m);
-      const int n = nv / p.v, node = nv - n * p.v;
-      const int64_t row = (int64_t)nv * p.t_out + t;
-      const int cb = cq * CW;
-      const float* bias = s_bias + (p.bias_per_node ? (valid ? node : 0) * (p.c_out + 4) : 0) + n0 + cb;
-      int64_t out_off;
-      if (p.out_layout == TIK_OUT_NODE_MAJOR) out_off = row * p.c_out + n0 + cb;
-      else if (p.out_layout == TIK_OUT_TIME_MAJOR) out_off = (((int64_t)n * p.t_out + t) * p.v + node) * (int64_t)p.c_out + n0 + cb;
-      else out_off = row * p.c_out_valid + n0 + cb;
-      uint8_t* stage_row = s_stage + (size_t)sbuf * (BN / 64) * kABytes + (size_t)r * 128;
-
-      mbar_wait(&tmem_full[acc], acc_phase);
-      tc_fence_after();
-      const uint32_t tmem_d = tmem_base + (uint32_t)(acc * BN + cb) + ((uint32_t)(lane_grp * 32) << 16);
-      uint32_t a[CW];
-#pragma unroll
-      for (int i = 0; i < CW / 16; ++i) tmem_ld16(tmem_d + (uint32_t)(16 * i), a + 16 * i);
-      tmem_ld_wait();
-      tc_fence_before();
-      __syncwarp();
-      if (lane == 0) mbar_arrive_cluster(mapa_u32(smem_u32(&tmem_empty[acc]), 0));   // the leader's barrier counts both CTAs
-      if (p.tma_store) mbar_wait(&stage_empty[sbuf], sphase ^ 1);
-      if (valid || p.tma_store) {
-#pragma unroll
-        for (int q = 0; q < CW / 8; ++q) {
-          const float4 b0 = *reinterpret_cast<const float4*>(bias + 8 * q);
-          const float4 b1 = *reinterpret_cast<const float4*>(bias + 8 * q + 4);
-          float v[8] = {__uint_as_float(a[8 * q + 0]) + b0.x, __uint_as_float(a[8 * q + 1]) + b0.y,
-                        __uint_as_float(a[8 * q + 2]) + b0.z, __uint_as_float(a[8 * q + 3]) + b0.w,
-                        __uint_as_float(a[8 * q + 4]) + b1.x, __uint_as_float(a[8 * q + 5]) + b1.y,
-                        __uint_as_float(a[8 * q + 6]) + b1.z, __uint_as_float(a[8 * q + 7]) + b1.w};
-          if (ACT == TIK_ACT_LEAKY) {
-#pragma unroll
-            for (int e = 0; e < 8; ++e) v[e] = v[e] > 0.f ? v[e] : v[e] * p.slope;
-          }
-          if (p.out_layout == TIK_OUT_ROWS_F32) {
-            float* o = reinterpret_cast<float*>(p.out) + out_off + 8 * q;
-#pragma unroll
-            for (int e = 0; e < 8; ++e)
-              if (valid && n0 + cb + 8 * q + e < p.c_out_valid) o[e] = (ACT == TIK_ACT_RELU) ? fmaxf(v[e], 0.f) : v[e];
-          } else {
-            uint4 u;
-            if (ACT == TIK_ACT_RELU) {
-              u.x = pack_bf16x2_relu(v[0], v[1]); u.y = pack_bf16x2_relu(v[2], v[3]);
-              u.z = pack_bf16x2_relu(v[4], v[5]); u.w = pack_bf16x2_relu(v[6], v[7]);
-            } else {
-              u.x = pack_bf16x2(v[0], v[1]); u.y = pack_bf16x2(v[2], v[3]);
-              u.z = pack_bf16x2(v[4], v[5]); u.w = pack_bf16x2(v[6], v[7]);
-            }
-            if (p.tma_store) {
-              const int col = cb + 8 * q;
-              const int j = (col & 63) >> 3;
-              *reinterpret_cast<uint4*>(stage_row + (size_t)(col >> 6) * kABytes + ((j ^ (r & 7)) << 4)) = u;
-            } else if (valid) {
-              *reinterpret_cast<uint4*>(reinterpret_cast<__nv_bfloat16*>(p.out) + out_off + 8 * q) = u;
-            }
-          }
-        }
-      }
-      if (p.tma_store) {
-        fence_proxy_async_smem();
-        __syncwarp();
-        if (lane == 0) mbar_arrive(&stage_full[sbuf]);
-        if (p.stage_bufs == 2) { if (++sbuf == 2) { sbuf = 0; sphase ^= 1; } } else { sphase ^= 1; }
-      }
-      if (++acc == 2) { acc = 0; acc_phase ^= 1; }
-    }
-  }
-  __syncwarp();
-  tc_fence_before();
-  __syncthreads();
-  cluster_sync_all();                                       // no CTA leaves while its peer may still signal its barriers / read its smem
-  if (warp == 2) {
-    tc_fence_after();
-    tmem_dealloc_2sm<512>(tmem_base);
-  }
 }
 
 // ------------------------------------------------------------------------------------------------ weight-stationary variant
@@ -781,7 +489,6 @@ __global__ void __launch_bounds__(kUmmaThreads, 1) rowgemm_ts_kernel(const __gri
     // ===================== TMA producer: activation chunks only =====================
     const bool leader = lane == 0;
     int stage = 0; uint32_t phase = 0;
-    const uint64_t pol = p.l2 ? l2_policy_evict_first() : 0;
     for (int ti = blockIdx.x; ti < n_tiles; ti += gridDim.x) {
       const int tile = p.rev ? n_tiles - 1 - ti : ti;
       const int tile_nv = tile / p.tiles_t;
@@ -800,7 +507,7 @@ __global__ void __launch_bounds__(kUmmaThreads, 1) rowgemm_ts_kernel(const __gri
             }
           }
           if (leader && !TIK_PROBE_ONLY((p.dbg_flags & 8) != 0))
-            tma_load_3d(ring + (size_t)stage * stage_bytes + (size_t)j * kABytes, &p.map_a[s], &full_bar[stage], c * kChunkK, ts, nv0, pol);
+            tma_load_3d(ring + (size_t)stage * stage_bytes + (size_t)j * kABytes, &p.map_a[s], &full_bar[stage], c * kChunkK, ts, nv0);
           __syncwarp();
           if (++j == group || kw + 1 == total_chunks) {
             j = 0;
@@ -1031,30 +738,6 @@ static int launch_variant(const UmmaParams& p, int smem_bytes, unsigned grid, cu
   return TIK_OK;
 }
 
-// Clusters of two: the grid is sized by how many clusters the device can hold at once (a second wave would double the time
-// of a persistent kernel), queried once per device.
-template <int ACT>
-static int launch_mc(const UmmaParams& p, int smem_bytes, cudaStream_t s) {
-  static int clusters[64] = {};
-  int dev = 0;
-  TIK_CUDA(cudaGetDevice(&dev));
-  if (!clusters[dev & 63]) {
-    TIK_CUDA(cudaFuncSetAttribute(rowgemm_umma_mc_kernel<ACT>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBudget + 2048));
-    TIK_CUDA(cudaFuncSetAttribute(rowgemm_umma_mc_kernel<ACT>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3(2 * (num_sms() / 2), 1, 1);
-    cfg.blockDim = dim3(kUmmaThreads, 1, 1);
-    cfg.dynamicSmemBytes = kSmemBudget + 2048;
-    int n = 0;
-    if (cudaOccupancyMaxActiveClusters(&n, rowgemm_umma_mc_kernel<ACT>, &cfg) != cudaSuccess || n <= 0) { (void)cudaGetLastError(); n = num_sms() / 2; }
-    clusters[dev & 63] = std::min(n, num_sms() / 2);
-  }
-  const int64_t items = ((p.tiles_m + 1) / 2) * p.n_tiles_n;
-  const unsigned grid = 2u * (unsigned)std::min<int64_t>(items, clusters[dev & 63]);
-  TIK_CUDA(launch_pdl(rowgemm_umma_mc_kernel<ACT>, grid, kUmmaThreads, (size_t)smem_bytes, s, p));
-  return TIK_OK;
-}
-
 int umma_prepare(const TikRowGemm* d, int64_t nv_capacity, UmmaPrepared** out) {
   TIK_CHECK_ARG(d->c_out % 64 == 0, "bf16 path: c_out=%d must be a multiple of 64", d->c_out);
   TIK_CHECK_ARG(nv_capacity >= d->nv && nv_capacity > 0, "nv capacity");
@@ -1164,47 +847,13 @@ int umma_prepare(const TikRowGemm* d, int64_t nv_capacity, UmmaPrepared** out) {
       }
     }
   }
-  // CTA-pair kernel for the 256-column layers whose weights have to be streamed: ring stage = A chunk + half a W chunk
-  // EXPERIMENT, opt-in (TIK_2CTA=1): parity-green but slower than one CTA per tile today (b6 temporal conv 324 vs
-  // 269 us, head 98 vs 84 us with two chunks per hand-off; profiles/r1_notes.md)
-  p.two_cta = (!p.ts && u->bn == 256 && !w_res && d->res_kind == TIK_RES_NONE && getenv("TIK_2CTA")) ? 1 : 0;
-  if (p.two_cta) {
-    sbufs = 2;
-    int fit = (kSmemBudget - bar_bytes - bias_bytes - sbufs * one_stage_tile) / (kABytes + b_bytes / 2);
-    if (fit < 4) { sbufs = 1; fit = (kSmemBudget - bar_bytes - bias_bytes - one_stage_tile) / (kABytes + b_bytes / 2); }
-    group = env_g ? atoi(env_g) : 2;                      // chunks per cross-CTA hand-off
-    if (group < 1) group = 1;
-    while (group > 1 && fit / group < 2) group >>= 1;
-    stages = fit / group > kMaxStages ? kMaxStages : fit / group;
-    uint64_t dims[2] = {(uint64_t)ktot, (uint64_t)d->c_out};
-    uint64_t strides[1] = {(uint64_t)ktot * 2};
-    uint32_t box[2] = {(uint32_t)kChunkK, (uint32_t)(u->bn / 2)};
-    uint32_t estr[2] = {1, 1};
-    int rc = encode_map(&p.map_w, d->w_dev, 2, dims, strides, box, estr);
-    if (rc != TIK_OK) { delete u; return rc; }
-  }
-  // Streamed 256-column weights: clusters of two CTAs share the stream (TMA multicast), see rowgemm_umma_body.
-  // EXPERIMENT, opt-in (TIK_MC=1): parity-green, and slower on one box in an A/B (tools/ab_trace.sh): b6 temporal conv
-  // 293 vs 270 us, b7 154 -> 161, head 85 -> 90.  Halving the L2 -> SM weight traffic does not help because these
-  // launches are bound by SHARED-MEMORY bandwidth, not L2: every operand byte is written once by TMA and read once by
-  // the SS-mode MMA -- per 64-wide K chunk 48 KB in + 48 KB out against 512 tensor cycles = 188 B/clk wanted, 128 B/clk
-  // available, i.e. at most 68 % tensor-pipe activity before the epilogue's own traffic (measured: 48-61 %).
-  p.mc = (!p.ts && !p.two_cta && u->bn == 256 && !w_res && getenv("TIK_MC")) ? 1 : 0;
-  if (p.mc) {
-    uint64_t dims[2] = {(uint64_t)ktot, (uint64_t)d->c_out};
-    uint64_t strides[1] = {(uint64_t)ktot * 2};
-    uint32_t box[2] = {(uint32_t)kChunkK, (uint32_t)(u->bn / 2)};
-    uint32_t estr[2] = {1, 1};
-    int rc = encode_map(&p.map_w, d->w_dev, 2, dims, strides, box, estr);
-    if (rc != TIK_OK) { delete u; return rc; }
-  }
   p.group = group;
   p.stage_bufs = sbufs;
   const int stage_out_bytes = sbufs * one_stage_tile;
   if (stages < 2) { delete u; set_error("bf16 path: bias table too large for shared memory"); return TIK_ERR_UNSUPPORTED; }
   p.w_resident = w_res; p.stages = stages;
   p.off_ring = (w_res && !p.ts) ? w_bytes : 0;
-  p.off_stage = p.off_ring + stages * group * (kABytes + (w_res ? 0 : (p.two_cta ? b_bytes / 2 : b_bytes)));
+  p.off_stage = p.off_ring + stages * group * (kABytes + (w_res ? 0 : b_bytes));
   p.off_bias = p.off_stage + stage_out_bytes;
   p.off_bar = p.off_bias + bias_bytes;
   if (p.tma_store) {
@@ -1236,7 +885,7 @@ int umma_launch(UmmaPrepared* u, const TikRowGemm* d, cudaStream_t s) {
   p.res_kind = d->res_kind; p.res = d->res_dev; p.res_w = d->res_w_dev;
   p.res_cin = d->res_cin; p.res_t_mul = d->res_t_mul; p.res_t_in = d->res_t_in;
   p.out = d->out_dev; p.out_layout = d->out_layout;
-  p.rev = launch_opts().rev; p.l2 = launch_opts().l2;
+  p.rev = launch_opts().rev;
   if (d->nv == 0 || d->t_out == 0) return TIK_OK;
   p.tiles_m = ceil_div(d->nv, p.vv) * ceil_div(d->t_out, p.tt);
   p.tiles_t = (int)ceil_div(d->t_out, p.tt);
@@ -1249,30 +898,6 @@ int umma_launch(UmmaPrepared* u, const TikRowGemm* d, cudaStream_t s) {
     if (d->act == TIK_ACT_LEAKY) return launch_variant<BN_, TIK_ACT_LEAKY>(p, u->smem_bytes, grid, s);  \
     return launch_variant<BN_, TIK_ACT_NONE>(p, u->smem_bytes, grid, s);                              \
   } while (0)
-  if (p.two_cta) {
-    static int attr2[64] = {};
-    int dev = 0;
-    TIK_CUDA(cudaGetDevice(&dev));
-    if (!attr2[dev & 63]) {
-      TIK_CUDA(cudaFuncSetAttribute(rowgemm_umma2_kernel<TIK_ACT_RELU>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBudget + 2048));
-      TIK_CUDA(cudaFuncSetAttribute(rowgemm_umma2_kernel<TIK_ACT_LEAKY>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBudget + 2048));
-      TIK_CUDA(cudaFuncSetAttribute(rowgemm_umma2_kernel<TIK_ACT_NONE>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBudget + 2048));
-      attr2[dev & 63] = 1;
-    }
-    TIK_CHECK_ARG(d->res_kind == TIK_RES_NONE, "CTA-pair kernel: residual changed after prepare");
-    const int64_t n_pairs = ((p.tiles_m + 1) / 2) * p.n_tiles_n;
-    const unsigned grid2 = 2u * (unsigned)std::min<int64_t>(n_pairs, num_sms() / 2);
-    if (d->act == TIK_ACT_RELU) rowgemm_umma2_kernel<TIK_ACT_RELU><<<grid2, kUmmaThreads, u->smem_bytes, s>>>(p);
-    else if (d->act == TIK_ACT_LEAKY) rowgemm_umma2_kernel<TIK_ACT_LEAKY><<<grid2, kUmmaThreads, u->smem_bytes, s>>>(p);
-    else rowgemm_umma2_kernel<TIK_ACT_NONE><<<grid2, kUmmaThreads, u->smem_bytes, s>>>(p);
-    TIK_LAUNCH_CHECK();
-    return TIK_OK;
-  }
-  if (p.mc) {
-    if (d->act == TIK_ACT_RELU) return launch_mc<TIK_ACT_RELU>(p, u->smem_bytes, s);
-    if (d->act == TIK_ACT_LEAKY) return launch_mc<TIK_ACT_LEAKY>(p, u->smem_bytes, s);
-    return launch_mc<TIK_ACT_NONE>(p, u->smem_bytes, s);
-  }
   if (p.ts) {
     static int ts_attr[64] = {};
     int dev = 0;
@@ -1309,7 +934,7 @@ int rowgemm_bf16(const TikRowGemm* d, cudaStream_t s) {
   static uint64_t tick = 0;
   constexpr size_t kCap = 32;
   // tuning / A-B switches are read at prepare time: with any of them set (tools, the variant tests) nothing is cached
-  if (getenv("TIK_UMMA_GROUP") || getenv("TIK_UMMA_OPT") || getenv("TIK_UMMA_BN") || getenv("TIK_NO_TS") || getenv("TIK_2CTA") ||
+  if (getenv("TIK_UMMA_GROUP") || getenv("TIK_UMMA_OPT") || getenv("TIK_UMMA_BN") || getenv("TIK_NO_TS") ||
       getenv("TIK_NO_ROWGEMM_CACHE")) {
     UmmaPrepared* u = nullptr;
     int rc = umma_prepare(d, d->nv, &u);

@@ -50,7 +50,7 @@ struct TcnHaloParams {
   int32_t region_bytes, stage_bufs, off_stage, off_bar;
   int64_t nv;
   int32_t n_tiles;
-  int32_t rev, l2;               // LaunchOpts: tiles walked last to first; evict-first hint on the H / X loads
+  int32_t rev;                   // LaunchOpts: tiles walked last to first
 };
 
 __global__ void __launch_bounds__(kThThreads, 1) tcn_halo_kernel(const __grid_constant__ TcnHaloParams p) {
@@ -118,7 +118,6 @@ __global__ void __launch_bounds__(kThThreads, 1) tcn_halo_kernel(const __grid_co
     if (lane == 0) {
       const uint32_t box_bytes = (uint32_t)(p.G * p.R * 128);
       int stage = 0; uint32_t phase = 0;
-      const uint64_t pol = p.l2 ? l2_policy_evict_first() : 0;
       for (int ti = blockIdx.x; ti < n_tiles; ti += gridDim.x) {
         const int tile = p.rev ? n_tiles - 1 - ti : ti;
         const int nv0 = (tile / p.segs) * p.G;
@@ -126,8 +125,8 @@ __global__ void __launch_bounds__(kThThreads, 1) tcn_halo_kernel(const __grid_co
         mbar_wait(&empty_bar[stage], phase ^ 1);
         mbar_expect_tx(&full_bar[stage], box_bytes * (uint32_t)chunks);
         uint8_t* dst = ring + (size_t)stage * p.stage_bytes;
-        for (int c = 0; c < p.kc; ++c) tma_load_3d(dst + (size_t)c * p.chunk_bytes, &p.map_h, &full_bar[stage], c * 64, t0 - 1, nv0, pol);
-        for (int c = 0; c < p.kc; ++c) tma_load_3d(dst + (size_t)(p.kc + c) * p.chunk_bytes, &p.map_x, &full_bar[stage], c * 64, t0 - 1, nv0, pol);
+        for (int c = 0; c < p.kc; ++c) tma_load_3d(dst + (size_t)c * p.chunk_bytes, &p.map_h, &full_bar[stage], c * 64, t0 - 1, nv0);
+        for (int c = 0; c < p.kc; ++c) tma_load_3d(dst + (size_t)(p.kc + c) * p.chunk_bytes, &p.map_x, &full_bar[stage], c * 64, t0 - 1, nv0);
         if (++stage == p.stages) { stage = 0; phase ^= 1; }
       }
     }
@@ -362,7 +361,7 @@ int tcn_halo_launch(TcnHaloPrepared* g, int64_t nv, cudaStream_t s) {
   TcnHaloParams p = g->p;
   p.nv = nv;
   p.n_tiles = (int32_t)((nv + p.G - 1) / p.G) * p.segs;
-  p.rev = launch_opts().rev; p.l2 = launch_opts().l2;
+  p.rev = launch_opts().rev;
   static bool attr_done[64] = {};
   int dev = 0;
   TIK_CUDA(cudaGetDevice(&dev));

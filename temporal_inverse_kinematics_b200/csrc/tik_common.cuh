@@ -68,9 +68,8 @@ __device__ __forceinline__ void pdl_launch_dependents() { asm volatile("griddepc
 
 // Per-launch options the plan sets before each tensor-core launch (thread-local; read when the launch fills its
 // parameters).  rev: walk the tiles from the last to the first -- consecutive kernels alternate, so each starts on the
-// part of its input the previous kernel wrote last, which is still in L2.  l2: read-once activation loads carry an
-// evict-first hint, so that they do not push the freshly written output out of L2.
-struct LaunchOpts { int rev; int l2; };
+// part of its input the previous kernel wrote last, which is still in L2.
+struct LaunchOpts { int rev; };
 LaunchOpts& launch_opts();
 
 // fp32 implicit-GEMM arguments (stgcn_simt.cu rowgemm_f32_kernel, rowgemm_tf32.cu): TikRowGemm with the K offsets resolved

@@ -15,10 +15,9 @@ int umma_launch(UmmaPrepared* u, const TikRowGemm* d, cudaStream_t s);
 void umma_free(UmmaPrepared* u);
 struct GcnFusedPrepared;
 bool gcn_fused_supported(int cin, int cout, int V, int K);
-int gcn_fused_frames(int T);          // frames per tile = the block size of the Abd operand
-int gcn_fused_frames(int T, int cin); // same; the 256-channel kernel holds at most 5 frames per tile
+int gcn_fused_frames(int T, int cin); // frames per tile = the block size of the Abd operand
 int gcn_fused_prepare(const void* x, const void* abd, const void* w, const float* bias, void* out, int64_t n_clips, int T, int V,
-                      int cin, int cout, int relu, GcnFusedPrepared** outp, int x_row = 0, int out_row = 0);
+                      int cin, int cout, int relu, GcnFusedPrepared** outp);
 int gcn_fused_launch(GcnFusedPrepared* g, int64_t n_clips, cudaStream_t s);
 void gcn_fused_free(GcnFusedPrepared* g);
 // 128B-swizzled bf16 tiled tensor map (rank <= 5, unit element strides), defined in gcn_fused.cu

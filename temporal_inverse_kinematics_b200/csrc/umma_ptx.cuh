@@ -21,11 +21,7 @@ __device__ __forceinline__ bool mbar_try_wait(uint64_t* bar, uint32_t parity) {
   uint32_t ok;
   asm volatile(
       "{\n\t.reg .pred p;\n\t"
-#ifdef TIK_TEST_WAIT
-      "mbarrier.test_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-#else
       "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-#endif
       "selp.u32 %0, 1, 0, p;\n\t}"
       : "=r"(ok)
       : "r"(smem_u32(bar)), "r"(parity)
@@ -64,22 +60,7 @@ __device__ __forceinline__ void fence_barrier_init() { asm volatile("fence.mbarr
 __device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
 __device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
 
-// L2 eviction policy for activations that are read exactly once by a kernel (`pol` argument of the TMA loads below; 0 = no
-// hint).  With read-once loads marked evict-first, what stays in the 126 MB L2 at the end of a kernel is the tail of the
-// tensor it WROTE -- which the next kernel, walking its tiles in the opposite direction (LaunchOpts::rev), reads first.
-__device__ __forceinline__ uint64_t l2_policy_evict_first() {
-  uint64_t pol;
-  asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(pol));
-  return pol;
-}
-__device__ __forceinline__ void tma_load_3d(void* dst, const CUtensorMap* map, uint64_t* bar, int c0, int c1, int c2, uint64_t pol = 0) {
-  if (pol != 0) {
-    asm volatile(
-        "cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes.L2::cache_hint [%0], [%1, {%3, %4, %5}], [%2], %6;"
-        ::"r"(smem_u32(dst)), "l"(reinterpret_cast<uint64_t>(map)), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "r"(c2), "l"(pol)
-        : "memory");
-    return;
-  }
+__device__ __forceinline__ void tma_load_3d(void* dst, const CUtensorMap* map, uint64_t* bar, int c0, int c1, int c2) {
   asm volatile(
       "cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5}], [%2];"
       ::"r"(smem_u32(dst)), "l"(reinterpret_cast<uint64_t>(map)), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "r"(c2)
@@ -276,76 +257,6 @@ __device__ __forceinline__ void mbar_arrive(uint64_t* bar) {
 // generic-proxy writes (st.shared) -> visible to the async proxy (UMMA / TMA reads of shared memory)
 __device__ __forceinline__ void fence_proxy_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
 
-// ------------------------------------------------------------------------------------------------ CTA pairs (cta_group::2)
-__device__ __forceinline__ uint32_t cluster_ctarank() {
-  uint32_t r;
-  asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
-  return r;
-}
-__device__ __forceinline__ void cluster_sync_all() {
-  asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory");
-  asm volatile("barrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
-// shared::cluster address of `local` (a shared::cta address) in CTA `rank` of the cluster
-__device__ __forceinline__ uint32_t mapa_u32(uint32_t local, uint32_t rank) {
-  uint32_t r;
-  asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r) : "r"(local), "r"(rank));
-  return r;
-}
-__device__ __forceinline__ void mbar_arrive_cluster(uint32_t cluster_addr) {
-  asm volatile("mbarrier.arrive.release.cluster.shared::cluster.b64 _, [%0];" ::"r"(cluster_addr) : "memory");
-}
-// TMA multicast: the box lands at the same shared-memory offset in every CTA of `mask`, and the bytes are counted on the
-// barrier at the same offset in each of them
-__device__ __forceinline__ void tma_load_2d_mc(void* dst, const CUtensorMap* map, uint64_t* bar, int c0, int c1, uint16_t mask) {
-  asm volatile(
-      "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster [%0], [%1, {%3, %4}], [%2], %5;"
-      ::"r"(smem_u32(dst)), "l"(reinterpret_cast<uint64_t>(map)), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "h"(mask)
-      : "memory");
-}
-// arrive on the barrier at this offset in every CTA of `mask` once the MMAs issued so far by this thread are done
-__device__ __forceinline__ void umma_commit_mc(uint64_t* bar, uint16_t mask) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;"
-               ::"r"(smem_u32(bar)), "h"(mask) : "memory");
-}
-// TMA loads of a CTA pair: the data lands in THIS CTA's shared memory, the bytes are counted on a barrier that may
-// live in the peer (shared::cluster address)
-__device__ __forceinline__ void tma_load_3d_2sm(void* dst, const CUtensorMap* map, uint32_t bar_cluster, int c0, int c1, int c2) {
-  asm volatile(
-      "cp.async.bulk.tensor.3d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5}], [%2];"
-      ::"r"(smem_u32(dst)), "l"(reinterpret_cast<uint64_t>(map)), "r"(bar_cluster), "r"(c0), "r"(c1), "r"(c2)
-      : "memory");
-}
-__device__ __forceinline__ void tma_load_2d_2sm(void* dst, const CUtensorMap* map, uint32_t bar_cluster, int c0, int c1) {
-  asm volatile(
-      "cp.async.bulk.tensor.2d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];"
-      ::"r"(smem_u32(dst)), "l"(reinterpret_cast<uint64_t>(map)), "r"(bar_cluster), "r"(c0), "r"(c1)
-      : "memory");
-}
-template <int kCols>
-__device__ __forceinline__ void tmem_alloc_2sm(uint32_t* dst_smem) {
-  asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(dst_smem)), "r"(kCols));
-  asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::);
-}
-template <int kCols>
-__device__ __forceinline__ void tmem_dealloc_2sm(uint32_t taddr) {
-  asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(kCols));
-}
-// D (+)= A . B^T across the CTA pair: M = 256 (128 rows from each CTA's A tile), B = N/2 rows from each CTA
-__device__ __forceinline__ void umma_bf16_2sm(uint32_t tmem_d, uint64_t desc_a, uint64_t desc_b, uint32_t idesc, uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n\t}"
-      ::"r"(tmem_d), "l"(desc_a), "l"(desc_b), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
-// arrive on the barrier at the same shared-memory offset in BOTH CTAs of the pair once the MMAs issued so far are done
-__device__ __forceinline__ void umma_commit_2sm(uint64_t* bar) {
-  asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;"
-               ::"r"(smem_u32(bar)), "h"((uint16_t)3) : "memory");
-}
-
 // MN-major operand, 128-byte swizzle: 64 contiguous elements per row, 8-row groups 1024 B apart (SBO),
 // next 64-element block of the MN dimension `lbo` bytes away (LBO).
 __device__ __forceinline__ uint64_t make_smem_desc_mnmajor_sw128(uint32_t smem_addr, uint32_t lbo_bytes) {
@@ -358,14 +269,7 @@ __device__ __forceinline__ uint64_t make_smem_desc_mnmajor_sw128(uint32_t smem_a
   return d;
 }
 
-__device__ __forceinline__ void tma_load_4d(void* dst, const CUtensorMap* map, uint64_t* bar, int c0, int c1, int c2, int c3, uint64_t pol = 0) {
-  if (pol != 0) {
-    asm volatile(
-        "cp.async.bulk.tensor.4d.shared::cluster.global.mbarrier::complete_tx::bytes.L2::cache_hint [%0], [%1, {%3, %4, %5, %6}], [%2], %7;"
-        ::"r"(smem_u32(dst)), "l"(reinterpret_cast<uint64_t>(map)), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "r"(c2), "r"(c3), "l"(pol)
-        : "memory");
-    return;
-  }
+__device__ __forceinline__ void tma_load_4d(void* dst, const CUtensorMap* map, uint64_t* bar, int c0, int c1, int c2, int c3) {
   asm volatile(
       "cp.async.bulk.tensor.4d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5, %6}], [%2];"
       ::"r"(smem_u32(dst)), "l"(reinterpret_cast<uint64_t>(map)), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "r"(c2), "r"(c3)

@@ -1,7 +1,7 @@
 #!/bin/bash
 # A/B of environment switches on the SAME box: per-kernel times of one configs[2] step (TIK_PLAN_TRACE) and the
 # bench value, alternating the settings, three rounds each.
-#   tools/ab_env.sh "TIK_SERPENTINE=0 TIK_L2_HINT=0" "TIK_SERPENTINE=1 TIK_L2_HINT=1" ...
+#   tools/ab_env.sh "TIK_SERPENTINE=0" "TIK_SERPENTINE=1" ...
 mkdir -p gpurun_out
 for r in 1 2 3; do
   for setting in "$@"; do
