@@ -112,6 +112,35 @@ int tik_lbs(const TikLbsModel* model, int dtype, const float* joints_dev, const 
             int fk_J, const float* transl_dev, int64_t F, void* workspace_dev, int64_t workspace_bytes, float* verts_dev,
             float* joints_out_dev, int joints_out_J, void* stream);
 
+/* ------------------------------------------------------------------ body keypoints
+ * Replaces the keypoint half of inference.py:70-79 amass_data_to_3d_keypoints and data_amass.py:176-218
+ * (run_smpl_inference -> generate_smplx_to_coco_mappings -> gather) without skinning the mesh: one kernel per call,
+ * thread per frame, rest skeleton Jt + Jd . betas per frame, FK over the 55 SMPL-X joints, and the landmark points
+ * (smplx VertexJointSelector vertices) as pose-blended, linearly skinned vertices.  Points 0..54 are the joints,
+ * 55..55+L-1 the landmarks.  Device arrays of a model, packed once by the caller (smpl_util.*.keypoint_pack): */
+#define TIK_KP_MAX_BETAS 16
+#define TIK_KP_MAX_SELECT 64
+typedef struct TikKeypointModel {
+  int32_t n_betas;                 /* B in [0, TIK_KP_MAX_BETAS] */
+  const float* joint_template_dev; /* (55,3)   J_regressor . v_template */
+  const float* joint_dirs_dev;     /* (55,3,B) J_regressor . shapedirs[..., :B]; NULL iff B == 0 */
+  int32_t n_landmarks;             /* L in [0, TIK_LBS_MAX_LANDMARKS]: points 55 .. 55+L-1 */
+  int32_t kmax;                    /* columns of the landmark skinning table, in [1, 55] when L > 0 */
+  const float* lm_template_dev;    /* (L,3) */
+  const float* lm_dirs_dev;        /* (L,3,B); NULL iff B == 0 */
+  const float* lm_posedirs_dev;    /* (3L,486) row 3l+c, or NULL: no pose blend (rigid landmarks) */
+  const int32_t* lm_skin_idx_dev;  /* (L,kmax) joint of each skinning weight (indices outside [0,55) are ignored) */
+  const float* lm_skin_w_dev;      /* (L,kmax) that weight (padding: 0) */
+} TikKeypointModel;
+/* pose_dev (F, pose_J, 3) axis-angle, pose_J in {22, 55, 60} (row pitch; joints >= min(pose_J,55) are identity, 55..59
+ * ignored); betas_dev NULL (zero betas), (B) for every frame (betas_per_frame = 0) or (F,B) (betas_per_frame = 1);
+ * transl_dev (F,3) or NULL; select_host: n_select in [1, TIK_KP_MAX_SELECT] point indices in [0, 55+L), HOST memory
+ * (repeats allowed); out_dev (F, n_select, 3) fp32.  fp32 arithmetic; no workspace; F = 0 is a no-op; CUDA-graph
+ * capturable.  Tiles of 64 frames move by bulk copies when every per-frame array is 16-byte aligned. */
+int tik_body_keypoints(const TikKeypointModel* m, const float* pose_dev, int pose_J, const float* betas_dev,
+                       int betas_per_frame, const float* transl_dev, const int32_t* select_host, int n_select,
+                       int64_t F, float* out_dev, void* stream);
+
 /* ------------------------------------------------------------------ ST-GCN primitives
  * dtype is TIK_F32 (SIMT fp32, 1e-4 parity path) or TIK_BF16 (tcgen05 tensor cores, fp32 accumulate). */
 

@@ -4,7 +4,8 @@ Mirrors reference common/smpl_util.py:8-82.  The reference delegates to the thir
 licensed SMPL-X model files.  ``load_smplx_models`` reads ``SMPLX_{MALE,FEMALE,NEUTRAL}.npz`` when the directory holds
 them (``SmplxBodyModel``: joints and vertices, ``return_mesh=True``) and otherwise builds *synthetic* body models
 (seeded kinematic tree + rest joints + linear joint shape directions; joints only).  Joints come from the FK kernels in
-libtik.so, vertices from its linear-blend-skinning kernels (``lbs``).
+libtik.so, vertices from its linear-blend-skinning kernels (``lbs``), and keypoints (joints + face landmarks, e.g.
+COCO-17) from one kernel that never skins the mesh (``keypoints``, ``run_smpl_keypoints``).
 """
 import ctypes as C
 import os
@@ -103,6 +104,25 @@ class SyntheticBodyModel:
         if betas is None:
             return self.rest_joints
         return self.rest_joints + self.joint_shapedirs @ np.asarray(betas, dtype=np.float32)[: self.joint_shapedirs.shape[2]]
+
+    def check_keypoints(self):
+        """``ValueError`` unless the model has the face landmarks ``keypoints`` needs (skeleton='full')."""
+        if self.skeleton != "full":
+            raise ValueError("keypoints need skeleton='full' (the body skeleton has no face landmarks)")
+
+    def keypoint_pack(self, device):
+        """The model as ``tik_body_keypoints`` reads it, cached per device: the 55 joints' rest positions and shape
+        directions, the five landmarks as points skinned with weight 1 to the head and no pose blend -- the rigid
+        landmark children of the 60-joint tree.  skeleton='body' has no landmarks (``ValueError``)."""
+        self.check_keypoints()
+        key = str(device)
+        if key not in getattr(self, "_kp", {}):
+            J, L = SMPLX_NUM_JOINTS, len(SMPLX_LANDMARK_NAMES)
+            self._kp = getattr(self, "_kp", {})
+            self._kp[key] = KeypointPack(device, self.rest_joints[:J], self.joint_shapedirs[:J], self.rest_joints[J:],
+                                         self.joint_shapedirs[J:], None, np.full((L, 1), SMPLX_LANDMARK_PARENT),
+                                         np.ones((L, 1)))
+        return self._kp[key]
 
 
 def read_smplx_npz(path):
@@ -210,6 +230,141 @@ class SmplxBodyModel:
             self._packed[key] = (t.to(torch.bfloat16) if dtype == "bf16" else t, torch.from_numpy(self.skin_idx).to(device),
                                  torch.from_numpy(self.skin_w).to(device))
         return self._packed[key]
+
+    def check_keypoints(self):
+        """``ValueError`` unless every landmark id is a vertex of the model (whatever the skeleton)."""
+        if not all(0 <= i < self.V for i in self.landmark_vertex_ids):
+            raise ValueError(f"landmark_vertex_ids {self.landmark_vertex_ids} must be vertex indices below V={self.V}")
+
+    def keypoint_pack(self, device):
+        """The model as ``tik_body_keypoints`` reads it, cached per device: Jt = J_regressor . v_template, Jd =
+        J_regressor . shapedirs[..., :10] (fp64, rounded once), and the rows of ``landmark_vertex_ids``: template,
+        shape directions, posedirs and skinning table.  ``ValueError`` when a landmark id is not below V."""
+        self.check_keypoints()
+        key = str(device)
+        if key not in getattr(self, "_kp", {}):
+            ids = self.landmark_vertex_ids
+            nz = (self.skin_w[ids] != 0).sum(axis=1)
+            kmax = max(1, int(nz.max()))
+            self._kp = getattr(self, "_kp", {})
+            self._kp[key] = KeypointPack(device, self.J_regressor @ self.v_template,
+                                         np.einsum("jv,vck->jck", self.J_regressor, self.shapedirs), self.v_template[ids],
+                                         self.shapedirs[ids], self.posedirs[ids].reshape(3 * len(ids), -1),
+                                         self.skin_idx[ids, :kmax], self.skin_w[ids, :kmax])
+        return self._kp[key]
+
+
+class KeypointPack:
+    """Device arrays of one body model for ``tik_body_keypoints`` and the ``TikKeypointModel`` that points at them
+    (``.c``).  Points 0..54 are the SMPL-X joints, 55.. the landmarks."""
+
+    def __init__(self, device, jt, jd, lm_t, lm_d, lm_posedirs, skin_idx, skin_w):
+        def dev(a, dt=torch.float32):
+            return torch.from_numpy(np.ascontiguousarray(a)).to(dt).to(device)
+        self.n_betas = int(jd.shape[2])
+        if self.n_betas > L.KP_MAX_BETAS:
+            raise ValueError(f"at most {L.KP_MAX_BETAS} shape directions, got {self.n_betas}")
+        self.jt, self.jd, self.lm_t, self.lm_d = dev(jt), dev(jd), dev(lm_t), dev(lm_d)
+        self.lm_posedirs = None if lm_posedirs is None else dev(lm_posedirs)
+        self.skin_idx, self.skin_w = dev(skin_idx, torch.int32), dev(skin_w)
+        self.n_landmarks, self.kmax = int(lm_t.shape[0]), int(skin_idx.shape[1])
+        c = L.TikKeypointModel()
+        c.n_betas, c.n_landmarks, c.kmax = self.n_betas, self.n_landmarks, self.kmax
+        c.joint_template_dev, c.joint_dirs_dev = self.jt.data_ptr(), self.jd.data_ptr() if self.n_betas else None
+        c.lm_template_dev, c.lm_dirs_dev = self.lm_t.data_ptr(), self.lm_d.data_ptr() if self.n_betas else None
+        c.lm_posedirs_dev = None if self.lm_posedirs is None else self.lm_posedirs.data_ptr()
+        c.lm_skin_idx_dev, c.lm_skin_w_dev = self.skin_idx.data_ptr(), self.skin_w.data_ptr()
+        self.c = c
+
+
+def keypoint_names():
+    """Names of the points ``keypoints`` can select: the 55 SMPL-X joints, then the five face landmarks."""
+    return list(SMPLX_FULL_JOINT_NAMES) + list(SMPLX_LANDMARK_NAMES)
+
+
+def keypoint_indices(select="coco"):
+    """'coco' (the order of generate_smplx_to_coco_mappings over the 60 full-skeleton names) or a list of point names
+    -> point indices.  ``ValueError`` for an unknown name or a selection outside [1, 64] points."""
+    from .keypoints_util import generate_smplx_to_coco_mappings
+    names = keypoint_names()
+    if isinstance(select, str):
+        if select != "coco":
+            raise ValueError(f"select must be 'coco' or a list of point names, got {select!r}")
+        return generate_smplx_to_coco_mappings(names)
+    select = list(select)
+    unknown = [n for n in select if n not in names]
+    if unknown:
+        raise ValueError(f"unknown point names {unknown}")
+    if not 1 <= len(select) <= L.KP_MAX_SELECT:
+        raise ValueError(f"select 1 to {L.KP_MAX_SELECT} points, got {len(select)}")
+    return [names.index(n) for n in select]
+
+
+def _aligned(t):
+    t = t.detach().float().contiguous()
+    return t.clone() if t.data_ptr() % 16 else t
+
+
+def keypoints(pose, model, betas=None, transl=None, select="coco"):
+    """Joints and face landmarks of a full-skeleton SMPL-X forward, in one kernel and without skinning the mesh.
+    pose (F, 22 | 55 | 60, 3) axis-angle CUDA tensor (22: hands / jaw / eyes identity; 60: joints past 54 ignored);
+    betas None, up to 10 values (every frame) or a CUDA tensor (F, <= 10) (one row per frame); transl (F,3) CUDA tensor or
+    None; select 'coco' or a list of names from ``keypoint_names()``.  model: ``SmplxBodyModel`` (landmarks are its
+    pose-blended, skinned vertices) or ``SyntheticBodyModel(skeleton='full')`` (rigid children of the head).
+    Returns (F, n, 3) fp32 CUDA."""
+    if not isinstance(model, (SmplxBodyModel, SyntheticBodyModel)):
+        raise TypeError("keypoints needs a SmplxBodyModel or a SyntheticBodyModel(skeleton='full')")
+    model.check_keypoints()
+    sel = keypoint_indices(select)
+    for name, t in (("pose", pose), ("transl", transl), ("betas", betas)):
+        if torch.is_tensor(t) and not t.is_cuda or (name == "pose" and not torch.is_tensor(pose)):
+            raise RuntimeError(f"keypoints: {name} must be a CUDA tensor -- there is no CPU fallback")
+    if transl is not None and not torch.is_tensor(transl):
+        raise RuntimeError("keypoints: transl must be a CUDA tensor -- there is no CPU fallback")
+    if pose.dim() != 3 or pose.shape[1] not in (22, SMPLX_NUM_JOINTS, 60) or pose.shape[2] != 3:
+        raise ValueError(f"keypoints: pose must be (F, 22 | 55 | 60, 3), got {tuple(pose.shape)}")
+    F, dev = pose.shape[0], pose.device
+    for name, t in (("transl", transl), ("betas", betas)):
+        if torch.is_tensor(t) and t.device != dev:
+            raise ValueError(f"keypoints: {name} is on {t.device}, pose on {dev}")
+    if transl is not None and tuple(transl.shape) != (F, 3):
+        raise ValueError(f"keypoints: transl must be ({F}, 3), got {tuple(transl.shape)}")
+    pack = model.keypoint_pack(dev)
+    B = pack.n_betas
+    per_frame, b = 0, None
+    if torch.is_tensor(betas) and betas.dim() == 2:
+        if betas.shape[0] != F or betas.shape[1] > min(SMPLX_NUM_BETAS, B):
+            raise ValueError(f"keypoints: per-frame betas must be ({F}, <= {min(SMPLX_NUM_BETAS, B)}), got {tuple(betas.shape)}")
+        b = _aligned(torch.nn.functional.pad(betas.detach().float(), (0, B - betas.shape[1])))
+        per_frame = 1
+    elif betas is not None:
+        v = (betas.detach().float().cpu().numpy() if torch.is_tensor(betas) else np.asarray(betas, dtype=np.float32)).reshape(-1)
+        if v.shape[0] > min(SMPLX_NUM_BETAS, B):
+            raise ValueError(f"keypoints: at most {min(SMPLX_NUM_BETAS, B)} betas, got {v.shape[0]}")
+        b = torch.from_numpy(np.pad(v, (0, B - v.shape[0]))).to(dev)
+    pose = _aligned(pose)
+    if transl is not None:
+        transl = _aligned(transl)
+    out = torch.empty((F, len(sel), 3), dtype=torch.float32, device=dev)
+    sel_c = (C.c_int32 * len(sel))(*sel)
+    with L.on_device(pose):
+        L.check(L.lib().tik_body_keypoints(C.byref(pack.c), L.ptr(pose), pose.shape[1], L.ptr(b), per_frame, L.ptr(transl),
+                                           sel_c, len(sel), F, L.ptr(out), L.stream_ptr(dev)))
+    return out
+
+
+def run_smpl_keypoints(data, smplx_models, device, apply_trans=True, apply_root_rot=True, apply_shape=True):
+    """COCO-17 keypoints (F, 17, 3) numpy of the same ``data`` dict and flags as ``run_smpl_inference``: equal to
+    ``smplx_joints_to_coco(run_smpl_inference(...))`` on a full-skeleton model, from one ``keypoints`` launch (the body of
+    the reference's amass_data_to_3d_keypoints, inference.py:70-79).  Works for every ``SmplxBodyModel`` and for
+    synthetic full-skeleton models."""
+    model = smplx_models[str(data["gender"])]
+    poses = torch.as_tensor(full_pose_from_amass(data["poses"], SMPLX_NUM_JOINTS)).to(device)
+    if not apply_root_rot:
+        poses[:, 0] = 0
+    transl = torch.as_tensor(np.asarray(data["trans"], dtype=np.float32)).to(device) if apply_trans else None
+    betas = np.asarray(data["betas"])[:SMPLX_NUM_BETAS] if apply_shape else None
+    return keypoints(poses, model, betas, transl, "coco").cpu().numpy()
 
 
 def load_smplx_models(smplx_dir, device, batch_size, skeleton="body"):
