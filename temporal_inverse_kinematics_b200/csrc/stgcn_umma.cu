@@ -850,7 +850,13 @@ int umma_prepare(const TikRowGemm* d, int64_t nv_capacity, UmmaPrepared** out) {
   p.group = group;
   p.stage_bufs = sbufs;
   const int stage_out_bytes = sbufs * one_stage_tile;
-  if (stages < 2) { delete u; set_error("bf16 path: bias table too large for shared memory"); return TIK_ERR_UNSUPPORTED; }
+  if (stages < 2) {
+    delete u;
+    if (env_o || env_g) set_error("bf16 path: no shared-memory plan with TIK_UMMA_OPT=%s TIK_UMMA_GROUP=%s fits this GEMM (c_out=%d, %d K chunks)",
+                                  env_o ? env_o : "-", env_g ? env_g : "-", d->c_out, p.total_chunks);
+    else set_error("bf16 path: bias table too large for shared memory");
+    return TIK_ERR_UNSUPPORTED;
+  }
   p.w_resident = w_res; p.stages = stages;
   p.off_ring = (w_res && !p.ts) ? w_bytes : 0;
   p.off_stage = p.off_ring + stages * group * (kABytes + (w_res ? 0 : b_bytes));
@@ -933,6 +939,8 @@ int rowgemm_bf16(const TikRowGemm* d, cudaStream_t s) {
   static std::vector<Entry> cache;
   static uint64_t tick = 0;
   constexpr size_t kCap = 32;
+  // no rows: a no-op, as on the fp32 path (umma_prepare would reject the empty tensor maps)
+  if (d->nv == 0) return TIK_OK;
   // tuning / A-B switches are read at prepare time: with any of them set (tools, the variant tests) nothing is cached
   if (getenv("TIK_UMMA_GROUP") || getenv("TIK_UMMA_OPT") || getenv("TIK_UMMA_BN") || getenv("TIK_NO_TS") ||
       getenv("TIK_NO_ROWGEMM_CACHE")) {

@@ -6,32 +6,10 @@ import os
 import pytest
 import torch
 
+from rowgemm_reference import reference
+
 pytestmark = pytest.mark.gpu
 V = 17
-
-
-def _reference(slabs, w, bias, nv, t_out, act, slope, residual):
-    acc = torch.zeros(nv, t_out, w.shape[0], dtype=torch.float64)
-    koff = 0
-    for a, t_mul, t_off in slabs:
-        t_in, c = a.shape[1], a.shape[2]
-        ts = torch.arange(t_out) * t_mul + t_off
-        ok = (ts >= 0) & (ts < t_in)
-        rows = torch.zeros(nv, t_out, c, dtype=torch.float64)
-        rows[:, ok] = a.double()[:, ts[ok]]
-        acc += rows @ w.double()[:, koff:koff + c].t()
-        koff += c
-    if bias.shape[0] > 1:
-        acc += bias.double()[torch.arange(nv) % V][:, None, :]
-    else:
-        acc += bias.double()[0]
-    if residual is not None:
-        acc += residual.double()
-    if act == "relu":
-        acc = acc.clamp_min(0)
-    elif act == "leaky":
-        acc = torch.where(acc > 0, acc, acc * slope)
-    return acc
 
 
 CASES = [
@@ -55,10 +33,8 @@ def test_tf32_rowgemm_matches_fp64(case):
     w = torch.randn(c_out, ktot, generator=g) / ktot ** 0.5
     bias = torch.randn(V if per_node else 1, c_out, generator=g)
     res = torch.randn(nv, t_out, c_out, generator=g) if with_res else None
-    want = _reference(slabs, w, bias, nv, t_out, act, 0.01, res)
+    want = reference(slabs, w, bias, nv, V, t_out, act, 0.01, res, out_layout=layout)
     shape = (nv, t_out, c_out) if layout == "node" else (n, t_out, V, c_out)
-    if layout == "time":
-        want = want.view(n, V, t_out, c_out).permute(0, 2, 1, 3)
     outs = {}
     for mode in ("tf32", "simt"):
         os.environ.pop("TIK_NO_TF32", None)
@@ -91,7 +67,7 @@ def test_tf32_head_output_rows_f32():
     out = guard[1:-1]
     ops.rowgemm([(a.cuda(), 1, 0)], w.cuda(), b.cuda(), 1, 1, rows, out_layout="rows_f32", c_out_valid=66, out=out)
     torch.cuda.synchronize()
-    want = a[0].double() @ w.double().t() + b.double()
+    want = reference([(a, 1, 0)], w, b, 1, 1, rows, out_layout="rows_f32", c_out_valid=66)
     assert bool((guard[0] == 777.0).all()) and bool((guard[-1] == 777.0).all())
     assert float((out.cpu().double() - want).abs().max() / want.abs().max()) < 2e-6
 
@@ -106,7 +82,7 @@ def test_tf32_long_k_accumulation_does_not_drift():
     w = torch.randn(n, k, device="cuda", generator=g).abs() / k
     b = torch.zeros(1, n, device="cuda")
     out = ops.rowgemm([(a, 1, 0)], w, b, 1, 1, rows)
-    want = a[0].double() @ w.double().t()
+    want = reference([(a, 1, 0)], w, b, 1, 1, rows)[0]
     assert float(((out[0].double() - want).abs() / want.abs()).max()) < 2e-6
 
 
@@ -136,22 +112,7 @@ def test_tf32_rowgemm_random_shapes():
         bias = torch.randn(v if per_node else 1, c_out, generator=g)
         res = torch.randn(nv, t_out, c_out, generator=g) if rnd.random() < 0.5 else None
         act = rnd.choice(["none", "relu", "leaky"])
-        acc = torch.zeros(nv, t_out, c_out, dtype=torch.float64)
-        koff = 0
-        for a, m, o in slabs:
-            ts = torch.arange(t_out) * m + o
-            ok = (ts >= 0) & (ts < a.shape[1])
-            rows = torch.zeros(nv, t_out, a.shape[2], dtype=torch.float64)
-            rows[:, ok] = a.double()[:, ts[ok]]
-            acc += rows @ w.double()[:, koff:koff + a.shape[2]].t()
-            koff += a.shape[2]
-        acc += bias.double()[torch.arange(nv) % v][:, None, :] if per_node else bias.double()[0]
-        if res is not None:
-            acc += res.double()
-        if act == "relu":
-            acc = acc.clamp_min(0)
-        elif act == "leaky":
-            acc = torch.where(acc > 0, acc, acc * 0.01)
+        acc = reference(slabs, w, bias, nv, v, t_out, act, 0.01, res)
         guard = torch.full((nv + 2, t_out, c_out), 4242.0, device="cuda")
         out = guard[1:-1]
         ops.rowgemm([(a.cuda(), m, o) for a, m, o in slabs], w.cuda(), bias.cuda(), nv, v, t_out, act=act, slope=0.01,
