@@ -65,6 +65,19 @@ int tik_quat_to_rotmat(const float* q_dev, float* R_dev, int64_t M, void* stream
 int tik_rotmat_to_quat(const float* R_dev, float* q_dev, int64_t M, void* stream);
 int tik_quat_to_aa(const float* q_dev, float* aa_dev, int64_t M, void* stream);
 
+/* Per-frame mean of overlapping window predictions (inference.py:56-67), for one window per frame: window w is centred
+ * on packed frame w.  preds (frames, T_out, D) -> out (frames, D), fp32.  Sequences as in TikSeqBatch: frame_start_dev
+ * (n_seqs+1) device table.  Frame j, local index i in its sequence of F_s frames, averages preds[j - o, o + h] over
+ * o = -h..h with 0 <= i - o < F_s, summed in ascending o from 0 and divided by the count (IEEE division).
+ * TIK_MEAN_EUCLIDEAN averages the D values; TIK_MEAN_ROTATION (D % 3 == 0) averages the Rodrigues matrices of each
+ * axis-angle triple, projects the mean back by Gram-Schmidt of its first two columns and returns axis-angle
+ * (tik_batch_rodrigues, tik_rot6d_to_rotmat, tik_rotmat_to_aa).  h = 0 copies preds[:, 0] in both modes.
+ * Requires 2h+1 <= T_out.  frames = 0 is a no-op.  CUDA-graph capturable. */
+#define TIK_MEAN_EUCLIDEAN 0
+#define TIK_MEAN_ROTATION 1
+int tik_window_mean(const float* preds_dev, int64_t frames, int T_out, int D, const int64_t* frame_start_dev,
+                    int64_t n_seqs, int h_w_size, int mode, float* out_dev, void* stream);
+
 /* ------------------------------------------------------------------ body forward kinematics
  * Replaces the joint output of common/smpl_util.py:22-82 run_smpl_inference -> smplx forward
  * (third-party; restated from the published SMPL chain, see oracle/fk_port.py).
@@ -330,6 +343,23 @@ int tik_stgcn_plan_run(TikPlan* plan, const float* x_dev, int64_t N, float* pose
  * model(...) of inference.py:37-52 without materialising the windows. */
 int tik_stgcn_plan_run_windows(TikPlan* plan, const float* seq_dev, const TikWindowing* win, int64_t n_windows,
                                float* poses_dev, void* feat_dev, void* stream);
+/* Ragged batch of sequences for the window mode: sequences s = 0..n_seqs-1 packed back to back in one
+ * (win->frames, V, c_in) buffer.  Sequence s holds packed frames [frame_start[s], frame_start[s+1]) and windows
+ * [window_start[s], window_start[s+1]); window n of sequence s, frame t, reads packed frame
+ * frame_start[s] + clamp(n*stride + t + offset, 0, F_s - 1), so the edge padding never reaches a neighbouring sequence.
+ * Both tables are DEVICE arrays of n_seqs+1 entries, non-decreasing, [0] = 0; frame_start[n_seqs] = win->frames,
+ * window_start[n_seqs] = n_windows.  The library cannot check them without a synchronisation: it clamps the sequence
+ * and frame indices it derives from them to the packed buffer, so a malformed table gives wrong values but no read
+ * outside it.  Windows come out in sequence order.  inference.sequence_tables builds the tables for the one-window-
+ * per-frame rule of forward_windows. */
+typedef struct TikSeqBatch {
+  int64_t n_seqs;                   /* >= 1 */
+  const int64_t* frame_start_dev;   /* (n_seqs+1) */
+  const int64_t* window_start_dev;  /* (n_seqs+1) */
+} TikSeqBatch;
+/* tik_stgcn_plan_run_windows over a ragged batch: poses (n_windows, T', head_out).  Chunks may split sequences. */
+int tik_stgcn_plan_run_seq_windows(TikPlan* plan, const float* seq_dev, const TikWindowing* win, const TikSeqBatch* seqs,
+                                   int64_t n_windows, float* poses_dev, void* feat_dev, void* stream);
 /* Measurement aid (synchronises the stream): one run with CUDA events around every kernel.
  * ms_by_kind[3] / launches_by_kind[3] = {stem, aggregate, implicit-GEMM}; flops_gemm = algorithmic
  * 2*rows*K*c_out summed over the implicit-GEMM launches. */
@@ -355,6 +385,9 @@ int tik_stgcn_latency_run(TikLatencyPlan* plan, const float* x_dev, int64_t N, f
 /* Same over sliding windows of one resident sequence (see TikWindowing / tik_stgcn_plan_run_windows). */
 int tik_stgcn_latency_run_windows(TikLatencyPlan* plan, const float* seq_dev, const TikWindowing* win, int64_t n_windows,
                                   float* poses_dev, void* stream);
+/* Same over a ragged batch of sequences (see TikSeqBatch), n_windows <= n_max. */
+int tik_stgcn_latency_run_seq_windows(TikLatencyPlan* plan, const float* seq_dev, const TikWindowing* win,
+                                      const TikSeqBatch* seqs, int64_t n_windows, float* poses_dev, void* stream);
 /* number of phases (= grid barriers + 1) of the plan */
 int tik_stgcn_latency_phases(const TikLatencyPlan* plan);
 void tik_stgcn_latency_destroy(TikLatencyPlan* plan);

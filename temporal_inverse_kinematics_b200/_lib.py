@@ -23,6 +23,7 @@ TIK_F32, TIK_BF16 = _H["TIK_F32"], _H["TIK_BF16"]
 MAX_BLOCKS, MAX_SLABS, MAX_JOINTS = _H["TIK_MAX_BLOCKS"], _H["TIK_MAX_SLABS"], _H["TIK_MAX_JOINTS"]
 LBS_MAX_LANDMARKS = _H["TIK_LBS_MAX_LANDMARKS"]
 KP_MAX_BETAS, KP_MAX_SELECT = _H["TIK_KP_MAX_BETAS"], _H["TIK_KP_MAX_SELECT"]
+MEAN_EUCLIDEAN, MEAN_ROTATION = _H["TIK_MEAN_EUCLIDEAN"], _H["TIK_MEAN_ROTATION"]
 ACT_NONE, ACT_RELU, ACT_LEAKY = 0, 1, 2
 RES_NONE, RES_IDENTITY, RES_STEM, RES_CONV = 0, 1, 2, 3
 OUT_NODE_MAJOR, OUT_TIME_MAJOR, OUT_ROWS_F32 = 0, 1, 2
@@ -44,6 +45,10 @@ class TikRowGemm(C.Structure):
 
 class TikWindowing(C.Structure):
     _fields_ = [("frames", i64), ("offset", i32), ("stride", i32), ("root_a", i32), ("root_b", i32)]
+
+
+class TikSeqBatch(C.Structure):
+    _fields_ = [("n_seqs", i64), ("frame_start_dev", vp), ("window_start_dev", vp)]
 
 
 class TikBlock(C.Structure):
@@ -96,6 +101,7 @@ _PROTOS = {
     "tik_quat_to_rotmat": (C.c_int, [vp, vp, i64, vp]),
     "tik_rotmat_to_quat": (C.c_int, [vp, vp, i64, vp]),
     "tik_quat_to_aa": (C.c_int, [vp, vp, i64, vp]),
+    "tik_window_mean": (C.c_int, [vp, i64, C.c_int, C.c_int, vp, i64, C.c_int, C.c_int, vp, vp]),
     "tik_fk_body": (C.c_int, [vp, C.c_int, C.POINTER(f32), C.POINTER(i32), C.c_int, vp, vp, vp, vp, i64, vp]),
     "tik_lbs_workspace_bytes": (C.c_int, [C.POINTER(TikLbsModel), C.c_int, i64, C.POINTER(i64)]),
     "tik_lbs": (C.c_int, [C.POINTER(TikLbsModel), C.c_int, vp, vp, vp, C.c_int, vp, i64, vp, i64, vp, vp, C.c_int, vp]),
@@ -115,6 +121,7 @@ _PROTOS = {
     "tik_stgcn_plan_create": (C.c_int, [C.POINTER(TikNet), C.c_int, i64, i64, C.c_int, vp, i64, C.POINTER(vp)]),
     "tik_stgcn_plan_run": (C.c_int, [vp, vp, i64, vp, vp, vp]),
     "tik_stgcn_plan_run_windows": (C.c_int, [vp, vp, C.POINTER(TikWindowing), i64, vp, vp, vp]),
+    "tik_stgcn_plan_run_seq_windows": (C.c_int, [vp, vp, C.POINTER(TikWindowing), C.POINTER(TikSeqBatch), i64, vp, vp, vp]),
     "tik_stgcn_plan_profile": (C.c_int, [vp, vp, i64, vp, vp, C.POINTER(C.c_double), C.POINTER(i64), C.POINTER(C.c_double)]),
     "tik_stgcn_plan_launches": (i64, [vp, i64]),
     "tik_stgcn_plan_destroy": (None, [vp]),
@@ -122,6 +129,7 @@ _PROTOS = {
     "tik_stgcn_latency_create": (C.c_int, [C.POINTER(TikNet), i64, C.c_int, vp, i64, C.POINTER(vp)]),
     "tik_stgcn_latency_run": (C.c_int, [vp, vp, i64, vp, vp]),
     "tik_stgcn_latency_run_windows": (C.c_int, [vp, vp, C.POINTER(TikWindowing), i64, vp, vp]),
+    "tik_stgcn_latency_run_seq_windows": (C.c_int, [vp, vp, C.POINTER(TikWindowing), C.POINTER(TikSeqBatch), i64, vp, vp]),
     "tik_stgcn_latency_phases": (C.c_int, [vp]),
     "tik_stgcn_latency_destroy": (None, [vp]),
     "tik_debug_latency_times": (C.c_int, [vp, vp]),

@@ -391,6 +391,75 @@ static int launch_conv(KB bulk_kernel, K kernel, const void* in, void* out, int6
   return TIK_OK;
 }
 
+// Per-frame mean of overlapping window predictions, one window per frame (inference.window_mean, reference
+// inference.py:56-67), for every sequence of a ragged batch in one launch.  One thread per output value (euclidean) or
+// per joint (rotation).  The sums run over o = -h..h in ascending order from 0 and end in one IEEE division by the
+// count: the operation order of inference._window_sum followed by acc / cnt, so the euclidean mean is bit-identical
+// to the per-sequence torch route, and the rotation mean goes through the same device functions as tik_batch_rodrigues,
+// tik_rot6d_to_rotmat and tik_rotmat_to_aa.
+template <int MODE>
+__global__ void __launch_bounds__(kConvThreads) window_mean_kernel(const float* __restrict__ preds, long long frames, int T_out,
+                                                                 int D, const int64_t* __restrict__ frame_start, long long n_seqs,
+                                                                 int h, float* __restrict__ out) {
+  const int per_frame = MODE == TIK_MEAN_ROTATION ? D / 3 : D;
+  const long long e = (long long)blockIdx.x * kConvThreads + threadIdx.x;
+  if (e >= frames * per_frame) return;
+  const long long j = e / per_frame;
+  const int d = (int)(e - j * per_frame) * (MODE == TIK_MEAN_ROTATION ? 3 : 1);
+  // sequence of frame j: the last s with frame_start[s] <= j; indices clamped to [0, frames) against malformed tables
+  long long lo = 0, hi = n_seqs - 1;
+  while (lo < hi) {
+    const long long mid = (lo + hi + 1) >> 1;
+    if (__ldg(frame_start + mid) <= j) lo = mid; else hi = mid - 1;
+  }
+  const long long f0 = min(max((long long)__ldg(frame_start + lo), 0ll), frames - 1);
+  const long long F = min(max((long long)__ldg(frame_start + lo + 1), f0 + 1), frames) - f0;
+  const long long i = j - f0;
+  float cnt = 0.f;
+  if (MODE == TIK_MEAN_EUCLIDEAN) {
+    float acc = 0.f;
+    for (int o = -h; o <= h; ++o) {
+      const long long src = i - o;
+      if (src < 0 || src >= F) continue;
+      acc += __ldg(preds + ((f0 + src) * T_out + o + h) * D + d);
+      cnt += 1.f;
+    }
+    out[j * D + d] = __fdiv_rn(acc, cnt);
+  } else {
+    float acc[9];
+#pragma unroll
+    for (int k = 0; k < 9; ++k) acc[k] = 0.f;
+    for (int o = -h; o <= h; ++o) {
+      const long long src = i - o;
+      if (src < 0 || src >= F) continue;
+      const float* p = preds + ((f0 + src) * T_out + o + h) * D + d;
+      const float a[3] = {__ldg(p), __ldg(p + 1), __ldg(p + 2)};
+      float R[9];
+      rodrigues_one(a, R);
+#pragma unroll
+      for (int k = 0; k < 9; ++k) acc[k] += R[k];
+      cnt += 1.f;
+    }
+#pragma unroll
+    for (int k = 0; k < 9; ++k) acc[k] = __fdiv_rn(acc[k], cnt);
+    const float x6[6] = {acc[0], acc[1], acc[3], acc[4], acc[6], acc[7]};   // first two columns, row by row (x6 of window_mean)
+    float R[9], aa[3];
+    rot6d_one(x6, R);
+    rotmat_to_aa_one(R, aa);
+#pragma unroll
+    for (int k = 0; k < 3; ++k) out[j * D + d + k] = aa[k];
+  }
+}
+
+// h = 0: every frame takes its own window's first prediction (preds[:, 0]) in both modes
+__global__ void __launch_bounds__(kConvThreads) window_first_kernel(const float* __restrict__ preds, long long frames, int T_out,
+                                                                  int D, float* __restrict__ out) {
+  const long long e = (long long)blockIdx.x * kConvThreads + threadIdx.x;
+  if (e >= frames * D) return;
+  const long long j = e / D;
+  out[e] = __ldg(preds + j * T_out * D + (e - j * D));
+}
+
 int launch_batch_rodrigues(const float* aa, float* R9, int64_t M, cudaStream_t s) {
   return launch_conv<3, 9>(rodrigues_bulk_kernel, rodrigues_kernel, aa, R9, M, s);
 }
@@ -418,5 +487,30 @@ int tik_quat_to_aa(const float* q, float* aa, int64_t M, void* stream) {
 }
 int tik_rotmat_to_aa(const float* R, float* aa, int64_t M, int kornia_quirk, void* stream) {
   return tik::launch_conv<9, 3>(tik::rotmat_to_aa_bulk_kernel, tik::rotmat_to_aa_kernel, R, aa, M, (cudaStream_t)stream, kornia_quirk);
+}
+int tik_window_mean(const float* preds, int64_t frames, int T_out, int D, const int64_t* frame_start, int64_t n_seqs,
+                    int h, int mode, float* out, void* stream) {
+  using namespace tik;
+  TIK_CHECK_ARG(preds && out && frame_start, "window mean: null preds, out or frame_start pointer");
+  TIK_CHECK_ARG(n_seqs >= 1, "window mean: n_seqs = %lld, need >= 1", (long long)n_seqs);
+  TIK_CHECK_ARG(frames >= 0 && T_out >= 1 && D >= 1, "window mean: bad shape frames=%lld T_out=%d D=%d", (long long)frames, T_out, D);
+  TIK_CHECK_ARG(mode == TIK_MEAN_EUCLIDEAN || mode == TIK_MEAN_ROTATION, "window mean: unknown mode %d", mode);
+  TIK_CHECK_ARG(h >= 0 && 2 * h + 1 <= T_out, "window mean: h_w_size = %d needs 2h+1 <= T_out = %d predictions per window", h, T_out);
+  TIK_CHECK_ARG(mode != TIK_MEAN_ROTATION || D % 3 == 0, "window mean: rotation mode needs D divisible by 3, got %d", D);
+  if (frames == 0) return TIK_OK;
+  const int per_frame = (mode == TIK_MEAN_ROTATION && h > 0) ? D / 3 : D;
+  const int64_t blocks = ceil_div(frames * per_frame, kConvThreads);
+  TIK_CHECK_ARG(blocks < (1ll << 31), "window mean: too many frames for one launch");
+  cudaStream_t s = (cudaStream_t)stream;
+  if (h == 0)
+    window_first_kernel<<<(unsigned)blocks, kConvThreads, 0, s>>>(preds, (long long)frames, T_out, D, out);
+  else if (mode == TIK_MEAN_EUCLIDEAN)
+    window_mean_kernel<TIK_MEAN_EUCLIDEAN><<<(unsigned)blocks, kConvThreads, 0, s>>>(preds, (long long)frames, T_out, D, frame_start,
+                                                                                     (long long)n_seqs, h, out);
+  else
+    window_mean_kernel<TIK_MEAN_ROTATION><<<(unsigned)blocks, kConvThreads, 0, s>>>(preds, (long long)frames, T_out, D, frame_start,
+                                                                                    (long long)n_seqs, h, out);
+  TIK_LAUNCH_CHECK();
+  return TIK_OK;
 }
 }

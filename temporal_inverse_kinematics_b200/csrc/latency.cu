@@ -75,6 +75,7 @@ struct LatParams {
   int64_t N;
   TikWindowing win;             // frames == 0: plain clips
   int64_t win_n0;
+  WinSeqs seqs;                 // ragged batch tables (n_seqs == 0: one sequence)
   unsigned long long* times;    // debug: [CTA][2 * phases] %globaltimer at the start and at the end of every phase's work (or null)
 };
 
@@ -96,9 +97,7 @@ __device__ void lat_stem(const LatPhase& ph, const LatParams& p, LatStemSmem& sm
     const int t = (int)(f - n * T);
     const float* fr;
     if (p.win.frames > 0) {
-      long long fi = (p.win_n0 + (long long)n) * p.win.stride + t + p.win.offset;
-      fi = fi < 0 ? 0 : (fi >= p.win.frames ? p.win.frames - 1 : fi);
-      fr = p.x + fi * (int64_t)VC;
+      fr = p.x + win_frame(win_clip(p.win, p.seqs, p.win_n0 + (long long)n), t) * (int64_t)VC;
     } else {
       fr = p.x + f * (int64_t)VC;
     }
@@ -622,13 +621,14 @@ int tik_stgcn_latency_create(const TikNet* net, int64_t n_max, int T, void* work
   return TIK_OK;
 }
 
-static int lat_run(TikLatencyPlan* P, const float* x, const TikWindowing* win, int64_t N, float* poses, void* stream) {
+static int lat_run(TikLatencyPlan* P, const float* x, const TikWindowing* win, const TikSeqBatch* seqs, int64_t N, float* poses,
+                   void* stream) {
   using namespace tik;
   TIK_CHECK_ARG(P && x && poses && N >= 0 && N <= P->n_max, "latency plan: N outside [0, n_max]");
   if (N == 0) return TIK_OK;
   LatParams p;
   p.phases = P->phases_dev; p.n_phases = P->n_phases; p.nbr = P->nbr_dev; p.n_nbr = P->n_nbr;
-  p.x = x; p.poses = poses; p.N = N; p.win_n0 = 0; p.times = P->times_dev;
+  p.x = x; p.poses = poses; p.N = N; p.win_n0 = 0; p.seqs = win_seqs(seqs); p.times = P->times_dev;
   if (win) p.win = *win; else { p.win.frames = 0; p.win.offset = 0; p.win.stride = 1; p.win.root_a = -1; p.win.root_b = -1; }
   void* args[] = {&p};
   TIK_CUDA(cudaLaunchCooperativeKernel((const void*)stgcn_latency_kernel, dim3((unsigned)P->grid), dim3(kLatThreads), args, P->smem, (cudaStream_t)stream));
@@ -636,7 +636,7 @@ static int lat_run(TikLatencyPlan* P, const float* x, const TikWindowing* win, i
 }
 
 int tik_stgcn_latency_run(TikLatencyPlan* plan, const float* x_dev, int64_t N, float* poses_dev, void* stream) {
-  return lat_run(plan, x_dev, nullptr, N, poses_dev, stream);
+  return lat_run(plan, x_dev, nullptr, nullptr, N, poses_dev, stream);
 }
 
 int tik_stgcn_latency_run_windows(TikLatencyPlan* plan, const float* seq_dev, const TikWindowing* win, int64_t n_windows,
@@ -644,7 +644,19 @@ int tik_stgcn_latency_run_windows(TikLatencyPlan* plan, const float* seq_dev, co
   using namespace tik;
   TIK_CHECK_ARG(plan && win && win->frames > 0 && win->stride >= 1, "latency plan: windowing needs frames > 0 and stride >= 1");
   TIK_CHECK_ARG((win->root_a < 0) == (win->root_b < 0) && win->root_a < plan->net.V && win->root_b < plan->net.V, "latency plan: bad root keypoints");
-  return lat_run(plan, seq_dev, win, n_windows, poses_dev, stream);
+  return lat_run(plan, seq_dev, win, nullptr, n_windows, poses_dev, stream);
+}
+
+int tik_stgcn_latency_run_seq_windows(TikLatencyPlan* plan, const float* seq_dev, const TikWindowing* win,
+                                      const TikSeqBatch* seqs, int64_t n_windows, float* poses_dev, void* stream) {
+  using namespace tik;
+  int rc = check_seq_windows(win, seqs, n_windows, "latency plan");
+  if (rc != TIK_OK) return rc;
+  TIK_CHECK_ARG(plan != nullptr, "latency plan: null plan");
+  TIK_CHECK_ARG(win->root_a < plan->net.V && win->root_b < plan->net.V, "latency plan: root keypoints (%d, %d) must be < V = %d",
+                win->root_a, win->root_b, plan->net.V);
+  TIK_CHECK_ARG(seq_dev && poses_dev, "latency plan: null sequence or poses pointer");
+  return lat_run(plan, seq_dev, win, seqs, n_windows, poses_dev, stream);
 }
 
 int tik_stgcn_latency_phases(const TikLatencyPlan* plan) { return plan ? plan->n_phases : 0; }

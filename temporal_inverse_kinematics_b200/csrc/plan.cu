@@ -171,21 +171,21 @@ static void ws_layout(const TikNet* net, int dtype, int64_t n, int64_t n_max, in
 }
 
 static int run_step(TikPlan* P, Step& st, const float* xc, int64_t n, int64_t clip_off, float* poses, cudaStream_t s,
-                    const TikWindowing* win = nullptr, int64_t win_n0 = 0) {
+                    const TikWindowing* win = nullptr, int64_t win_n0 = 0, const WinSeqs& seqs = WinSeqs{nullptr, nullptr, 0}) {
   const TikNet& net = P->net;
   const int V = net.V;
   if (st.kind == Step::STEM) {
     const TikBlock& b = *st.blk;
     return stem_gcn_impl(P->dtype, xc, net.in_scale_dev, net.in_shift_dev, b.agg_dev, reinterpret_cast<const float*>(b.w_gcn_dev),
                          b.b_gcn_dev, st.dst, st.dst2 ? b.w_res_stem_dev : nullptr, st.dst2, b.stride, n, st.t, V, b.c_in, net.K,
-                         b.c_out, 1, win, win_n0, s);
+                         b.c_out, 1, win, win_n0, seqs, s);
   }
   if (st.kind == Step::AGG) {
     // planes are spaced for a full chunk (the tensor maps are baked for n_chunk clips)
     return tik_aggregate(P->dtype, st.src, st.blk->agg_dev, st.dst, P->n_chunk, st.t, V, st.c, net.K, s);
   }
   if (st.kind == Step::FUSED_GCN) return gcn_fused_launch(st.fused, n, s);
-  if (st.kind == Step::STEM_BLOCK) return stem_block_launch(st.stem_block, xc, n, win, win_n0, s);
+  if (st.kind == Step::STEM_BLOCK) return stem_block_launch(st.stem_block, xc, n, win, win_n0, seqs, s);
   if (st.kind == Step::TCN_HALO) return tcn_halo_launch(st.halo, n * V, s);
   TikRowGemm g = st.g;
   if (g.v == 1) {             // head: rows = n * T'
@@ -201,8 +201,9 @@ static int run_step(TikPlan* P, Step& st, const float* xc, int64_t n, int64_t cl
 
 static int run_impl(TikPlan* P, const float* x, int64_t N, float* poses, void* feat_out, cudaStream_t s,
                     std::vector<cudaEvent_t>* events, std::vector<std::pair<Step*, int64_t>>* trace,
-                    const TikWindowing* win = nullptr) {
+                    const TikWindowing* win = nullptr, const TikSeqBatch* seq_batch = nullptr) {
   const TikNet& net = P->net;
+  const WinSeqs seqs = win_seqs(seq_batch);
   const int V = net.V, T = P->T;
   auto mark = [&](Step* st, int64_t n) -> int {
     if (!events) return TIK_OK;
@@ -224,7 +225,7 @@ static int run_impl(TikPlan* P, const float* x, int64_t N, float* poses, void* f
         int rc = mark(&st, n);
         if (rc != TIK_OK) return rc;
         launch_opts() = {serp ? (k & 1) : 0};              // consecutive kernels walk the clips in opposite directions
-        rc = run_step(P, st, xc, n, n0, nullptr, s, win, b0 + n0);
+        rc = run_step(P, st, xc, n, n0, nullptr, s, win, b0 + n0, seqs);
         launch_opts() = {0};
         if (rc != TIK_OK) return rc;
         ++k;
@@ -477,6 +478,19 @@ int tik_stgcn_plan_run_windows(TikPlan* P, const float* seq, const TikWindowing*
   TIK_CHECK_ARG(P->net.blocks[0].res_kind != TIK_RES_STEM || P->net.blocks[0].c_in <= 8, "window mode needs the stem path");
   TIK_CHECK_ARG(P->net.head_hidden == 0 || poses, "poses pointer required");
   return run_impl(P, seq, n_windows, poses, feat_out, (cudaStream_t)stream, nullptr, nullptr, win);
+}
+
+int tik_stgcn_plan_run_seq_windows(TikPlan* P, const float* seq, const TikWindowing* win, const TikSeqBatch* seqs,
+                                   int64_t n_windows, float* poses, void* feat_out, void* stream) {
+  using namespace tik;
+  int rc = check_seq_windows(win, seqs, n_windows, "plan");
+  if (rc != TIK_OK) return rc;
+  TIK_CHECK_ARG(P != nullptr, "plan: null plan");
+  TIK_CHECK_ARG(win->root_a < P->net.V && win->root_b < P->net.V, "plan: root keypoints (%d, %d) must be < V = %d",
+                win->root_a, win->root_b, P->net.V);
+  TIK_CHECK_ARG(seq != nullptr, "plan: null sequence pointer");
+  TIK_CHECK_ARG(P->net.head_hidden == 0 || poses, "poses pointer required");
+  return run_impl(P, seq, n_windows, poses, feat_out, (cudaStream_t)stream, nullptr, nullptr, win, seqs);
 }
 
 int tik_stgcn_plan_profile(TikPlan* P, const float* x, int64_t N, float* poses, void* stream, double* ms_by_kind,

@@ -43,7 +43,8 @@ __global__ void __launch_bounds__(kStemThreads, (KCR <= 4 ? 3 : 1))
 stem_gcn_kernel(const float* __restrict__ x, const float* __restrict__ in_scale, const float* __restrict__ in_shift,
                 const float* __restrict__ agg, const float* __restrict__ w, const float* __restrict__ bias,
                 OutT* __restrict__ out, const float* __restrict__ res_w, OutT* __restrict__ res_out, int res_stride,
-                int T, int V, int Cin, int K, int Cout, int relu, const TikWindowing win, long long win_n0, long long n_clips) {
+                int T, int V, int Cin, int K, int Cout, int relu, const TikWindowing win, long long win_n0, const WinSeqs seqs,
+                long long n_clips) {
   extern __shared__ __align__(16) float smem[];
   const int KC = K * Cin, VC = V * Cin;
   float* s_raw = smem;                                // [frames][V*Cin] raw input
@@ -78,15 +79,14 @@ stem_gcn_kernel(const float* __restrict__ x, const float* __restrict__ in_scale,
     const int nf = min(kStemFrames, T - t0);
     __syncthreads();                                  // previous tile's readers are done with the staging arrays
     const float* gx = x + (n * T + t0) * (int64_t)VC; // (N,T,V,C): frames contiguous
+    // window mode: clip n is window win_n0 + n of the resident sequence(s); root-centred on 0.5*(kp[a]+kp[b])
+    // (InferenceDataset, data_amass.py:232-235)
+    const WinClip clip = win.frames > 0 ? win_clip(win, seqs, win_n0 + (long long)n) : WinClip{0, 0, 0};
     for (int i = threadIdx.x; i < nf * VC; i += kStemThreads) {
       const int vc = i % VC;
       float raw;
       if (win.frames > 0) {
-        // window mode: clip n is a window of one resident sequence (F,V,C); frame = clamp(n*stride + t + offset),
-        // i.e. sample_window's edge padding (data_amass.py:18-42), root-centred on 0.5*(kp[a]+kp[b]) (:232-235)
-        long long fi = (win_n0 + (long long)n) * win.stride + (t0 + i / VC) + win.offset;
-        fi = fi < 0 ? 0 : (fi >= win.frames ? win.frames - 1 : fi);
-        const float* fr = x + fi * VC;
+        const float* fr = x + win_frame(clip, t0 + i / VC) * VC;
         raw = __ldg(fr + vc);
         if (win.root_a >= 0) {
           const int c = vc % Cin;
@@ -151,7 +151,8 @@ stem_gcn_kernel(const float* __restrict__ x, const float* __restrict__ in_scale,
 template <class T>
 static int launch_stem(const float* x, const float* sc, const float* sh, const float* agg, const float* w,
                        const float* bias, void* out, const float* res_w, void* res_out, int res_stride, int64_t N,
-                       int Tn, int V, int Cin, int K, int Cout, int relu, const TikWindowing& win, int64_t win_n0, cudaStream_t s) {
+                       int Tn, int V, int Cin, int K, int Cout, int relu, const TikWindowing& win, int64_t win_n0, const WinSeqs& seqs,
+                       cudaStream_t s) {
   const size_t KC = (size_t)K * Cin;
   size_t smem = sizeof(float) * (2 * (size_t)kStemFrames * V * Cin + (size_t)kStemFrames * V * KC + (size_t)K * V * V);
   TIK_CHECK_ARG(KC <= (size_t)kStemMaxKCReg, "stem: K*Cin=%zu > %d is not instantiated", KC, kStemMaxKCReg);
@@ -170,11 +171,11 @@ static int launch_stem(const float* x, const float* sc, const float* sh, const f
   if (KC <= 4 && Cin <= 4)
     stem_gcn_kernel<T, 4, 4><<<gx, kStemThreads, smem, s>>>(x, sc, sh, agg, w, bias, reinterpret_cast<T*>(out), res_w,
                                                           reinterpret_cast<T*>(res_out), res_stride, Tn, V, Cin, K, Cout, relu, win,
-                                                          (long long)win_n0, (long long)N);
+                                                          (long long)win_n0, seqs, (long long)N);
   else
     stem_gcn_kernel<T, 16, 8><<<gx, kStemThreads, smem, s>>>(x, sc, sh, agg, w, bias, reinterpret_cast<T*>(out), res_w,
                                                           reinterpret_cast<T*>(res_out), res_stride, Tn, V, Cin, K, Cout, relu, win,
-                                                          (long long)win_n0, (long long)N);
+                                                          (long long)win_n0, seqs, (long long)N);
   TIK_LAUNCH_CHECK();
   return TIK_OK;
 }
@@ -185,20 +186,20 @@ namespace tik {
 int stem_gcn_impl(int dtype, const float* x, const float* in_scale, const float* in_shift, const float* agg,
                   const float* w, const float* bias, void* out, const float* res_w, void* res_out,
                   int res_stride, int64_t N, int T, int V, int Cin, int K, int Cout, int relu,
-                  const TikWindowing* winp, int64_t win_n0, cudaStream_t s);
+                  const TikWindowing* winp, int64_t win_n0, const WinSeqs& seqs, cudaStream_t s);
 }
 
 extern "C" int tik_stem_gcn(int dtype, const float* x, const float* in_scale, const float* in_shift, const float* agg,
                             const float* w, const float* bias, void* out, const float* res_w, void* res_out,
                             int res_stride, int64_t N, int T, int V, int Cin, int K, int Cout, int relu, void* stream) {
   return tik::stem_gcn_impl(dtype, x, in_scale, in_shift, agg, w, bias, out, res_w, res_out, res_stride, N, T, V, Cin, K, Cout,
-                            relu, nullptr, 0, (cudaStream_t)stream);
+                            relu, nullptr, 0, tik::WinSeqs{nullptr, nullptr, 0}, (cudaStream_t)stream);
 }
 
 int tik::stem_gcn_impl(int dtype, const float* x, const float* in_scale, const float* in_shift, const float* agg,
                        const float* w, const float* bias, void* out, const float* res_w, void* res_out,
                        int res_stride, int64_t N, int T, int V, int Cin, int K, int Cout, int relu,
-                       const TikWindowing* winp, int64_t win_n0, cudaStream_t s) {
+                       const TikWindowing* winp, int64_t win_n0, const WinSeqs& seqs, cudaStream_t s) {
   using namespace tik;
   TikWindowing win;
   if (winp) win = *winp; else { win.frames = 0; win.offset = 0; win.stride = 1; win.root_a = -1; win.root_b = -1; }
@@ -212,9 +213,9 @@ int tik::stem_gcn_impl(int dtype, const float* x, const float* in_scale, const f
   TIK_CHECK_ARG(res_w == nullptr || res_stride >= 1, "stem: bad residual stride");
   if (N == 0) return TIK_OK;
   if (dtype == TIK_F32)
-    return launch_stem<float>(x, in_scale, in_shift, agg, w, bias, out, res_w, res_out, res_stride, N, T, V, Cin, K, Cout, relu, win, win_n0, s);
+    return launch_stem<float>(x, in_scale, in_shift, agg, w, bias, out, res_w, res_out, res_stride, N, T, V, Cin, K, Cout, relu, win, win_n0, seqs, s);
   if (dtype == TIK_BF16)
-    return launch_stem<__nv_bfloat16>(x, in_scale, in_shift, agg, w, bias, out, res_w, res_out, res_stride, N, T, V, Cin, K, Cout, relu, win, win_n0, s);
+    return launch_stem<__nv_bfloat16>(x, in_scale, in_shift, agg, w, bias, out, res_w, res_out, res_stride, N, T, V, Cin, K, Cout, relu, win, win_n0, seqs, s);
   set_error("bad dtype %d", dtype);
   return TIK_ERR_INVALID;
 }

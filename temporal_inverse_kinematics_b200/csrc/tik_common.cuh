@@ -72,6 +72,52 @@ __device__ __forceinline__ void pdl_launch_dependents() { asm volatile("griddepc
 struct LaunchOpts { int rev; };
 LaunchOpts& launch_opts();
 
+// Window mode (TikWindowing): the packed-sequence tables of a ragged batch (TikSeqBatch), or n_seqs == 0 for one
+// sequence spanning all win.frames frames.
+struct WinSeqs { const int64_t* frame_start; const int64_t* window_start; long long n_seqs; };
+static inline WinSeqs win_seqs(const TikSeqBatch* b) {
+  return b ? WinSeqs{b->frame_start_dev, b->window_start_dev, (long long)b->n_seqs} : WinSeqs{nullptr, nullptr, 0};
+}
+
+// Host checks of a ragged-batch window call that need no plan (the tables themselves live on the device).
+static inline int check_seq_windows(const TikWindowing* win, const TikSeqBatch* seqs, int64_t n_windows, const char* who) {
+  TIK_CHECK_ARG(win != nullptr && seqs != nullptr, "%s: null windowing or sequence batch", who);
+  TIK_CHECK_ARG(seqs->n_seqs >= 1, "%s: n_seqs = %lld, need >= 1", who, (long long)seqs->n_seqs);
+  TIK_CHECK_ARG(seqs->frame_start_dev && seqs->window_start_dev, "%s: null frame_start or window_start table", who);
+  TIK_CHECK_ARG(n_windows >= 0, "%s: n_windows = %lld < 0", who, (long long)n_windows);
+  TIK_CHECK_ARG(win->frames > 0 && win->stride >= 1, "%s: windowing needs frames > 0 and stride >= 1", who);
+  TIK_CHECK_ARG((win->root_a < 0) == (win->root_b < 0), "%s: root_a and root_b must both be set or both be negative", who);
+  return TIK_OK;
+}
+
+// One window's frames: frame t reads packed frame f0 + clamp(base + t, 0, last).
+struct WinClip { long long base, f0, last; };
+
+#ifdef __CUDACC__
+// Looked up once per window (global window index g): the sequence is the last s with window_start[s] <= g (a binary
+// search, ceil(log2 S) + 1 loads), so sequences without windows are skipped.  Indices read from the tables are
+// clamped to the packed buffer: a malformed table gives wrong frames, never a read outside [0, win.frames).
+// Without tables: base = g*stride + offset, f0 = 0, last = frames - 1, today's single-sequence index.
+__device__ __forceinline__ WinClip win_clip(const TikWindowing& win, const WinSeqs& sq, long long g) {
+  if (sq.n_seqs <= 0) return WinClip{g * win.stride + win.offset, 0, win.frames - 1};
+  long long lo = 0, hi = sq.n_seqs - 1;
+  while (lo < hi) {
+    const long long mid = (lo + hi + 1) >> 1;
+    if (__ldg(sq.window_start + mid) <= g) lo = mid; else hi = mid - 1;
+  }
+  const long long n = g - (long long)__ldg(sq.window_start + lo), frames = win.frames;
+  const long long f0 = min(max((long long)__ldg(sq.frame_start + lo), 0ll), frames - 1);
+  const long long f1 = min(max((long long)__ldg(sq.frame_start + lo + 1), f0 + 1), frames);
+  return WinClip{n * win.stride + win.offset, f0, f1 - f0 - 1};
+}
+// Packed frame of frame t of the window: the edge padding of sample_window (mmskeleton/datasets/data_amass.py:18-42)
+// inside the window's own sequence.
+__device__ __forceinline__ long long win_frame(const WinClip& c, long long t) {
+  const long long fi = c.base + t;
+  return c.f0 + (fi < 0 ? 0 : (fi >= c.last ? c.last : fi));
+}
+#endif
+
 // fp32 implicit-GEMM arguments (stgcn_simt.cu rowgemm_f32_kernel, rowgemm_tf32.cu): TikRowGemm with the K offsets resolved
 struct F32Slab { const float* a; int c, t_in, t_mul, t_off, koff; };
 struct F32Args {
@@ -101,6 +147,6 @@ int launch_batch_rodrigues(const float* aa, float* R9, int64_t M, cudaStream_t s
 int stem_gcn_impl(int dtype, const float* x, const float* in_scale, const float* in_shift, const float* agg,
                   const float* w, const float* bias, void* out, const float* res_w, void* res_out,
                   int res_stride, int64_t N, int T, int V, int Cin, int K, int Cout, int relu,
-                  const TikWindowing* winp, int64_t win_n0, cudaStream_t s);
+                  const TikWindowing* winp, int64_t win_n0, const WinSeqs& seqs, cudaStream_t s);
 
 }  // namespace tik

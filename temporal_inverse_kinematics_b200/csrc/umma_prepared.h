@@ -4,7 +4,7 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
-#include "../../include/tik.h"
+#include "tik_common.cuh"
 
 namespace tik {
 struct UmmaPrepared;
@@ -27,7 +27,8 @@ struct StemBlockPrepared;
 bool stem_block_supported(const TikNet* net, int dtype);
 int64_t stem_block_workspace_bytes();
 int stem_block_prepare(const TikNet* net, void* w16_dev, void* out, int64_t n_clips, int T, StemBlockPrepared** outp);
-int stem_block_launch(StemBlockPrepared* g, const float* x, int64_t n_clips, const TikWindowing* win, int64_t win_n0, cudaStream_t s);
+int stem_block_launch(StemBlockPrepared* g, const float* x, int64_t n_clips, const TikWindowing* win, int64_t win_n0,
+                      const WinSeqs& seqs, cudaStream_t s);
 void stem_block_free(StemBlockPrepared* g);
 struct TcnHaloPrepared;
 // Stride-1 temporal conv + identity residual, weight-stationary, each activation row loaded once; tcn_halo.cu

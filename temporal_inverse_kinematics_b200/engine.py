@@ -321,6 +321,18 @@ class Plan:
                                                        L.stream_ptr(seq.device)))
         return poses
 
+    def run_seq_windows(self, seq, tables, n_windows, offset, stride, root):
+        """run_windows over a ragged batch of sequences packed in seq (frames, V, C): ``tables`` is the int64 device
+        tensor (2, n_seqs+1) of frame_start / window_start (inference.sequence_tables).  Window n of sequence s, frame
+        t = seq[frame_start[s] + clamp(n*stride + t + offset, 0, F_s - 1)]; windows come out in sequence order."""
+        p = self.packed
+        win, seqs = _seq_windowing(seq, tables, offset, stride, root)
+        poses = torch.empty((n_windows, self.T_out, p.head_out), dtype=torch.float32, device=seq.device)
+        with L.on_device(seq):
+            L.check(L.lib().tik_stgcn_plan_run_seq_windows(self.handle, L.ptr(seq), C.byref(win), C.byref(seqs), n_windows,
+                                                           L.ptr(poses), None, L.stream_ptr(seq.device)))
+        return poses
+
     def run(self, x, want_feat=False):
         p = self.packed
         N = x.shape[0]
@@ -373,6 +385,27 @@ class LatencyPlan:
             L.check(L.lib().tik_stgcn_latency_run_windows(self.handle, L.ptr(seq), C.byref(win), n_windows, L.ptr(poses),
                                                           L.stream_ptr(seq.device)))
         return poses
+
+    def run_seq_windows(self, seq, tables, n_windows, offset, stride, root):
+        """Plan.run_seq_windows in one cooperative launch (n_windows <= n_max)."""
+        p = self.packed
+        win, seqs = _seq_windowing(seq, tables, offset, stride, root)
+        poses = torch.empty((n_windows, self.T_out, p.head_out), dtype=torch.float32, device=seq.device)
+        with L.on_device(seq):
+            L.check(L.lib().tik_stgcn_latency_run_seq_windows(self.handle, L.ptr(seq), C.byref(win), C.byref(seqs), n_windows,
+                                                              L.ptr(poses), L.stream_ptr(seq.device)))
+        return poses
+
+
+def _seq_windowing(seq, tables, offset, stride, root):
+    """TikWindowing + TikSeqBatch of a ragged window call; tables (2, n_seqs+1) int64 on seq's device."""
+    if tables.dtype != torch.int64 or tables.dim() != 2 or tables.shape[0] != 2 or not tables.is_contiguous() \
+            or tables.device != seq.device:
+        raise ValueError("tables must be a contiguous (2, n_seqs+1) int64 tensor on the sequence's device")
+    win = L.TikWindowing(seq.shape[0], offset, stride, root[0] if root else -1, root[1] if root else -1)
+    row = tables.stride(0) * tables.element_size()
+    seqs = L.TikSeqBatch(tables.shape[1] - 1, tables.data_ptr(), tables.data_ptr() + row)
+    return win, seqs
 
 
 MAX_HEAD_CLIPS = 16384   # clips whose features are kept for one head launch (143 MB in bf16 at T=64)

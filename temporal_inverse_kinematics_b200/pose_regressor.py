@@ -7,6 +7,7 @@ Mirrors reference pose_trainer.py:66-133 (PoseRegressor) and :136-144 (IKPoseTra
 import argparse
 import os
 
+import numpy as np
 import torch
 import torch.nn as nn
 
@@ -92,13 +93,17 @@ class PoseRegressor(engine.EngineHolder, nn.Module, _ComputeDtypeMixin):
         return {"poses": poses}
 
 
-    def forward_windows(self, seq, win_frames, offset=0, stride=1, root=None, n_windows=None):
+    def forward_windows(self, seq, win_frames, offset=0, stride=1, root=None, n_windows=None, lengths=None):
         """Sliding-window inference over ONE sequence without materialising the windows.
 
         seq (F, V, C) CUDA fp32.  Window n, frame t is seq[clamp(n*stride + t + offset, 0, F-1)], optionally
         root-centred on 0.5*(kp[root[0]] + kp[root[1]]).  `offset=-(win//2)` with one window per frame reproduces
         InferenceDataset / sample_window (reference data_amass.py:18-42,221-236); `offset=0` gives plain
-        [n, n+win) windows (BASELINE config 5).  Returns {'poses': (n_windows, T', 66)}."""
+        [n, n+win) windows (BASELINE config 5).  Returns {'poses': (n_windows, T', 66)}.
+
+        lengths (host ints, sum = F): seq packs several sequences back to back and every one gets the windows it would
+        get on its own (n_windows must be None), clamped to its own frames; they come out in sequence order, in one
+        pass, equal bit for bit to torch.cat of the per-sequence calls (inference.sequence_tables)."""
         engine.require_cuda_eval(self, seq, "PoseRegressor.forward_windows")
         if seq.dim() != 3 or seq.shape[1] != self.backbone.A.size(1) or seq.shape[2] != self.backbone.st_gcn_networks[0].in_channels:
             raise ValueError(f"expected a (F, {self.backbone.A.size(1)}, C) sequence, got {tuple(seq.shape)}")
@@ -109,12 +114,28 @@ class PoseRegressor(engine.EngineHolder, nn.Module, _ComputeDtypeMixin):
             raise ValueError(f"root must be a pair of keypoint indices in [0, {V}), got {root!r}")
         if F < 1 or int(stride) < 1 or int(win_frames) < 1:
             raise ValueError("forward_windows needs a non-empty sequence, stride >= 1 and win_frames >= 1")
+        if lengths is not None:
+            return {"poses": self._forward_seq_windows(seq, int(win_frames), int(offset), int(stride), root, n_windows, lengths)}
         if n_windows is None:
             n_windows = F if offset < 0 else max(0, (F - win_frames - offset) // stride + 1)
         if n_windows == 0:
             return {"poses": seq.new_zeros((0, self.backbone.out_frames(win_frames), self.pose_dim))}
         plan = self.plan_for(n_windows, win_frames)
         return {"poses": plan.run_windows(seq, n_windows, offset, stride, root)}
+
+    def _forward_seq_windows(self, seq, win_frames, offset, stride, root, n_windows, lengths):
+        from .inference import sequence_tables
+        if n_windows is not None:
+            raise ValueError("forward_windows: n_windows follows from lengths; pass one or the other")
+        frame_start, window_start = sequence_tables(lengths, win_frames, offset, stride)
+        if int(frame_start[-1]) != seq.shape[0]:
+            raise ValueError(f"lengths sum to {int(frame_start[-1])} frames, the packed sequence has {seq.shape[0]}")
+        n_windows = int(window_start[-1])
+        if n_windows == 0:
+            return seq.new_zeros((0, self.backbone.out_frames(win_frames), self.pose_dim))
+        tables = torch.from_numpy(np.stack([frame_start, window_start])).to(seq.device)
+        plan = self.plan_for(n_windows, win_frames)
+        return plan.run_seq_windows(seq, tables, n_windows, offset, stride, root)
 
 
 class IterativePoseRegressor(engine.EngineHolder, nn.Module, _ComputeDtypeMixin):
