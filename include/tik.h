@@ -172,10 +172,11 @@ int tik_stem_gcn(int dtype, const float* x_dev, const float* in_scale_dev, const
                  const float* res_w_dev, void* res_out_dev, int res_stride,
                  int64_t N, int T, int V, int Cin, int K, int Cout, int relu, void* stream);
 
-/* Window mode of the stem (SURVEY.md section 8f row 1): instead of materialised (N,T,V,C) clips the stem reads one
- * resident sequence (frames,V,C); clip n, frame t is sequence frame clamp(n*stride + t + offset, 0, frames-1) --
- * the edge padding of sample_window (mmskeleton/datasets/data_amass.py:18-42) -- minus the root
- * 0.5*(kp[root_a] + kp[root_b]) of that frame (InferenceDataset, data_amass.py:232-235; root_a < 0: no centring). */
+/* Window mode of the stem (SURVEY.md section 8f row 1): the stem reads one resident sequence (frames,V,C); clip n,
+ * frame t is sequence frame clamp(n*stride + t + offset, 0, frames-1) -- the edge padding of sample_window
+ * (mmskeleton/datasets/data_amass.py:18-42) -- minus the root 0.5*(kp[root_a] + kp[root_b]) of that frame
+ * (InferenceDataset, data_amass.py:232-235; root_a < 0: no centring).  A batch of materialised (N,T,V,C) clips is the
+ * same read with frames = N*T, offset = 0, stride = T and no root: the library runs every batch that way. */
 typedef struct TikWindowing {
   int64_t frames;
   int32_t offset, stride, root_a, root_b;

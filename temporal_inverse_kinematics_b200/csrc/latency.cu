@@ -70,12 +70,11 @@ struct LatParams {
   const LatPhase* phases;
   const LatNbr* nbr;            // one neighbour table per block
   int n_phases, n_nbr;
-  const float* x;               // (N,T,V,Cin) clips, or one (frames,V,Cin) sequence in window mode
+  const float* x;               // (frames,V,Cin) input read through win: clip n is window n
   float* poses;
   int64_t N;
-  TikWindowing win;             // frames == 0: plain clips
-  int64_t win_n0;
-  WinSeqs seqs;                 // ragged batch tables (n_seqs == 0: one sequence)
+  TikWindowing win;
+  WinSeqs seqs;                 // ragged batch tables (n_seqs == 0: none)
   unsigned long long* times;    // debug: [CTA][2 * phases] %globaltimer at the start and at the end of every phase's work (or null)
 };
 
@@ -95,16 +94,11 @@ __device__ void lat_stem(const LatPhase& ph, const LatParams& p, LatStemSmem& sm
   for (int64_t f = blockIdx.x; f < frames; f += gridDim.x) {
     const int64_t n = f / T;
     const int t = (int)(f - n * T);
-    const float* fr;
-    if (p.win.frames > 0) {
-      fr = p.x + win_frame(win_clip(p.win, p.seqs, p.win_n0 + (long long)n), t) * (int64_t)VC;
-    } else {
-      fr = p.x + f * (int64_t)VC;
-    }
+    const float* fr = p.x + win_frame(win_clip(p.win, p.seqs, n), t) * (int64_t)VC;
     __syncthreads();                                   // the previous frame's readers are done
     if (tid < VC) {
       float raw = __ldg(fr + tid);
-      if (p.win.frames > 0 && p.win.root_a >= 0) {
+      if (p.win.root_a >= 0) {
         const int ci = tid % Cin;
         raw -= 0.5f * (__ldg(fr + p.win.root_a * Cin + ci) + __ldg(fr + p.win.root_b * Cin + ci));
       }
@@ -621,42 +615,39 @@ int tik_stgcn_latency_create(const TikNet* net, int64_t n_max, int T, void* work
   return TIK_OK;
 }
 
-static int lat_run(TikLatencyPlan* P, const float* x, const TikWindowing* win, const TikSeqBatch* seqs, int64_t N, float* poses,
+// Every run of a latency plan: clip n of the N clips is window n of x read through win (the entry point has checked
+// win itself, or built it for a plain batch).  Every argument check of the three entry points is here.
+static int lat_run(TikLatencyPlan* P, const float* x, const TikWindowing& win, const tik::WinSeqs& seqs, int64_t N, float* poses,
                    void* stream) {
   using namespace tik;
-  TIK_CHECK_ARG(P && x && poses && N >= 0 && N <= P->n_max, "latency plan: N outside [0, n_max]");
+  TIK_CHECK_ARG(P != nullptr, "latency plan: null plan");
+  TIK_CHECK_ARG(x && poses, "latency plan: null input or poses pointer");
+  TIK_CHECK_ARG(N >= 0 && N <= P->n_max, "latency plan: N = %lld outside [0, n_max = %lld]", (long long)N, (long long)P->n_max);
+  TIK_CHECK_ARG(win.root_a < P->net.V && win.root_b < P->net.V, "latency plan: root keypoints (%d, %d) must be < V = %d",
+                win.root_a, win.root_b, P->net.V);
   if (N == 0) return TIK_OK;
   LatParams p;
   p.phases = P->phases_dev; p.n_phases = P->n_phases; p.nbr = P->nbr_dev; p.n_nbr = P->n_nbr;
-  p.x = x; p.poses = poses; p.N = N; p.win_n0 = 0; p.seqs = win_seqs(seqs); p.times = P->times_dev;
-  if (win) p.win = *win; else { p.win.frames = 0; p.win.offset = 0; p.win.stride = 1; p.win.root_a = -1; p.win.root_b = -1; }
+  p.x = x; p.poses = poses; p.N = N; p.win = win; p.seqs = seqs; p.times = P->times_dev;
   void* args[] = {&p};
   TIK_CUDA(cudaLaunchCooperativeKernel((const void*)stgcn_latency_kernel, dim3((unsigned)P->grid), dim3(kLatThreads), args, P->smem, (cudaStream_t)stream));
   return TIK_OK;
 }
 
 int tik_stgcn_latency_run(TikLatencyPlan* plan, const float* x_dev, int64_t N, float* poses_dev, void* stream) {
-  return lat_run(plan, x_dev, nullptr, nullptr, N, poses_dev, stream);
+  return lat_run(plan, x_dev, tik::plain_windowing(N, plan ? plan->T : 0), tik::WinSeqs{}, N, poses_dev, stream);
 }
 
 int tik_stgcn_latency_run_windows(TikLatencyPlan* plan, const float* seq_dev, const TikWindowing* win, int64_t n_windows,
                                   float* poses_dev, void* stream) {
-  using namespace tik;
-  TIK_CHECK_ARG(plan && win && win->frames > 0 && win->stride >= 1, "latency plan: windowing needs frames > 0 and stride >= 1");
-  TIK_CHECK_ARG((win->root_a < 0) == (win->root_b < 0) && win->root_a < plan->net.V && win->root_b < plan->net.V, "latency plan: bad root keypoints");
-  return lat_run(plan, seq_dev, win, nullptr, n_windows, poses_dev, stream);
+  int rc = tik::check_windowing(win, "latency plan");
+  return rc != TIK_OK ? rc : lat_run(plan, seq_dev, *win, tik::WinSeqs{}, n_windows, poses_dev, stream);
 }
 
 int tik_stgcn_latency_run_seq_windows(TikLatencyPlan* plan, const float* seq_dev, const TikWindowing* win,
                                       const TikSeqBatch* seqs, int64_t n_windows, float* poses_dev, void* stream) {
-  using namespace tik;
-  int rc = check_seq_windows(win, seqs, n_windows, "latency plan");
-  if (rc != TIK_OK) return rc;
-  TIK_CHECK_ARG(plan != nullptr, "latency plan: null plan");
-  TIK_CHECK_ARG(win->root_a < plan->net.V && win->root_b < plan->net.V, "latency plan: root keypoints (%d, %d) must be < V = %d",
-                win->root_a, win->root_b, plan->net.V);
-  TIK_CHECK_ARG(seq_dev && poses_dev, "latency plan: null sequence or poses pointer");
-  return lat_run(plan, seq_dev, win, seqs, n_windows, poses_dev, stream);
+  int rc = tik::check_seq_windows(win, seqs, n_windows, "latency plan");
+  return rc != TIK_OK ? rc : lat_run(plan, seq_dev, *win, tik::win_seqs(*seqs), n_windows, poses_dev, stream);
 }
 
 int tik_stgcn_latency_phases(const TikLatencyPlan* plan) { return plan ? plan->n_phases : 0; }

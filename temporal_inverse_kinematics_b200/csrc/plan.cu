@@ -170,13 +170,15 @@ static void ws_layout(const TikNet* net, int dtype, int64_t n, int64_t n_max, in
   L->total_bytes = off;
 }
 
-static int run_step(TikPlan* P, Step& st, const float* xc, int64_t n, int64_t clip_off, float* poses, cudaStream_t s,
-                    const TikWindowing* win = nullptr, int64_t win_n0 = 0, const WinSeqs& seqs = WinSeqs{nullptr, nullptr, 0}) {
+// Clip k of the n clips of this step is window win_n0 + k of x read through win (the stem steps; the other steps read
+// the workspace).
+static int run_step(TikPlan* P, Step& st, const float* x, int64_t n, int64_t clip_off, float* poses, cudaStream_t s,
+                    const TikWindowing& win, int64_t win_n0, const WinSeqs& seqs) {
   const TikNet& net = P->net;
   const int V = net.V;
   if (st.kind == Step::STEM) {
     const TikBlock& b = *st.blk;
-    return stem_gcn_impl(P->dtype, xc, net.in_scale_dev, net.in_shift_dev, b.agg_dev, reinterpret_cast<const float*>(b.w_gcn_dev),
+    return stem_gcn_impl(P->dtype, x, net.in_scale_dev, net.in_shift_dev, b.agg_dev, reinterpret_cast<const float*>(b.w_gcn_dev),
                          b.b_gcn_dev, st.dst, st.dst2 ? b.w_res_stem_dev : nullptr, st.dst2, b.stride, n, st.t, V, b.c_in, net.K,
                          b.c_out, 1, win, win_n0, seqs, s);
   }
@@ -185,7 +187,7 @@ static int run_step(TikPlan* P, Step& st, const float* xc, int64_t n, int64_t cl
     return tik_aggregate(P->dtype, st.src, st.blk->agg_dev, st.dst, P->n_chunk, st.t, V, st.c, net.K, s);
   }
   if (st.kind == Step::FUSED_GCN) return gcn_fused_launch(st.fused, n, s);
-  if (st.kind == Step::STEM_BLOCK) return stem_block_launch(st.stem_block, xc, n, win, win_n0, seqs, s);
+  if (st.kind == Step::STEM_BLOCK) return stem_block_launch(st.stem_block, x, n, win, win_n0, seqs, s);
   if (st.kind == Step::TCN_HALO) return tcn_halo_launch(st.halo, n * V, s);
   TikRowGemm g = st.g;
   if (g.v == 1) {             // head: rows = n * T'
@@ -199,12 +201,18 @@ static int run_step(TikPlan* P, Step& st, const float* xc, int64_t n, int64_t cl
   return P->dtype == TIK_BF16 ? umma_launch(st.prep, &g, s) : rowgemm_f32_presplit(&g, st.w_big, st.w_small, s);
 }
 
-static int run_impl(TikPlan* P, const float* x, int64_t N, float* poses, void* feat_out, cudaStream_t s,
-                    std::vector<cudaEvent_t>* events, std::vector<std::pair<Step*, int64_t>>* trace,
-                    const TikWindowing* win = nullptr, const TikSeqBatch* seq_batch = nullptr) {
+// Every run of a plan: clip n of the N clips is window n of x read through win.  The entry points check win itself (or
+// build it for a plain batch: plain_windowing); every other argument check of the four of them is here.
+static int run_impl(TikPlan* P, const float* x, const TikWindowing& win, const WinSeqs& seqs, int64_t N, float* poses,
+                    void* feat_out, cudaStream_t s, std::vector<cudaEvent_t>* events = nullptr,
+                    std::vector<std::pair<Step*, int64_t>>* trace = nullptr) {
+  TIK_CHECK_ARG(P != nullptr, "plan: null plan");
+  TIK_CHECK_ARG(x != nullptr, "plan: null input pointer");
+  TIK_CHECK_ARG(N >= 0, "plan: N = %lld < 0", (long long)N);
+  TIK_CHECK_ARG(win.root_a < P->net.V && win.root_b < P->net.V, "plan: root keypoints (%d, %d) must be < V = %d",
+                win.root_a, win.root_b, P->net.V);
+  TIK_CHECK_ARG(P->net.head_hidden == 0 || poses, "plan: poses pointer required");
   const TikNet& net = P->net;
-  const WinSeqs seqs = win_seqs(seq_batch);
-  const int V = net.V, T = P->T;
   auto mark = [&](Step* st, int64_t n) -> int {
     if (!events) return TIK_OK;
     cudaEvent_t e;
@@ -219,13 +227,12 @@ static int run_impl(TikPlan* P, const float* x, int64_t N, float* poses, void* f
     const int64_t nb = std::min<int64_t>(P->n_max, N - b0);
     for (int64_t n0 = 0; n0 < nb; n0 += P->n_chunk) {
       const int64_t n = std::min<int64_t>(P->n_chunk, nb - n0);
-      const float* xc = win ? x : x + (b0 + n0) * (int64_t)T * V * net.c_in;   // window mode: x is the whole sequence
       int k = 0;
       for (auto& st : P->chunk_steps) {
         int rc = mark(&st, n);
         if (rc != TIK_OK) return rc;
         launch_opts() = {serp ? (k & 1) : 0};              // consecutive kernels walk the clips in opposite directions
-        rc = run_step(P, st, xc, n, n0, nullptr, s, win, b0 + n0, seqs);
+        rc = run_step(P, st, x, n, n0, nullptr, s, win, b0 + n0, seqs);
         launch_opts() = {0};
         if (rc != TIK_OK) return rc;
         ++k;
@@ -236,7 +243,7 @@ static int run_impl(TikPlan* P, const float* x, int64_t N, float* poses, void* f
       int rc = mark(&st, nb);
       if (rc != TIK_OK) return rc;
       launch_opts() = {serp && nb <= P->n_chunk ? (k & 1) : 0};   // several chunks: the features were not written in one sweep
-      rc = run_step(P, st, nullptr, nb, 0, poses ? poses + b0 * (int64_t)P->T_out * net.head_out : nullptr, s);
+      rc = run_step(P, st, nullptr, nb, 0, poses ? poses + b0 * (int64_t)P->T_out * net.head_out : nullptr, s, win, 0, seqs);
       launch_opts() = {0};
       if (rc != TIK_OK) return rc;
       ++k;
@@ -462,46 +469,31 @@ int tik_stgcn_plan_create(const TikNet* net, int dtype, int64_t n_chunk, int64_t
 
 int tik_stgcn_plan_run(TikPlan* P, const float* x, int64_t N, float* poses, void* feat_out, void* stream) {
   using namespace tik;
-  TIK_CHECK_ARG(P && x && N >= 0, "bad arguments");
-  TIK_CHECK_ARG(P->net.head_hidden == 0 || poses, "poses pointer required");
-  return run_impl(P, x, N, poses, feat_out, (cudaStream_t)stream, nullptr, nullptr);
+  return run_impl(P, x, plain_windowing(N, P ? P->T : 0), WinSeqs{}, N, poses, feat_out, (cudaStream_t)stream);
 }
 
 int tik_stgcn_plan_run_windows(TikPlan* P, const float* seq, const TikWindowing* win, int64_t n_windows, float* poses,
                                void* feat_out, void* stream) {
   using namespace tik;
-  TIK_CHECK_ARG(P && seq && win && n_windows >= 0, "bad arguments");
-  TIK_CHECK_ARG(win->frames > 0 && win->stride >= 1, "windowing needs frames > 0 and stride >= 1");
-  TIK_CHECK_ARG((win->root_a < 0) == (win->root_b < 0), "windowing: root_a and root_b must both be set or both be negative");
-  TIK_CHECK_ARG(win->root_a < P->net.V && win->root_b < P->net.V, "windowing: root keypoints (%d, %d) must be < V = %d",
-                win->root_a, win->root_b, P->net.V);
-  TIK_CHECK_ARG(P->net.blocks[0].res_kind != TIK_RES_STEM || P->net.blocks[0].c_in <= 8, "window mode needs the stem path");
-  TIK_CHECK_ARG(P->net.head_hidden == 0 || poses, "poses pointer required");
-  return run_impl(P, seq, n_windows, poses, feat_out, (cudaStream_t)stream, nullptr, nullptr, win);
+  int rc = check_windowing(win, "plan");
+  return rc != TIK_OK ? rc : run_impl(P, seq, *win, WinSeqs{}, n_windows, poses, feat_out, (cudaStream_t)stream);
 }
 
 int tik_stgcn_plan_run_seq_windows(TikPlan* P, const float* seq, const TikWindowing* win, const TikSeqBatch* seqs,
                                    int64_t n_windows, float* poses, void* feat_out, void* stream) {
   using namespace tik;
   int rc = check_seq_windows(win, seqs, n_windows, "plan");
-  if (rc != TIK_OK) return rc;
-  TIK_CHECK_ARG(P != nullptr, "plan: null plan");
-  TIK_CHECK_ARG(win->root_a < P->net.V && win->root_b < P->net.V, "plan: root keypoints (%d, %d) must be < V = %d",
-                win->root_a, win->root_b, P->net.V);
-  TIK_CHECK_ARG(seq != nullptr, "plan: null sequence pointer");
-  TIK_CHECK_ARG(P->net.head_hidden == 0 || poses, "poses pointer required");
-  return run_impl(P, seq, n_windows, poses, feat_out, (cudaStream_t)stream, nullptr, nullptr, win, seqs);
+  return rc != TIK_OK ? rc : run_impl(P, seq, *win, win_seqs(*seqs), n_windows, poses, feat_out, (cudaStream_t)stream);
 }
 
 int tik_stgcn_plan_profile(TikPlan* P, const float* x, int64_t N, float* poses, void* stream, double* ms_by_kind,
                            int64_t* launches_by_kind, double* flops_gemm) {
   using namespace tik;
-  TIK_CHECK_ARG(P && x && N >= 0 && ms_by_kind && launches_by_kind && flops_gemm, "bad arguments");
-  TIK_CHECK_ARG(P->net.head_hidden == 0 || poses, "poses pointer required");
+  TIK_CHECK_ARG(ms_by_kind && launches_by_kind && flops_gemm, "plan profile: null output pointer");
   std::vector<cudaEvent_t> ev;
   std::vector<std::pair<Step*, int64_t>> trace;
   cudaStream_t s = (cudaStream_t)stream;
-  int rc = run_impl(P, x, N, poses, nullptr, s, &ev, &trace);
+  int rc = run_impl(P, x, plain_windowing(N, P ? P->T : 0), WinSeqs{}, N, poses, nullptr, s, &ev, &trace);
   if (rc != TIK_OK) return rc;
   TIK_CUDA(cudaStreamSynchronize(s));
   for (int k = 0; k < 3; ++k) { ms_by_kind[k] = 0; launches_by_kind[k] = 0; }

@@ -78,22 +78,15 @@ stem_gcn_kernel(const float* __restrict__ x, const float* __restrict__ in_scale,
     const int t0 = (int)(tile - n * tiles_t) * kStemFrames;
     const int nf = min(kStemFrames, T - t0);
     __syncthreads();                                  // previous tile's readers are done with the staging arrays
-    const float* gx = x + (n * T + t0) * (int64_t)VC; // (N,T,V,C): frames contiguous
-    // window mode: clip n is window win_n0 + n of the resident sequence(s); root-centred on 0.5*(kp[a]+kp[b])
-    // (InferenceDataset, data_amass.py:232-235)
-    const WinClip clip = win.frames > 0 ? win_clip(win, seqs, win_n0 + (long long)n) : WinClip{0, 0, 0};
+    // clip n is window win_n0 + n of the input; root-centred on 0.5*(kp[a]+kp[b]) (InferenceDataset, data_amass.py:232-235)
+    const WinClip clip = win_clip(win, seqs, win_n0 + (long long)n);
     for (int i = threadIdx.x; i < nf * VC; i += kStemThreads) {
       const int vc = i % VC;
-      float raw;
-      if (win.frames > 0) {
-        const float* fr = x + win_frame(clip, t0 + i / VC) * VC;
-        raw = __ldg(fr + vc);
-        if (win.root_a >= 0) {
-          const int c = vc % Cin;
-          raw -= 0.5f * (__ldg(fr + win.root_a * Cin + c) + __ldg(fr + win.root_b * Cin + c));
-        }
-      } else {
-        raw = __ldg(gx + i);
+      const float* fr = x + win_frame(clip, t0 + i / VC) * VC;
+      float raw = __ldg(fr + vc);
+      if (win.root_a >= 0) {
+        const int c = vc % Cin;
+        raw -= 0.5f * (__ldg(fr + win.root_a * Cin + c) + __ldg(fr + win.root_b * Cin + c));
       }
       s_raw[i] = raw;
       s_bn[i] = fmaf(raw, __ldg(in_scale + vc), __ldg(in_shift + vc));
@@ -182,29 +175,19 @@ static int launch_stem(const float* x, const float* sc, const float* sh, const f
 
 }  // namespace tik
 
-namespace tik {
-int stem_gcn_impl(int dtype, const float* x, const float* in_scale, const float* in_shift, const float* agg,
-                  const float* w, const float* bias, void* out, const float* res_w, void* res_out,
-                  int res_stride, int64_t N, int T, int V, int Cin, int K, int Cout, int relu,
-                  const TikWindowing* winp, int64_t win_n0, const WinSeqs& seqs, cudaStream_t s);
-}
-
 extern "C" int tik_stem_gcn(int dtype, const float* x, const float* in_scale, const float* in_shift, const float* agg,
                             const float* w, const float* bias, void* out, const float* res_w, void* res_out,
                             int res_stride, int64_t N, int T, int V, int Cin, int K, int Cout, int relu, void* stream) {
   return tik::stem_gcn_impl(dtype, x, in_scale, in_shift, agg, w, bias, out, res_w, res_out, res_stride, N, T, V, Cin, K, Cout,
-                            relu, nullptr, 0, tik::WinSeqs{nullptr, nullptr, 0}, (cudaStream_t)stream);
+                            relu, tik::plain_windowing(N, T), 0, tik::WinSeqs{}, (cudaStream_t)stream);
 }
 
+// The windowing comes from the caller's entry point, which has checked it (or built it: plain_windowing).
 int tik::stem_gcn_impl(int dtype, const float* x, const float* in_scale, const float* in_shift, const float* agg,
                        const float* w, const float* bias, void* out, const float* res_w, void* res_out,
                        int res_stride, int64_t N, int T, int V, int Cin, int K, int Cout, int relu,
-                       const TikWindowing* winp, int64_t win_n0, const WinSeqs& seqs, cudaStream_t s) {
+                       const TikWindowing& win, int64_t win_n0, const WinSeqs& seqs, cudaStream_t s) {
   using namespace tik;
-  TikWindowing win;
-  if (winp) win = *winp; else { win.frames = 0; win.offset = 0; win.stride = 1; win.root_a = -1; win.root_b = -1; }
-  TIK_CHECK_ARG(win.frames == 0 || (win.stride >= 1 && win.root_a < V && win.root_b < V && (win.root_a < 0) == (win.root_b < 0)),
-                "stem: bad windowing");
   TIK_CHECK_ARG(x && in_scale && in_shift && agg && w && bias && out, "null pointer");
   TIK_CHECK_ARG(N >= 0 && T > 0 && V > 0 && V <= kStemMaxV && Cin > 0 && K > 0 && K <= 5 && K * Cin <= kStemMaxKC &&
                     Cout > 0 && Cout % 8 == 0,

@@ -69,7 +69,7 @@ struct StemBlockParams {
   const float* bias2; int32_t bias2_per_node;
   int32_t n_clips, T, V, lo, tiles_t;       // lo = output frames per tile, tiles_t = ceil(T / lo)
   TikWindowing win; long long win_n0;
-  WinSeqs seqs;                             // ragged batch tables (n_seqs == 0: one sequence)
+  WinSeqs seqs;                             // ragged batch tables (n_seqs == 0: none)
   unsigned long long* dbg;                  // TIK_PROBE builds: clock64 timeline of CTA 0, tile iteration 4
 };
 
@@ -377,15 +377,13 @@ __global__ void __launch_bounds__(kSbThreads, 1) stem_block_kernel(const __grid_
         const int n = tile / p.tiles_t, tt = tile - n * p.tiles_t;
         const int t_first = tt * p.lo - 1;
         const uint32_t dst = smem_u32(s_rawbuf + (it % kSbRawBufs) * (kSbL * kSbMaxV * 4)) + (uint32_t)tid * 4u;
-        // window mode: clip n is window win_n0 + n of the resident sequence(s)
-        const WinClip clip = p.win.frames > 0 ? win_clip(p.win, p.seqs, p.win_n0 + (long long)n) : WinClip{0, 0, 0};
+        const WinClip clip = win_clip(p.win, p.seqs, p.win_n0 + (long long)n);   // clip n is window win_n0 + n of the input
 #pragma unroll
         for (int k = 0; k < 3; ++k) {
           if (el_l[k] >= 0) {
             const int t = t_first + el_l[k];
             const bool ok = t >= 0 && t < p.T;
-            const long long fi = p.win.frames > 0 ? win_frame(clip, t) : (long long)n * p.T + t;
-            const float* src = ok ? p.x + fi * VC + el_vc[k] : p.x;
+            const float* src = ok ? p.x + win_frame(clip, t) * VC + el_vc[k] : p.x;
             asm volatile("cp.async.ca.shared.global [%0], [%1], 4, %2;" ::"r"(dst + (uint32_t)(k * NB) * 4u), "l"(src), "r"(ok ? 4 : 0) : "memory");
           }
         }
@@ -560,13 +558,13 @@ int stem_block_prepare(const TikNet* net, void* w16_dev, void* out, int64_t n_cl
   return TIK_OK;
 }
 
-int stem_block_launch(StemBlockPrepared* g, const float* x, int64_t n_clips, const TikWindowing* win, int64_t win_n0,
+int stem_block_launch(StemBlockPrepared* g, const float* x, int64_t n_clips, const TikWindowing& win, int64_t win_n0,
                       const WinSeqs& seqs, cudaStream_t s) {
   TIK_CHECK_ARG(g && x && n_clips <= g->cap, "stem block: n_clips exceeds the prepared capacity");
   if (n_clips <= 0) return TIK_OK;
   StemBlockParams p = g->p;
   p.x = x; p.n_clips = (int32_t)n_clips;
-  if (win) p.win = *win; else { p.win.frames = 0; p.win.offset = 0; p.win.stride = 1; p.win.root_a = -1; p.win.root_b = -1; }
+  p.win = win;
   p.win_n0 = (long long)win_n0;
   p.seqs = seqs;
 #ifdef TIK_PROBE

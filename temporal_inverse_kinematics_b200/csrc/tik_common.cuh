@@ -72,11 +72,24 @@ __device__ __forceinline__ void pdl_launch_dependents() { asm volatile("griddepc
 struct LaunchOpts { int rev; };
 LaunchOpts& launch_opts();
 
-// Window mode (TikWindowing): the packed-sequence tables of a ragged batch (TikSeqBatch), or n_seqs == 0 for one
-// sequence spanning all win.frames frames.
+// Every run reads its input through a TikWindowing.  A batch of N clips of T frames is window mode over its own N*T
+// frames with stride T and no root: clip n, frame t reads frame n*T + t, which is always inside [0, N*T - 1], so the
+// clamp never applies and the loaded address is that of the (N,T,V,C) layout.
+static inline TikWindowing plain_windowing(int64_t N, int T) { return TikWindowing{N * T, 0, T, -1, -1}; }
+
+// The packed-sequence tables of a ragged batch (TikSeqBatch), or n_seqs == 0 for one sequence spanning all
+// win.frames frames.
 struct WinSeqs { const int64_t* frame_start; const int64_t* window_start; long long n_seqs; };
-static inline WinSeqs win_seqs(const TikSeqBatch* b) {
-  return b ? WinSeqs{b->frame_start_dev, b->window_start_dev, (long long)b->n_seqs} : WinSeqs{nullptr, nullptr, 0};
+static inline WinSeqs win_seqs(const TikSeqBatch& b) {
+  return WinSeqs{b.frame_start_dev, b.window_start_dev, (long long)b.n_seqs};
+}
+
+// Host checks of a caller's windowing that need no plan.
+static inline int check_windowing(const TikWindowing* win, const char* who) {
+  TIK_CHECK_ARG(win != nullptr, "%s: null windowing", who);
+  TIK_CHECK_ARG(win->frames > 0 && win->stride >= 1, "%s: windowing needs frames > 0 and stride >= 1", who);
+  TIK_CHECK_ARG((win->root_a < 0) == (win->root_b < 0), "%s: root_a and root_b must both be set or both be negative", who);
+  return TIK_OK;
 }
 
 // Host checks of a ragged-batch window call that need no plan (the tables themselves live on the device).
@@ -85,9 +98,7 @@ static inline int check_seq_windows(const TikWindowing* win, const TikSeqBatch* 
   TIK_CHECK_ARG(seqs->n_seqs >= 1, "%s: n_seqs = %lld, need >= 1", who, (long long)seqs->n_seqs);
   TIK_CHECK_ARG(seqs->frame_start_dev && seqs->window_start_dev, "%s: null frame_start or window_start table", who);
   TIK_CHECK_ARG(n_windows >= 0, "%s: n_windows = %lld < 0", who, (long long)n_windows);
-  TIK_CHECK_ARG(win->frames > 0 && win->stride >= 1, "%s: windowing needs frames > 0 and stride >= 1", who);
-  TIK_CHECK_ARG((win->root_a < 0) == (win->root_b < 0), "%s: root_a and root_b must both be set or both be negative", who);
-  return TIK_OK;
+  return check_windowing(win, who);
 }
 
 // One window's frames: frame t reads packed frame f0 + clamp(base + t, 0, last).
@@ -97,7 +108,7 @@ struct WinClip { long long base, f0, last; };
 // Looked up once per window (global window index g): the sequence is the last s with window_start[s] <= g (a binary
 // search, ceil(log2 S) + 1 loads), so sequences without windows are skipped.  Indices read from the tables are
 // clamped to the packed buffer: a malformed table gives wrong frames, never a read outside [0, win.frames).
-// Without tables: base = g*stride + offset, f0 = 0, last = frames - 1, today's single-sequence index.
+// Without tables: base = g*stride + offset, f0 = 0, last = frames - 1 (one sequence, or a plain batch of clips).
 __device__ __forceinline__ WinClip win_clip(const TikWindowing& win, const WinSeqs& sq, long long g) {
   if (sq.n_seqs <= 0) return WinClip{g * win.stride + win.offset, 0, win.frames - 1};
   long long lo = 0, hi = sq.n_seqs - 1;
@@ -147,6 +158,6 @@ int launch_batch_rodrigues(const float* aa, float* R9, int64_t M, cudaStream_t s
 int stem_gcn_impl(int dtype, const float* x, const float* in_scale, const float* in_shift, const float* agg,
                   const float* w, const float* bias, void* out, const float* res_w, void* res_out,
                   int res_stride, int64_t N, int T, int V, int Cin, int K, int Cout, int relu,
-                  const TikWindowing* winp, int64_t win_n0, const WinSeqs& seqs, cudaStream_t s);
+                  const TikWindowing& win, int64_t win_n0, const WinSeqs& seqs, cudaStream_t s);
 
 }  // namespace tik

@@ -27,7 +27,7 @@ struct StemBlockPrepared;
 bool stem_block_supported(const TikNet* net, int dtype);
 int64_t stem_block_workspace_bytes();
 int stem_block_prepare(const TikNet* net, void* w16_dev, void* out, int64_t n_clips, int T, StemBlockPrepared** outp);
-int stem_block_launch(StemBlockPrepared* g, const float* x, int64_t n_clips, const TikWindowing* win, int64_t win_n0,
+int stem_block_launch(StemBlockPrepared* g, const float* x, int64_t n_clips, const TikWindowing& win, int64_t win_n0,
                       const WinSeqs& seqs, cudaStream_t s);
 void stem_block_free(StemBlockPrepared* g);
 struct TcnHaloPrepared;

@@ -313,25 +313,15 @@ class Plan:
     def run_windows(self, seq, n_windows, offset, stride, root):
         """Sliding windows of one resident sequence (F,V,C): window n, frame t = seq[clamp(n*stride + t + offset)],
         root-centred on 0.5*(kp[root[0]] + kp[root[1]]) if root is given.  Nothing is materialised."""
-        p = self.packed
-        win = L.TikWindowing(seq.shape[0], offset, stride, root[0] if root else -1, root[1] if root else -1)
-        poses = torch.empty((n_windows, self.T_out, p.head_out), dtype=torch.float32, device=seq.device)
-        with L.on_device(seq):
-            L.check(L.lib().tik_stgcn_plan_run_windows(self.handle, L.ptr(seq), C.byref(win), n_windows, L.ptr(poses), None,
-                                                       L.stream_ptr(seq.device)))
-        return poses
+        win, _ = _windowing(seq, offset, stride, root)
+        return _launch(self, L.lib().tik_stgcn_plan_run_windows, seq, n_windows, C.byref(win), n_windows)
 
     def run_seq_windows(self, seq, tables, n_windows, offset, stride, root):
         """run_windows over a ragged batch of sequences packed in seq (frames, V, C): ``tables`` is the int64 device
         tensor (2, n_seqs+1) of frame_start / window_start (inference.sequence_tables).  Window n of sequence s, frame
         t = seq[frame_start[s] + clamp(n*stride + t + offset, 0, F_s - 1)]; windows come out in sequence order."""
-        p = self.packed
-        win, seqs = _seq_windowing(seq, tables, offset, stride, root)
-        poses = torch.empty((n_windows, self.T_out, p.head_out), dtype=torch.float32, device=seq.device)
-        with L.on_device(seq):
-            L.check(L.lib().tik_stgcn_plan_run_seq_windows(self.handle, L.ptr(seq), C.byref(win), C.byref(seqs), n_windows,
-                                                           L.ptr(poses), None, L.stream_ptr(seq.device)))
-        return poses
+        win, seqs = _windowing(seq, offset, stride, root, tables)
+        return _launch(self, L.lib().tik_stgcn_plan_run_seq_windows, seq, n_windows, C.byref(win), C.byref(seqs), n_windows)
 
     def run(self, x, want_feat=False):
         p = self.packed
@@ -371,41 +361,39 @@ class LatencyPlan:
         return 1
 
     def run(self, x):
-        p = self.packed
-        poses = torch.empty((x.shape[0], self.T_out, p.head_out), dtype=torch.float32, device=x.device)
-        with L.on_device(x):
-            L.check(L.lib().tik_stgcn_latency_run(self.handle, L.ptr(x), x.shape[0], L.ptr(poses), L.stream_ptr(x.device)))
-        return poses
+        return _launch(self, L.lib().tik_stgcn_latency_run, x, x.shape[0], x.shape[0])
 
     def run_windows(self, seq, n_windows, offset, stride, root):
-        p = self.packed
-        win = L.TikWindowing(seq.shape[0], offset, stride, root[0] if root else -1, root[1] if root else -1)
-        poses = torch.empty((n_windows, self.T_out, p.head_out), dtype=torch.float32, device=seq.device)
-        with L.on_device(seq):
-            L.check(L.lib().tik_stgcn_latency_run_windows(self.handle, L.ptr(seq), C.byref(win), n_windows, L.ptr(poses),
-                                                          L.stream_ptr(seq.device)))
-        return poses
+        win, _ = _windowing(seq, offset, stride, root)
+        return _launch(self, L.lib().tik_stgcn_latency_run_windows, seq, n_windows, C.byref(win), n_windows)
 
     def run_seq_windows(self, seq, tables, n_windows, offset, stride, root):
         """Plan.run_seq_windows in one cooperative launch (n_windows <= n_max)."""
-        p = self.packed
-        win, seqs = _seq_windowing(seq, tables, offset, stride, root)
-        poses = torch.empty((n_windows, self.T_out, p.head_out), dtype=torch.float32, device=seq.device)
-        with L.on_device(seq):
-            L.check(L.lib().tik_stgcn_latency_run_seq_windows(self.handle, L.ptr(seq), C.byref(win), C.byref(seqs), n_windows,
-                                                              L.ptr(poses), L.stream_ptr(seq.device)))
-        return poses
+        win, seqs = _windowing(seq, offset, stride, root, tables)
+        return _launch(self, L.lib().tik_stgcn_latency_run_seq_windows, seq, n_windows, C.byref(win), C.byref(seqs), n_windows)
 
 
-def _seq_windowing(seq, tables, offset, stride, root):
-    """TikWindowing + TikSeqBatch of a ragged window call; tables (2, n_seqs+1) int64 on seq's device."""
+def _windowing(seq, offset, stride, root, tables=None):
+    """TikWindowing over seq (frames, V, C) and, for a ragged batch, the TikSeqBatch of ``tables`` (2, n_seqs+1) int64
+    on seq's device (None without tables)."""
+    win = L.TikWindowing(seq.shape[0], offset, stride, root[0] if root else -1, root[1] if root else -1)
+    if tables is None:
+        return win, None
     if tables.dtype != torch.int64 or tables.dim() != 2 or tables.shape[0] != 2 or not tables.is_contiguous() \
             or tables.device != seq.device:
         raise ValueError("tables must be a contiguous (2, n_seqs+1) int64 tensor on the sequence's device")
-    win = L.TikWindowing(seq.shape[0], offset, stride, root[0] if root else -1, root[1] if root else -1)
     row = tables.stride(0) * tables.element_size()
-    seqs = L.TikSeqBatch(tables.shape[1] - 1, tables.data_ptr(), tables.data_ptr() + row)
-    return win, seqs
+    return win, L.TikSeqBatch(tables.shape[1] - 1, tables.data_ptr(), tables.data_ptr() + row)
+
+
+def _launch(plan, entry, x, n, *args):
+    """poses (n, T', head_out) fp32 of one run of a Plan or LatencyPlan: entry(handle, x, *args, poses, [feat,] stream),
+    where the throughput plan's entry points take a feature output (not requested here) after the poses."""
+    poses = torch.empty((n, plan.T_out, plan.packed.head_out), dtype=torch.float32, device=x.device)
+    feat = (None,) if isinstance(plan, Plan) else ()
+    with L.on_device(x):
+        L.check(entry(plan.handle, L.ptr(x), *args, L.ptr(poses), *feat, L.stream_ptr(x.device)))
+    return poses
 
 
 MAX_HEAD_CLIPS = 16384   # clips whose features are kept for one head launch (143 MB in bf16 at T=64)

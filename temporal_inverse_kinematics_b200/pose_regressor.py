@@ -114,28 +114,24 @@ class PoseRegressor(engine.EngineHolder, nn.Module, _ComputeDtypeMixin):
             raise ValueError(f"root must be a pair of keypoint indices in [0, {V}), got {root!r}")
         if F < 1 or int(stride) < 1 or int(win_frames) < 1:
             raise ValueError("forward_windows needs a non-empty sequence, stride >= 1 and win_frames >= 1")
+        tables = None
         if lengths is not None:
-            return {"poses": self._forward_seq_windows(seq, int(win_frames), int(offset), int(stride), root, n_windows, lengths)}
-        if n_windows is None:
+            from .inference import sequence_tables
+            if n_windows is not None:
+                raise ValueError("forward_windows: n_windows follows from lengths; pass one or the other")
+            win_frames, offset, stride = int(win_frames), int(offset), int(stride)
+            tables = np.stack(sequence_tables(lengths, win_frames, offset, stride))
+            if int(tables[0, -1]) != F:
+                raise ValueError(f"lengths sum to {int(tables[0, -1])} frames, the packed sequence has {F}")
+            n_windows = int(tables[1, -1])
+        elif n_windows is None:
             n_windows = F if offset < 0 else max(0, (F - win_frames - offset) // stride + 1)
         if n_windows == 0:
             return {"poses": seq.new_zeros((0, self.backbone.out_frames(win_frames), self.pose_dim))}
         plan = self.plan_for(n_windows, win_frames)
-        return {"poses": plan.run_windows(seq, n_windows, offset, stride, root)}
-
-    def _forward_seq_windows(self, seq, win_frames, offset, stride, root, n_windows, lengths):
-        from .inference import sequence_tables
-        if n_windows is not None:
-            raise ValueError("forward_windows: n_windows follows from lengths; pass one or the other")
-        frame_start, window_start = sequence_tables(lengths, win_frames, offset, stride)
-        if int(frame_start[-1]) != seq.shape[0]:
-            raise ValueError(f"lengths sum to {int(frame_start[-1])} frames, the packed sequence has {seq.shape[0]}")
-        n_windows = int(window_start[-1])
-        if n_windows == 0:
-            return seq.new_zeros((0, self.backbone.out_frames(win_frames), self.pose_dim))
-        tables = torch.from_numpy(np.stack([frame_start, window_start])).to(seq.device)
-        plan = self.plan_for(n_windows, win_frames)
-        return plan.run_seq_windows(seq, tables, n_windows, offset, stride, root)
+        if tables is None:
+            return {"poses": plan.run_windows(seq, n_windows, offset, stride, root)}
+        return {"poses": plan.run_seq_windows(seq, torch.from_numpy(tables).to(seq.device), n_windows, offset, stride, root)}
 
 
 class IterativePoseRegressor(engine.EngineHolder, nn.Module, _ComputeDtypeMixin):

@@ -225,6 +225,22 @@ def test_bf16_forward_windows_equals_materialised_windows(win, offset, stride):
     assert float((got.cpu() - ref).abs().max()) < TOL_BF16_ABS
 
 
+@pytest.mark.parametrize("dtype,chunk,low_latency", [("fp32", None, False), ("bf16", 3, False), ("fp32", None, True)])
+def test_batch_is_window_mode_with_stride_T(dtype, chunk, low_latency):
+    """A batch of N clips of T frames is window mode over its own N*T frames with stride T, offset 0 and no root: the
+    stem kernels load the same addresses either way, so model(x) equals forward_windows bit for bit (fp32 stem kernel,
+    fused first block over several chunks, latency plan)."""
+    from temporal_inverse_kinematics_b200 import engine
+    n, t = 8, 40
+    m, _ = _model(dtype=dtype)
+    m.chunk_clips, m.low_latency = chunk, low_latency
+    assert isinstance(m.plan_for(n, t), engine.LatencyPlan) == low_latency
+    x = synth.make_clips(n, t, seed=55).cuda()
+    want = m(x)["poses"]
+    got = m.forward_windows(x.reshape(n * t, 17, 3), t, offset=0, stride=t, root=None, n_windows=n)["poses"]
+    assert torch.equal(got, want)
+
+
 @pytest.mark.parametrize("switch", ["TIK_NO_STEM_BLOCK", "TIK_NO_TS", "TIK_NO_FUSED_GCN", "TIK_NO_TCN_HALO"])
 def test_bf16_kernel_variants_agree(monkeypatch, switch):
     """Every specialised tensor-core kernel has a more general one behind it (first block: stem + temporal conv;
