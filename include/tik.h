@@ -396,12 +396,6 @@ void tik_stgcn_latency_destroy(TikLatencyPlan* plan);
  * at the start and at the end of every phase's work in every CTA (NULL switches it off).  tools/latency_phases.py. */
 int tik_debug_latency_times(TikLatencyPlan* plan, void* dev_buf);
 
-/* Experiment hook, not used by the product path: makes the tensor-core kernel read its A operand `rows`
- * rows below the tile start (mode 1 also sets the descriptor's base-offset field).  See DESIGN.md. */
-int tik_debug_set_umma_shift(int rows, int mode);
-/* Probe hook: device buffer of 16 uint64 receiving a clock64 timeline of CTA 0 (NULL switches it off). */
-int tik_debug_set_umma_times(void* dev_buf16);
-
 #ifdef __cplusplus
 }
 #endif

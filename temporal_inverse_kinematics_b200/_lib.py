@@ -133,8 +133,6 @@ _PROTOS = {
     "tik_stgcn_latency_phases": (C.c_int, [vp]),
     "tik_stgcn_latency_destroy": (None, [vp]),
     "tik_debug_latency_times": (C.c_int, [vp, vp]),
-    "tik_debug_set_umma_shift": (C.c_int, [C.c_int, C.c_int]),
-    "tik_debug_set_umma_times": (C.c_int, [vp]),
 }
 
 _lib = None

@@ -21,20 +21,8 @@ def _nvcc():
     raise RuntimeError("nvcc not found")
 
 
-STAMP = os.path.join(HERE, "build", "flavour.txt")
-
-
-def _flavour():
-    return "probe" if os.environ.get("TIK_PROBE") == "1" else "release"
-
-
 def _stale():
     if not os.path.exists(LIB):
-        return True
-    try:
-        if open(STAMP).read().strip() != _flavour():     # a probe build must never be mistaken for the product library
-            return True
-    except OSError:
         return True
     t = os.path.getmtime(LIB)
     deps = [os.path.join(CSRC, s) for s in SOURCES + HEADERS] + [os.path.abspath(__file__)]
@@ -50,8 +38,6 @@ def build(force=False, verbose=False):
              "--expt-relaxed-constexpr"]
     if verbose:
         flags += ["-Xptxas", "-v"]
-    if os.environ.get("TIK_PROBE") == "1":          # in-kernel clock64 probes for tools/umma_probe.py
-        flags += ["-DTIK_PROBE"]
     variant = os.environ.get("TIK_BUILD_VARIANT")   # A/B library next to the product one: build/libtik_<name>.so with -D<NAME>
     obj_dir = os.path.join(HERE, "build", variant) if variant else os.path.join(HERE, "build")
     if variant:
@@ -73,9 +59,6 @@ def build(force=False, verbose=False):
         raise RuntimeError("nvcc failed")
     out = os.path.join(HERE, "build", f"libtik_{variant}.so") if variant else LIB
     subprocess.check_call([_nvcc(), "-shared", "-Wno-deprecated-gpu-targets", "-o", out, *objs, "-cudart", "static"])
-    if not variant:
-        with open(STAMP, "w") as f:
-            f.write(_flavour() + "\n")
     return out
 
 

@@ -70,15 +70,7 @@ struct StemBlockParams {
   int32_t n_clips, T, V, lo, tiles_t;       // lo = output frames per tile, tiles_t = ceil(T / lo)
   TikWindowing win; long long win_n0;
   WinSeqs seqs;                             // ragged batch tables (n_seqs == 0: none)
-  unsigned long long* dbg;                  // TIK_PROBE builds: clock64 timeline of CTA 0, tile iteration 4
 };
-
-#ifdef TIK_PROBE
-extern unsigned long long* g_dbg_times;   // stgcn_umma.cu (tik_debug_set_umma_times)
-#define SB_T(i) do { if (p.dbg != nullptr && blockIdx.x == 0) p.dbg[32 + (i)] = clock64(); } while (0)
-#else
-#define SB_T(i) do { } while (0)
-#endif
 
 __device__ __forceinline__ uint32_t bf16_bits(float v) { return (uint32_t)__bfloat16_as_ushort(__float2bfloat16_rn(v)); }
 
@@ -169,7 +161,6 @@ __global__ void __launch_bounds__(kSbThreads, 1) stem_block_kernel(const __grid_
   const uint32_t tmem_base = *tmem_slot;
   pdl_launch_dependents();
   pdl_wait();                                               // tables above are constants; x may come from a previous kernel
-  if (threadIdx.x == 0) SB_T(0);
 
   if (warp == 0) {
     // ===================== weights (once) + TMA store issuer =====================
@@ -182,13 +173,10 @@ __global__ void __launch_bounds__(kSbThreads, 1) stem_block_kernel(const __grid_
         const int n = tile / p.tiles_t, tt = tile - n * p.tiles_t;
         const int b = it & 1;
         mbar_wait(&stage_full[b], (uint32_t)((it >> 1) & 1));
-        if (it == 4) SB_T(20);
         tma_store_4d(&p.map_out, s_h + (size_t)b * kSbHBytes + 1024, 0, tt * p.lo, 0, n);
         tma_store_commit();
         tma_store_wait_read0();
         mbar_arrive(&h_empty[b]);
-        if (it == 4) SB_T(21);
-        if (it == 5) SB_T(22);
       }
       tma_store_wait0();
     }
@@ -203,10 +191,8 @@ __global__ void __launch_bounds__(kSbThreads, 1) stem_block_kernel(const __grid_
     // waits for the previous final pass.
     auto issue_ah = [&](int it) {
       const int b = it & 1;
-      if (it == 4 && leader) SB_T(6);
       mbar_wait(&a0_full[b], (uint32_t)((it >> 1) & 1));
       tc_fence_after();
-      if (it == 4 && leader) SB_T(7);
       if (leader) {
 #pragma unroll
         for (int j = 0; j < 2; ++j)
@@ -220,7 +206,6 @@ __global__ void __launch_bounds__(kSbThreads, 1) stem_block_kernel(const __grid_
       const int b = it & 1;
       mbar_wait(&tmem_empty[b], (uint32_t)(((it >> 1) & 1) ^ 1));
       tc_fence_after();
-      if (it == 4 && leader) SB_T(8);
       if (leader) {
 #pragma unroll
         for (int j = 0; j < 2; ++j)
@@ -234,10 +219,8 @@ __global__ void __launch_bounds__(kSbThreads, 1) stem_block_kernel(const __grid_
     for (int it = 0; it < my_tiles; ++it) {
       const int b = it & 1;
       if (it + 1 < my_tiles) issue_ah(it + 1);
-      if (it == 4 && leader) SB_T(9);
       mbar_wait(&h_full[b], (uint32_t)((it >> 1) & 1));
       tc_fence_after();
-      if (it == 4 && leader) SB_T(10);
       if (leader) {
         const uint32_t hb = h_u32 + (uint32_t)b * kSbHBytes + 1024u;
 #pragma unroll
@@ -252,7 +235,6 @@ __global__ void __launch_bounds__(kSbThreads, 1) stem_block_kernel(const __grid_
           }
         }
         umma_commit(&d3_full[b]);
-        if (it == 4) SB_T(11);
       }
       __syncwarp();
       if (it + 1 < my_tiles) issue_ar(it + 1);
@@ -269,12 +251,9 @@ __global__ void __launch_bounds__(kSbThreads, 1) stem_block_kernel(const __grid_
       const int tile = (int)blockIdx.x + it * (int)gridDim.x;
       const int tt = tile % p.tiles_t;
       const int t_first = tt * p.lo - 1;                  // frame of tile row l = 0
-      if (it == 4 && threadIdx.x == 64) SB_T(12);
       mbar_wait(&da_full[b], ph);
       tc_fence_after();
-      if (it == 4 && threadIdx.x == 64) SB_T(13);
       mbar_wait(&h_empty[b], ph ^ 1);                     // the store that read this buffer as a staging tile is done
-      if (it == 4 && threadIdx.x == 64) SB_T(15);
       uint8_t* hb = s_h + (size_t)b * kSbHBytes + 1024;
 #pragma unroll
       for (int j = 0; j < 2; ++j) {                       // one 128-row MMA tile at a time: 32 live accumulator registers
@@ -300,13 +279,10 @@ __global__ void __launch_bounds__(kSbThreads, 1) stem_block_kernel(const __grid_
           *reinterpret_cast<uint4*>(hb + (size_t)h * 128 + (((half * 4 + q) ^ (h & 7)) << 4)) = u;
         }
       }
-      if (it == 4 && threadIdx.x == 64) SB_T(23);
       tc_fence_before();
       fence_proxy_async_smem();
-      if (it == 4 && threadIdx.x == 64) SB_T(24);
       __syncwarp();
       if (lane == 0) mbar_arrive(&h_full[b]);
-      if (it == 4 && threadIdx.x == 64) SB_T(16);
     }
   } else if (warp < 2 + kSbEpiWarps) {
     // ===================== final group (8 warps): RD + b2 -> ReLU -> bf16 -> staging tile (aliases H0) =====================
@@ -314,14 +290,10 @@ __global__ void __launch_bounds__(kSbThreads, 1) stem_block_kernel(const __grid_
     const int half = (warp - 2 - kSbEpiWarps / 2) >> 2;
     const int i_row = lane_grp * 32 + lane;
     const uint32_t lane_off = (uint32_t)(lane_grp * 32) << 16;
-    const bool probe_thread = threadIdx.x == 32 * (2 + kSbEpiWarps / 2);
-    (void)probe_thread;
     for (int it = 0; it < my_tiles; ++it) {
       const int b = it & 1;
-      if (it == 4 && probe_thread) SB_T(17);
       mbar_wait(&d3_full[b], (uint32_t)((it >> 1) & 1));
       tc_fence_after();
-      if (it == 4 && probe_thread) SB_T(18);
       uint8_t* stage = s_h + (size_t)b * kSbHBytes + 1024;
 #pragma unroll
       for (int j = 0; j < 2; ++j) {
@@ -355,7 +327,6 @@ __global__ void __launch_bounds__(kSbThreads, 1) stem_block_kernel(const __grid_
       fence_proxy_async_smem();
       __syncwarp();
       if (lane == 0) mbar_arrive(&stage_full[b]);
-      if (it == 4 && probe_thread) SB_T(19);
     }
   } else {
     // ===================== builders: raw keypoints -> one K=16 operand slice per tile row =====================
@@ -394,16 +365,11 @@ __global__ void __launch_bounds__(kSbThreads, 1) stem_block_kernel(const __grid_
     prefetch(1);
     for (int it = 0; it < my_tiles; ++it) {
       const int b = it & 1;
-      if (it == 4 && tid == 0) SB_T(1);
       prefetch(it + 2);
-      if (it == 4 && tid == 0) SB_T(28);
       asm volatile("cp.async.wait_group 2;" ::: "memory");
-      if (it == 4 && tid == 0) SB_T(29);
       named_bar_sync(3, NB);                                // every thread's copies of tile `it` have landed
       const float* raw = s_rawbuf + (it % kSbRawBufs) * (kSbL * kSbMaxV * 4);
-      if (it == 4 && tid == 0) SB_T(2);
       mbar_wait(&a0_empty[b], (uint32_t)(((it >> 1) & 1) ^ 1));
-      if (it == 4 && tid == 0) SB_T(3);
       const int h = tid;
       if (h < V * kSbL) {
         const int v = h / kSbL, l = h - v * kSbL;
@@ -433,7 +399,6 @@ __global__ void __launch_bounds__(kSbThreads, 1) stem_block_kernel(const __grid_
 #pragma unroll
             for (int c = 0; c < CIN; ++c) agg[c] = fmaf(w[k][c], xv[k][c], agg[c]);
         }
-        if (it == 4 && tid == 0) SB_T(25);
         // slots: [agg_hi(CIN) | agg_lo(CIN) | xs_hi(CIN) | xs_lo(CIN) | 0...]
         uint32_t e[16];
 #pragma unroll
@@ -453,14 +418,10 @@ __global__ void __launch_bounds__(kSbThreads, 1) stem_block_kernel(const __grid_
         *reinterpret_cast<uint4*>(row + ((0 ^ (h & 7)) << 4)) = p0;
         *reinterpret_cast<uint4*>(row + ((1 ^ (h & 7)) << 4)) = p1;
       }
-      if (it == 4 && tid == 0) SB_T(26);
       fence_proxy_async_smem();
-      if (it == 4 && tid == 0) SB_T(27);
       __syncwarp();
       if (lane == 0) mbar_arrive(&a0_full[b]);
-      if (it == 4 && tid == 0) SB_T(4);
       named_bar_sync(3, NB);                                // the raw buffer is refilled by the next prefetch
-      if (it == 4 && tid == 0) SB_T(5);
     }
     asm volatile("cp.async.wait_group 0;" ::: "memory");
   }
@@ -567,9 +528,6 @@ int stem_block_launch(StemBlockPrepared* g, const float* x, int64_t n_clips, con
   p.win = win;
   p.win_n0 = (long long)win_n0;
   p.seqs = seqs;
-#ifdef TIK_PROBE
-  p.dbg = g_dbg_times;
-#endif
   static bool attr_done[64] = {};
   int dev = 0;
   TIK_CUDA(cudaGetDevice(&dev));

@@ -75,9 +75,6 @@ struct UmmaParams {
   const __nv_bfloat16* w_gmem;     // ts: (c_out, ktot) row-major weights
   int32_t ktot;
   int32_t rev;                     // LaunchOpts: tiles walked last to first
-  unsigned long long* dbg_times;   // probe hook: clock64 timeline of CTA 0 (tools/umma_probe.py)
-  int32_t dbg_flags;               // probe hook: 1 skip epilogue body, 2 skip residual, 4 skip MMAs, 8 skip A loads
-  int32_t dbg_shift_rows, dbg_base_offset_mode;   // experiment hook: A operand read at a row offset (tik_debug_set_umma_shift)
 };
 
 __device__ __forceinline__ float apply_act(float v, int act, float slope) {
@@ -86,19 +83,9 @@ __device__ __forceinline__ float apply_act(float v, int act, float slope) {
   return v;
 }
 
-// clock64 timeline probes (tools/umma_probe.py): compiled in only with -DTIK_PROBE (TIK_PROBE=1 python -m ...build)
-#ifdef TIK_PROBE
-#define TIK_T(i) do { if (p.dbg_times != nullptr && blockIdx.x == 0) p.dbg_times[i] = clock64(); } while (0)
-#define TIK_PROBE_ONLY(x) (x)
-#else
-#define TIK_T(i) do { } while (0)
-#define TIK_PROBE_ONLY(x) false
-#endif
-
 template <int BN, int ACT>
 __global__ void __launch_bounds__(kUmmaThreads, 1) rowgemm_umma_kernel(const __grid_constant__ UmmaParams p) {
   constexpr int kBBytes = BN * kChunkK * 2;
-  if (threadIdx.x == 0) TIK_T(0);
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);   // 1024-aligned; pointer arithmetic on the shared base keeps the address space (LDS / STS, not generic LD / ST)
   uint8_t* w_res = smem;                                    // resident weights: total_chunks x (BN x 64) tiles
@@ -143,7 +130,6 @@ __global__ void __launch_bounds__(kUmmaThreads, 1) rowgemm_umma_kernel(const __g
   const uint32_t tmem_base = *tmem_slot;
   pdl_launch_dependents();                                  // the next kernel may begin its own prologue
   pdl_wait();                                               // everything below reads what the previous kernel wrote
-  if (threadIdx.x == 0) TIK_T(1);
 
   if (warp == 0) {
     // ===================== TMA producer =====================
@@ -155,7 +141,6 @@ __global__ void __launch_bounds__(kUmmaThreads, 1) rowgemm_umma_kernel(const __g
       for (int kc = 0; kc < p.total_chunks; ++kc) tma_load_2d(w_res + (size_t)kc * kBBytes, &p.map_w, w_full, kc * kChunkK, 0);
     }
     const uint32_t tx_bytes = (uint32_t)(p.a_box_bytes + (p.w_resident ? 0 : kBBytes));
-    const bool skip_a = (p.dbg_flags & 8) != 0;
     const int group = p.group, total_chunks = p.total_chunks;
     int stage = 0; uint32_t phase = 0;
     for (int g = g0; g < num_tiles; g += gstep) {
@@ -170,23 +155,16 @@ __global__ void __launch_bounds__(kUmmaThreads, 1) rowgemm_umma_kernel(const __g
         const int ts = t0 * p.t_mul[s] + p.t_off[s];
         const int nc = p.chunks[s];
         for (int c = 0; c < nc; ++c, ++kw) {
-          const bool p3 = TIK_PROBE_ONLY(leader && kw == 0 && tile == (int)blockIdx.x + 3 * (int)gridDim.x);
-          if (p3) TIK_T(25);
           if (j == 0) {
             mbar_wait(&empty_bar[stage], phase ^ 1);
             const int in_stage = min(group, total_chunks - kw);
-            if (leader) {
-              if (skip_a && p.w_resident) mbar_arrive(&full_bar[stage]);
-              else mbar_expect_tx(&full_bar[stage], (skip_a ? (uint32_t)kBBytes : tx_bytes) * (uint32_t)in_stage);
-            }
+            if (leader) mbar_expect_tx(&full_bar[stage], tx_bytes * (uint32_t)in_stage);
           }
-          if (p3) TIK_T(26);
           uint8_t* sa = ring + (size_t)stage * stage_bytes + (size_t)j * chunk_bytes;
           if (leader) {
-            if (!skip_a) tma_load_3d(sa, &p.map_a[s], &full_bar[stage], c * kChunkK, ts, nv0);
+            tma_load_3d(sa, &p.map_a[s], &full_bar[stage], c * kChunkK, ts, nv0);
             if (!p.w_resident) tma_load_2d(sa + kABytes, &p.map_w, &full_bar[stage], kw * kChunkK, n0);
           }
-          if (p3) TIK_T(27);
           __syncwarp();
           if (++j == group || kw + 1 == total_chunks) {
             j = 0;
@@ -194,68 +172,43 @@ __global__ void __launch_bounds__(kUmmaThreads, 1) rowgemm_umma_kernel(const __g
           }
         }
       }
-      if (tile == blockIdx.x && leader) TIK_T(2);
     }
-    if (leader) TIK_T(11);
   } else if (warp == 1) {
     // ===================== MMA issuer =====================
     // Warp-uniform loop, one lane issues tcgen05.mma / tcgen05.commit.
     constexpr uint32_t idesc = make_idesc_bf16(kTileM, BN);
     const bool leader = lane == 0;
-    const bool skip_mma = (p.dbg_flags & 4) != 0;
     if (p.w_resident) mbar_wait(w_full, 0);
     const uint32_t ring_u32 = smem_u32(ring), wres_u32 = smem_u32(w_res);
     const uint64_t desc_hi = make_smem_desc_kmajor_sw128(0);          // everything but the start address
-    const uint32_t shift_bytes = (uint32_t)p.dbg_shift_rows * 128u;
     int stage = 0; uint32_t phase = 0;
     int acc = 0; uint32_t acc_phase = 0;
     const int total_chunks = p.total_chunks, group = p.group;
     for (int g = g0; g < num_tiles; g += gstep) {
-      const int tile = tile_of(g);
-      const bool m3 = TIK_PROBE_ONLY(leader && tile == (int)blockIdx.x + 3 * (int)gridDim.x);
-      if (m3) TIK_T(16);
       mbar_wait(&tmem_empty[acc], acc_phase ^ 1);        // epilogue has drained this accumulator
       tc_fence_after();
-      if (m3) TIK_T(17);
       const uint32_t tmem_d = tmem_base + (uint32_t)(acc * BN);
       for (int kc = 0; kc < total_chunks; kc += group) {
         mbar_wait(&full_bar[stage], phase);
         tc_fence_after();
-        if (m3 && kc < 2 * group) TIK_T(18 + 3 * (kc / group));
-        if (tile == blockIdx.x && kc == 0 && leader) TIK_T(3);
         const int in_stage = min(group, total_chunks - kc);
         for (int j = 0; j < in_stage; ++j) {
           const uint32_t sa = ring_u32 + (uint32_t)stage * (uint32_t)stage_bytes + (uint32_t)j * (uint32_t)chunk_bytes;
           const uint32_t sb = p.w_resident ? wres_u32 + (uint32_t)(kc + j) * (uint32_t)kBBytes : sa + kABytes;
           // descriptor = constant high part | (address >> 4); +2 per 16-element (32 B) K step inside the swizzled row
-          uint64_t da = desc_hi | (uint64_t)(((sa + shift_bytes) >> 4) & 0x3FFF);
-          if (p.dbg_base_offset_mode) da |= (uint64_t)(((sa + shift_bytes) >> 7) & 7u) << 49;
+          const uint64_t da = desc_hi | (uint64_t)((sa >> 4) & 0x3FFF);
           const uint64_t db = desc_hi | (uint64_t)((sb >> 4) & 0x3FFF);
-          if (leader && !skip_mma) {
+          if (leader) {
 #pragma unroll
             for (int k = 0; k < kChunkK / 16; ++k)
               umma_bf16(tmem_d, da + (uint64_t)(2 * k), db + (uint64_t)(2 * k), idesc, (kc | j | k) != 0 ? 1u : 0u);
-            if (TIK_PROBE_ONLY((p.dbg_flags & 96) != 0)) {   // issue-cost experiment: 12 extra MMAs, same accumulator (32) or alternating (64)
-              const uint32_t other = (p.dbg_flags & 64) ? tmem_base + (uint32_t)((acc ^ 1) * BN) : tmem_d;
-#pragma unroll
-              for (int k = 0; k < 12; ++k)
-                umma_bf16((k & 1) ? other : tmem_d, da + (uint64_t)(2 * (k & 3)), db + (uint64_t)(2 * (k & 3)), idesc, 1u);
-            }
           }
         }
-        if (leader) {
-          if (m3 && kc < 2 * group) TIK_T(19 + 3 * (kc / group));
-          umma_commit(&empty_bar[stage]);                  // frees this ring slot once the MMAs have read it
-          if (m3 && kc < 2 * group) TIK_T(20 + 3 * (kc / group));
-        }
+        if (leader) umma_commit(&empty_bar[stage]);        // frees this ring slot once the MMAs have read it
         __syncwarp();
         if (++stage == stages) { stage = 0; phase ^= 1; }
       }
-      if (leader) {
-        umma_commit(&tmem_full[acc]);                      // accumulator complete -> epilogue
-        if (tile == blockIdx.x) TIK_T(4);
-        if (m3) TIK_T(24);
-      }
+      if (leader) umma_commit(&tmem_full[acc]);          // accumulator complete -> epilogue
       __syncwarp();
       if (++acc == 2) { acc = 0; acc_phase ^= 1; }
     }
@@ -272,7 +225,7 @@ __global__ void __launch_bounds__(kUmmaThreads, 1) rowgemm_umma_kernel(const __g
         const int n0 = (tile - tm * ntn) * BN;
         const int tile_nv = tm / tiles_t, tile_t = tm - tile_nv * tiles_t;
         mbar_wait(&stage_full[sbuf], sphase);
-        for (int c = 0; c < ((p.dbg_flags & 16) ? 0 : BN / 64); ++c)
+        for (int c = 0; c < BN / 64; ++c)
           tma_store_3d(&p.map_out, s_stage + ((size_t)sbuf * (BN / 64) + c) * kABytes, n0 + c * 64, tile_t * p.tt, tile_nv * p.vv);
         tma_store_commit();
         if (p.stage_bufs == 2) {
@@ -296,7 +249,7 @@ __global__ void __launch_bounds__(kUmmaThreads, 1) rowgemm_umma_kernel(const __g
     const int cq = (warp - 2) >> 2;              // column quarter
     const int r = lane_grp * 32 + lane;          // tile row == TMEM lane
     const int nv_l = r / p.tt, t_l = r - nv_l * p.tt;
-    const bool use_res = p.res_kind == TIK_RES_IDENTITY && !(p.dbg_flags & 2);
+    const bool use_res = p.res_kind == TIK_RES_IDENTITY;
     const int ntn = p.n_tiles_n, tiles_t = p.tiles_t;
     int acc = 0; uint32_t acc_phase = 0;
     int sbuf = 0; uint32_t sphase = 0;
@@ -319,12 +272,8 @@ __global__ void __launch_bounds__(kUmmaThreads, 1) rowgemm_umma_kernel(const __g
       else out_off = row * p.c_out_valid + n0 + cb;
       uint8_t* stage_row = s_stage + (size_t)sbuf * (BN / 64) * kABytes + (size_t)r * 128;
 
-      const bool t3 = TIK_PROBE_ONLY((tile == (int)blockIdx.x + 3 * (int)gridDim.x) && threadIdx.x == 64);   // 4th tile of CTA 0
-      if (t3) TIK_T(12);
       mbar_wait(&tmem_full[acc], acc_phase);
       tc_fence_after();
-      if (t3) TIK_T(13);
-      if (tile == blockIdx.x && threadIdx.x == 64) TIK_T(5);
       const uint32_t tmem_d = tmem_base + (uint32_t)(acc * BN + cb) + ((uint32_t)(lane_grp * 32) << 16);
       uint32_t a[CW];
 #pragma unroll
@@ -336,7 +285,7 @@ __global__ void __launch_bounds__(kUmmaThreads, 1) rowgemm_umma_kernel(const __g
       if (lane == 0) mbar_arrive(&tmem_empty[acc]);
       // the store issued from this staging tile (stage_bufs tiles ago) must have finished reading it
       if (p.tma_store) mbar_wait(&stage_empty[sbuf], sphase ^ 1);
-      if ((valid || p.tma_store) && !(p.dbg_flags & 1)) {
+      if (valid || p.tma_store) {
 #pragma unroll
         for (int q = 0; q < CW / 8; ++q) {       // 8 columns = one 16-byte bf16 piece
           const float4 b0 = *reinterpret_cast<const float4*>(bias + 8 * q);
@@ -384,20 +333,15 @@ __global__ void __launch_bounds__(kUmmaThreads, 1) rowgemm_umma_kernel(const __g
           }
         }
       }
-      if (tile == blockIdx.x && threadIdx.x == 64) TIK_T(6);
-      if (t3) TIK_T(14);
       if (p.tma_store) {
         fence_proxy_async_smem();                           // st.shared -> visible to the TMA (async proxy)
         __syncwarp();
         if (lane == 0) mbar_arrive(&stage_full[sbuf]);      // 16 warps -> the store warp issues the tile
-        if (tile == blockIdx.x && threadIdx.x == 64) TIK_T(7);
-        if (t3) TIK_T(15);
         if (p.stage_bufs == 2) { if (++sbuf == 2) { sbuf = 0; sphase ^= 1; } } else { sphase ^= 1; }
       }
       if (++acc == 2) { acc = 0; acc_phase ^= 1; }
     }
   }
-  if (threadIdx.x == 64) TIK_T(8);
   __syncwarp();
   tc_fence_before();
   __syncthreads();
@@ -405,7 +349,6 @@ __global__ void __launch_bounds__(kUmmaThreads, 1) rowgemm_umma_kernel(const __g
     tc_fence_after();
     tmem_dealloc<2 * BN>(tmem_base);
   }
-  if (threadIdx.x == 64) TIK_T(10);
 }
 
 // ------------------------------------------------------------------------------------------------ weight-stationary variant
@@ -501,12 +444,9 @@ __global__ void __launch_bounds__(kUmmaThreads, 1) rowgemm_ts_kernel(const __gri
         for (int c = 0; c < nc; ++c, ++kw) {
           if (j == 0) {
             mbar_wait(&empty_bar[stage], phase ^ 1);
-            if (leader) {
-              if (TIK_PROBE_ONLY((p.dbg_flags & 8) != 0)) mbar_arrive(&full_bar[stage]);
-              else mbar_expect_tx(&full_bar[stage], (uint32_t)p.a_box_bytes * (uint32_t)min(group, total_chunks - kw));
-            }
+            if (leader) mbar_expect_tx(&full_bar[stage], (uint32_t)p.a_box_bytes * (uint32_t)min(group, total_chunks - kw));
           }
-          if (leader && !TIK_PROBE_ONLY((p.dbg_flags & 8) != 0))
+          if (leader)
             tma_load_3d(ring + (size_t)stage * stage_bytes + (size_t)j * kABytes, &p.map_a[s], &full_bar[stage], c * kChunkK, ts, nv0);
           __syncwarp();
           if (++j == group || kw + 1 == total_chunks) {
@@ -537,7 +477,7 @@ __global__ void __launch_bounds__(kUmmaThreads, 1) rowgemm_ts_kernel(const __gri
       int sidx = 0;
       for (int kc = 0; kc < total_chunks; kc += group, ++sidx) {
         if (!full_ready) mbar_wait(&full_bar[stage], phase);
-        if (!TIK_PROBE_ONLY((p.dbg_flags & 32) != 0)) tc_fence_after();
+        tc_fence_after();
         int nstage = stage + 1; uint32_t nphase = phase;
         if (nstage == stages) { nstage = 0; nphase ^= 1; }
         const bool last_stage = sidx + 1 == stages_per_tile;
@@ -550,16 +490,13 @@ __global__ void __launch_bounds__(kUmmaThreads, 1) rowgemm_ts_kernel(const __gri
         for (int j = 0; j < in_stage; ++j) {
           const uint32_t sa = ring_u32 + (uint32_t)stage * (uint32_t)stage_bytes + (uint32_t)j * (uint32_t)kABytes;
           const uint64_t db = desc_hi | (uint64_t)((sa >> 4) & 0x3FFF);
-          if (leader && !TIK_PROBE_ONLY((p.dbg_flags & 4) != 0)) {
+          if (leader) {
 #pragma unroll
             for (int k = 0; k < kChunkK / 16; ++k)
               umma_bf16_ts(tmem_d, tmem_w + (uint32_t)((kc + j) * 32 + k * 8), db + (uint64_t)(2 * k), idesc, (kc | j | k) != 0 ? 1u : 0u);
           }
         }
-        if (leader) {
-          if (TIK_PROBE_ONLY((p.dbg_flags & 64) != 0)) mbar_arrive(&empty_bar[stage]);   // experiment: cost of tcgen05.commit
-          else umma_commit(&empty_bar[stage]);
-        }
+        if (leader) umma_commit(&empty_bar[stage]);
         __syncwarp();
         stage = nstage; phase = nphase;
         full_ready = nfull; acc_ready = nacc;
@@ -577,7 +514,7 @@ __global__ void __launch_bounds__(kUmmaThreads, 1) rowgemm_ts_kernel(const __gri
         const int tile = p.rev ? n_tiles - 1 - ti : ti;
         const int tile_nv = tile / p.tiles_t, tile_t = tile - tile_nv * p.tiles_t;
         mbar_wait(&stage_full[sbuf], sphase);
-        for (int c = 0; c < (TIK_PROBE_ONLY((p.dbg_flags & 16) != 0) ? 0 : regions); ++c)
+        for (int c = 0; c < regions; ++c)
           tma_store_3d(&p.map_out, s_stage + ((size_t)sbuf * regions + c) * kABytes, c * 64, tile_t * p.tt, tile_nv * p.vv);
         tma_store_commit();
         if (p.stage_bufs == 2) {
@@ -627,7 +564,7 @@ __global__ void __launch_bounds__(kUmmaThreads, 1) rowgemm_ts_kernel(const __gri
       __syncwarp();
       if (lane == 0) mbar_arrive(&tmem_empty[acc]);
       mbar_wait(&stage_empty[sbuf], sphase ^ 1);
-      if (grp_ok && !TIK_PROBE_ONLY((p.dbg_flags & 1) != 0)) {
+      if (grp_ok) {
         const uint32_t st_u32 = smem_u32(s_stage + (size_t)sbuf * regions * kABytes);
 #pragma unroll
         for (int h = 0; h < 2; ++h) {
@@ -878,12 +815,8 @@ int umma_prepare(const TikRowGemm* d, int64_t nv_capacity, UmmaPrepared** out) {
   return TIK_OK;
 }
 
-static int g_dbg_shift_rows = 0, g_dbg_base_offset_mode = 0, g_dbg_flags = 0;
-unsigned long long* g_dbg_times = nullptr;   // also read by stem_block.cu in TIK_PROBE builds
-
 int umma_launch(UmmaPrepared* u, const TikRowGemm* d, cudaStream_t s) {
   UmmaParams& p = u->p;
-  p.dbg_shift_rows = g_dbg_shift_rows; p.dbg_base_offset_mode = g_dbg_base_offset_mode; p.dbg_flags = g_dbg_flags; p.dbg_times = g_dbg_times;
   TIK_CHECK_ARG(d->nv <= u->nv_capacity, "nv exceeds prepared capacity");
   p.nv = d->nv; p.v = d->v; p.t_out = d->t_out; p.c_out = d->c_out; p.c_out_valid = d->c_out_valid;
   p.bias = d->bias_dev; p.bias_per_node = d->bias_per_node;
@@ -987,16 +920,3 @@ int rowgemm_bf16(const TikRowGemm* d, cudaStream_t s) {
 }
 
 }  // namespace tik
-
-// Experiment hook (not part of the product path): read the A operand `rows` rows below the tile start, with the
-// descriptor's base-offset field either 0 (mode 0) or (start_address >> 7) & 7 (mode 1).
-extern "C" int tik_debug_set_umma_shift(int rows, int mode) {
-  tik::g_dbg_shift_rows = rows;
-  tik::g_dbg_base_offset_mode = mode & 0xff;
-  tik::g_dbg_flags = mode >> 8;      // probe flags ride in the upper bits (tools/umma_probe.py)
-  return TIK_OK;
-}
-extern "C" int tik_debug_set_umma_times(void* dev_buf16) {
-  tik::g_dbg_times = reinterpret_cast<unsigned long long*>(dev_buf16);
-  return TIK_OK;
-}

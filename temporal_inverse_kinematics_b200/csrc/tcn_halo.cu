@@ -7,7 +7,7 @@
 // Here a tile is G whole row groups (clip x node) with a one-frame halo on each side:
 //   rows j*(T+2) + (t+1),  t = -1 .. T        (the halo rows are TMA out-of-bounds zero fill = the conv's zero padding)
 // and the three taps are the SAME shared-memory tile read at row offsets 0, 1, 2 (a K-major 128B-swizzled operand may
-// start at any 128-byte row: tests/tools/gpu_check.py shift).  As in rowgemm_ts_kernel the GEMM is computed transposed,
+// start at any 128-byte row: DESIGN.md §3 (iii)).  As in rowgemm_ts_kernel the GEMM is computed transposed,
 //   D^T[c_out (TMEM lanes), n (TMEM columns)] = sum_taps W_tap (TMEM) . Htile[n + tap, :]^T  +  I . Xtile[n + 1, :]^T
 // with the BN-folded weights (and the identity block that carries the residual) written once per CTA into tensor
 // memory, N = the tile's rows rounded up to 16; output column n = j*(T+2) + t is valid for t < T.

@@ -1,6 +1,6 @@
 """Step-by-step GPU diagnostics (run on the B200 box; each stage in its own process via tests/tools/gpu_check.sh).
 
-    python tests/tools/gpu_check.py simt | umma | net
+    python tests/tools/gpu_check.py simt | umma | fused | net
 """
 import os
 import sys
@@ -129,28 +129,6 @@ def stage_umma():
     return ok
 
 
-def stage_shift():
-    """Experiment: can a 128B-swizzled K-major A operand start at an arbitrary ROW (not 1024 B) offset?"""
-    lib = _lib.lib()
-    g = torch.Generator().manual_seed(1)
-    a = torch.randn(1, 128, 64, generator=g).bfloat16()
-    w = (torch.randn(64, 64, generator=g) / 8).bfloat16()
-    b = torch.zeros(1, 64)
-    full = (a[0].float() @ w.float().t())
-    for shift in (1, 2, 8, 9, 17):
-        for mode in (0, 1):
-            lib.tik_debug_set_umma_shift(shift, mode)
-            y = ops.rowgemm([(a.cuda(), 1, 0)], w.cuda(), b.cuda(), 1, 1, 128, act="none")
-            torch.cuda.synchronize()
-            lib.tik_debug_set_umma_shift(0, 0)
-            got = y[0, :128 - shift].float().cpu()
-            want = full[shift:]
-            err = float((got - want).abs().max())
-            print(f"[shift] rows={shift} base_offset_mode={mode}: max err vs shifted rows {err:.3e} "
-                  f"(vs unshifted {float((got - full[:128 - shift]).abs().max()):.3e})", flush=True)
-    return True
-
-
 def stage_fused():
     """Fused graph conv (aggregation as a block-structured MMA with an MN-major B operand) vs a torch emulation."""
     ok = True
@@ -207,6 +185,6 @@ def stage_net():
 
 if __name__ == "__main__":
     stage = sys.argv[1]
-    ok = {"simt": stage_simt, "umma": stage_umma, "net": stage_net, "shift": stage_shift, "fused": stage_fused}[stage]()
+    ok = {"simt": stage_simt, "umma": stage_umma, "net": stage_net, "fused": stage_fused}[stage]()
     print(f"stage {stage}: {'PASS' if ok else 'FAIL'}")
     sys.exit(0 if ok else 1)

@@ -1,5 +1,8 @@
-"""Where does a tensor-core tile spend its time?  Times one layer-shaped launch with parts switched off
-(probe flags of tik_debug_set_umma_shift): 1 = epilogue body off, 2 = residual off, 4 = MMAs off, 8 = A loads off."""
+"""Whole-batch timings of the bf16 implicit GEMM (ops.rowgemm) at layer shapes of the network.
+
+    python tools/umma_probe.py grp [shape]   ring-stage grouping (TIK_UMMA_GROUP) x shared-memory option (TIK_UMMA_OPT)
+    python tools/umma_probe.py fill          DRAM or the L2 -> shared-memory fill: which binds the temporal conv?
+"""
 import os
 import sys
 
@@ -7,7 +10,7 @@ import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
-from temporal_inverse_kinematics_b200 import _lib, ops  # noqa: E402
+from temporal_inverse_kinematics_b200 import ops  # noqa: E402
 
 
 def bench(fn, reps=20):
@@ -21,83 +24,6 @@ def bench(fn, reps=20):
     e1.record()
     torch.cuda.synchronize()
     return e0.elapsed_time(e1) / reps * 1e3
-
-
-NAMES = ["entry", "setup", "prod_tile0", "mma_full0", "mma_done0", "epi_full0", "epi_body0", "epi_store0", "epi_end", "store_wait",
-         "exit", "prod_end", "t3_start", "t3_full", "t3_body", "t3_store",
-         "M.top", "M.tmem_empty", "M.full0", "M.issued0", "M.commit0", "M.full1", "M.issued1", "M.commit1", "M.done", "P.top", "P.empty", "P.issued",
-         "x28", "x29", "x30", "x31"]
-
-
-def _print_tl(fl, tl):
-    print(f"   flags={fl} timeline: " + ", ".join(f"{n}={tl[i] - tl[0]}" for i, n in enumerate(NAMES) if tl[i]), flush=True)
-
-
-def case(name, n, t_in, t_out, cin_slabs, c_out, stride, residual):
-    V = 17
-    nv = n * V
-    g = torch.Generator(device="cuda").manual_seed(0)
-    srcs = [torch.randn(nv, t_in, c, device="cuda", generator=g).bfloat16() for c in sorted(set(cin_slabs))]
-    by_c = {s.shape[-1]: s for s in srcs}
-    pad = (len(cin_slabs) - 1) // 2 if len(cin_slabs) >= 3 else 0
-    slabs = []
-    for i, c in enumerate(cin_slabs):
-        off = (i - 1) if (len(cin_slabs) >= 3 and i < 3) else 0
-        slabs.append((by_c[c], stride if t_in != t_out or i < 3 else 1, off))
-    w = (torch.randn(c_out, sum(cin_slabs), device="cuda", generator=g) * 0.05).bfloat16()
-    b = torch.zeros(1, c_out, device="cuda")
-    res = torch.randn(nv, t_out, c_out, device="cuda", generator=g).bfloat16() if residual else None
-    lib = _lib.lib()
-    out = []
-    for flags in (0, 16, 1, 1 | 4 | 8):
-        lib.tik_debug_set_umma_shift(0, flags << 8)
-        us = bench(lambda: ops.rowgemm(slabs, w, b, nv, V, t_out, act="relu", residual=res))
-        out.append(f"flags={flags}: {us:7.1f}us")
-    lib.tik_debug_set_umma_shift(0, 0)
-    for fl in (0, 32, 64):
-        tb = torch.zeros(32, dtype=torch.int64, device="cuda")
-        lib.tik_debug_set_umma_times(_lib.ptr(tb))
-        lib.tik_debug_set_umma_shift(0, fl << 8)
-        for _ in range(3):
-            ops.rowgemm(slabs, w, b, nv, V, t_out, act="relu", residual=res)
-        torch.cuda.synchronize()
-        lib.tik_debug_set_umma_times(None)
-        lib.tik_debug_set_umma_shift(0, 0)
-        tl = tb.cpu().tolist()
-        _print_tl(fl, tl)
-    tiles = -(-nv * t_out // 128)
-    print(f"{name}: tiles={tiles} | " + " | ".join(out), flush=True)
-    return
-    if True:
-        tl = []
-    names = ["entry", "setup", "prod_tile0", "mma_full0", "mma_done0", "epi_full0", "epi_body0", "epi_store0", "epi_end", "store_wait",
-             "exit", "prod_end", "t3_start", "t3_full", "t3_body", "t3_store"]
-    print("   timeline(cycles from entry): " + ", ".join(f"{n}={tl[i] - tl[0]}" for i, n in enumerate(names) if tl[i]), flush=True)
-    tiles = -(-nv * t_out // 128)
-    print(f"{name}: tiles={tiles} | " + " | ".join(out), flush=True)
-
-
-def big():
-    """Whole-batch sized b1 temporal conv (4096 clips): which resource binds when everything streams from HBM?"""
-    V, n, T, C = 17, 4096, 64, 64
-    nv = n * V
-    g = torch.Generator(device="cuda").manual_seed(0)
-    h = torch.randn(nv, T, C, device="cuda", generator=g).bfloat16()
-    r0 = torch.randn(nv, T, C, device="cuda", generator=g).bfloat16()
-    w = (torch.randn(C, 4 * C, device="cuda", generator=g) * 0.05).bfloat16()
-    b = torch.zeros(1, C, device="cuda")
-    lib = _lib.lib()
-    for name, slabs in [("3 taps + residual slab", [(h, 1, -1), (h, 1, 0), (h, 1, 1), (r0, 1, 0)]),
-                        ("1 tap + residual slab (x2 K)", [(h, 1, 0), (r0, 1, 0), (h, 1, 0), (r0, 1, 0)]),
-                        ("1 tap only (K=64)", [(h, 1, 0)])]:
-        ww = w[:, : 64 * len(slabs)].contiguous()
-        res = []
-        for flags in (0, 16, 1, 1 | 16, 8, 8 | 1 | 16):
-            lib.tik_debug_set_umma_shift(0, flags << 8)
-            us = bench(lambda: ops.rowgemm(slabs, ww, b, nv, V, T, act="relu"), reps=5)
-            res.append(f"flags={flags}: {us:7.1f}us")
-        lib.tik_debug_set_umma_shift(0, 0)
-        print(f"big {name}: " + " | ".join(res), flush=True)
 
 
 def grp():
@@ -142,30 +68,6 @@ def grp():
     os.environ.pop("TIK_UMMA_OPT", None)
 
 
-def tsflags():
-    """Weight-stationary temporal conv at whole-batch size with parts switched off (probe build)."""
-    V, n = 17, 4096
-    g = torch.Generator(device="cuda").manual_seed(0)
-    nv = n * V
-    h = torch.randn(nv, 32, 128, device="cuda", generator=g).bfloat16()
-    x = torch.randn(nv, 32, 128, device="cuda", generator=g).bfloat16()
-    slabs = [(h, 1, -1), (h, 1, 0), (h, 1, 1), (x, 1, 0)]
-    w = (torch.randn(128, 512, device="cuda", generator=g) * 0.05).bfloat16()
-    b = torch.zeros(1, 128, device="cuda")
-    lib = _lib.lib()
-    for grp_ in ("", "1", "2"):
-        if grp_:
-            os.environ["TIK_UMMA_GROUP"] = grp_
-        res = []
-        for flags in (0, 1 | 4 | 8 | 16, 1 | 4 | 8 | 16 | 64):
-            lib.tik_debug_set_umma_shift(0, flags << 8)
-            us = bench(lambda: ops.rowgemm(slabs, w, b, nv, V, 32, act="relu"), reps=5)
-            res.append(f"f{flags}: {us:6.1f}")
-        lib.tik_debug_set_umma_shift(0, 0)
-        print(f"ts b3 tcn G={grp_ or 'auto'}: " + " | ".join(res), flush=True)
-    os.environ.pop("TIK_UMMA_GROUP", None)
-
-
 def fill():
     """Is the temporal conv bound by DRAM or by the L2 -> shared-memory fill?  Same K and fill bytes, different
     numbers of distinct tensors behind the four K slabs."""
@@ -187,29 +89,7 @@ def fill():
 
 
 if __name__ == "__main__":
-    if len(sys.argv) > 1 and sys.argv[1] == "fill":
-        fill()
-        sys.exit(0)
-    if len(sys.argv) > 1 and sys.argv[1] == "tsflags":
-        tsflags()
-        sys.exit(0)
-    if len(sys.argv) > 1 and sys.argv[1] == "grp":
-        grp()
-        sys.exit(0)
-    if len(sys.argv) > 1 and sys.argv[1] == "big":
-        big()
-        sys.exit(0)
-    if len(sys.argv) > 1 and sys.argv[1] == "tlbig":
-        case("b1 tcn  3x64    T64 +slab, 4096 clips", 4096, 64, 64, [64, 64, 64, 64], 64, 1, False)
-        case("b3 tcn  3x128+128 T32, 4096 clips", 4096, 32, 32, [128, 128, 128, 128], 128, 1, False)
-        sys.exit(0)
-    if len(sys.argv) > 1 and sys.argv[1] == "tl":
-        case("b1 tcn  3x64    T64 +slab", 128, 64, 64, [64, 64, 64, 64], 64, 1, False)
-        case("b3 tcn  3x128+128 T32", 128, 32, 32, [128, 128, 128, 128], 128, 1, False)
-        sys.exit(0)
-    case("b1 gcn  64->64  T64", 128, 64, 64, [64], 64, 1, False)
-    case("b1 tcn  3x64    T64 +res", 128, 64, 64, [64, 64, 64], 64, 1, True)
-    case("b3 gcn 128->128 T32", 128, 32, 32, [128], 128, 1, False)
-    case("b3 tcn  3x128   T32 +res", 128, 32, 32, [128, 128, 128], 128, 1, True)
-    case("b6 tcn  3x256+128 s2 T16->8", 128, 16, 8, [256, 256, 256, 128], 256, 2, False)
-    case("b3 tcn x4 clips", 512, 32, 32, [128, 128, 128], 128, 1, True)
+    modes = {"grp": grp, "fill": fill}
+    if len(sys.argv) < 2 or sys.argv[1] not in modes:
+        sys.exit(__doc__)
+    modes[sys.argv[1]]()
