@@ -8,8 +8,9 @@
 // Neither H0 nor R0 ever reaches HBM (the two-kernel path writes and re-reads both: 2.2 GB per 4096 clips); the
 // kernel reads the raw (N,T,V,3) fp32 keypoints and writes the node-major bf16 block output.
 //
-// A tile is 12 output frames x V nodes of one clip, computed from 14 input frames (one halo frame each side).
-// Rows are node-major inside the tile, h = v*14 + l (238 rows = two 128-row MMA tiles), so a temporal tap is a
+// A tile is lo = min(T, 13) output frames x V nodes of one clip, computed from 15 input frames (one halo frame each
+// side; rows past lo + 1 are zero).  Rows are node-major inside the tile, h = v*15 + l (V <= 17: at most 255 rows = two
+// 128-row MMA tiles), so a temporal tap is a
 // shift of the A operand by one 128-byte shared-memory row and a tap at a tile edge never crosses a node boundary
 // into a valid output row.
 //   builders (8 warps, SIMT): data_bn, adjacency aggregation and the residual's scaled input, written as ONE

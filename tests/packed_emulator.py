@@ -46,7 +46,7 @@ def stem_block_applies(packed):
     net = packed.net
     b = net.blocks[0]
     return (packed.tdtype == torch.bfloat16 and net.n_blocks > 1 and net.K == 1 and net.c_in == 3 and b.c_out == 64
-            and b.kt == 3 and b.stride == 1 and net.V <= 18 and b.res_kind in (0, 2))
+            and b.kt == 3 and b.stride == 1 and net.V <= 17 and b.res_kind in (0, 2))   # V * 15 tile rows <= 256
 
 
 def forward(packed, x):

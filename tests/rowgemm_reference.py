@@ -4,8 +4,17 @@
 
 A row is (row group nv = clip*V + node, frame t); slab s reads frame t*t_mul + t_off of its source, zero outside
 [0, t_in).  Works on whatever device the inputs live on (CPU for small cases, the GPU's fp64 units for head-sized ones).
+
+compare / verdict are the per-element comparator of a kernel result against this reference: |got - ref| <= R_BF16 |ref|
++ C_ACC S, plus a rounding-bias check (error model and measurement: tests/test_bf16_rowgemm.py).  The tik_rowgemm tests
+and the per-block plan tests (tests/test_gpu_plan_blocks.py) share it.
 """
 import torch
+
+R_BF16 = 2.0 ** -8            # half a bf16 ulp, relative: the output rounding
+C_ACC = 2.0 ** -20            # fp32 accumulation error relative to S
+BIAS_MAX_ULP = 0.1
+BIAS_MIN_ELEMS = 4096
 
 
 def gather(a, t_out, t_mul, t_off):
@@ -68,3 +77,44 @@ def reference(slabs, w, bias, nv, v, t_out, act="none", slope=0.01, residual=Non
     if not with_scale:
         return out
     return out, to_layout(scale, nv, v, t_out, out_layout, c_out_valid)
+
+
+def ulp_bf16(x):
+    """Spacing of bf16 numbers at |x| (x = m 2^e with 0.5 <= |m| < 1: eight significant bits -> 2^(e-8))."""
+    _, e = torch.frexp(x)
+    return torch.ldexp(torch.ones_like(x), e - 8)
+
+
+def compare(got, ref, scale, bf16_out):
+    """-> dict: ratio = max |got - ref| / tol, need_c = the smallest c that passes, and the rounding-bias means (in
+    bf16 ulps) over the well-conditioned elements."""
+    got, ref, scale = got.double(), ref.double(), scale.double()
+    r = R_BF16 if bf16_out else 0.0
+    err = (got - ref).abs()
+    tol = r * ref.abs() + C_ACC * scale
+    ratio = torch.where(tol > 0, err / tol.clamp_min(1e-300), torch.where(err > 0, torch.inf, 0.0))
+    excess = (err - r * ref.abs()).clamp_min(0)
+    need_c = torch.where(scale > 0, excess / scale.clamp_min(1e-300), torch.where(excess > 0, torch.inf, 0.0))
+    st = {"ratio": float(ratio.max()) if ratio.numel() else 0.0, "need_c": float(need_c.max()) if need_c.numel() else 0.0,
+          "finite": bool(torch.isfinite(got).all()), "n_bias": 0, "mean_ulp": 0.0, "toward_ulp": 0.0}
+    if bf16_out:
+        u = ulp_bf16(ref)
+        well = (ref != 0) & (C_ACC * scale <= u / 16)
+        st["n_bias"] = int(well.sum())
+        if st["n_bias"]:
+            d = ((got - ref) / u)[well]
+            st["mean_ulp"] = float(d.mean())
+            st["toward_ulp"] = float((d * ref.sign()[well]).mean())
+    return st
+
+
+def verdict(st):
+    """Reasons the comparator rejects a result (empty: accepted)."""
+    bad = []
+    if not st["finite"]:
+        bad.append("non-finite output")
+    if not st["ratio"] <= 1.0:
+        bad.append(f"max err/tol {st['ratio']:.3g}")
+    if st["n_bias"] >= BIAS_MIN_ELEMS and (abs(st["mean_ulp"]) >= BIAS_MAX_ULP or abs(st["toward_ulp"]) >= BIAS_MAX_ULP):
+        bad.append(f"rounding bias {st['mean_ulp']:+.3f} / {st['toward_ulp']:+.3f} ulp")
+    return bad

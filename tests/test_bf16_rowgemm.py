@@ -26,56 +26,10 @@ import ctypes as C
 import pytest
 import torch
 
-from rowgemm_reference import gather, reference, to_layout
+from rowgemm_reference import BIAS_MIN_ELEMS, compare, gather, reference, to_layout, ulp_bf16, verdict
 
-R_BF16 = 2.0 ** -8
-C_ACC = 2.0 ** -20
-BIAS_MAX_ULP = 0.1
-BIAS_MIN_ELEMS = 4096
 ACT_CODE = {"none": 0, "relu": 1, "leaky": 2}
 TUNING_VARS = ("TIK_UMMA_GROUP", "TIK_UMMA_OPT", "TIK_UMMA_BN", "TIK_NO_TS", "TIK_NO_ROWGEMM_CACHE")
-
-
-# ------------------------------------------------------------------------------------------------ comparator
-def ulp_bf16(x):
-    """Spacing of bf16 numbers at |x| (x = m 2^e with 0.5 <= |m| < 1: eight significant bits -> 2^(e-8))."""
-    _, e = torch.frexp(x)
-    return torch.ldexp(torch.ones_like(x), e - 8)
-
-
-def compare(got, ref, scale, bf16_out):
-    """-> dict: ratio = max |got - ref| / tol, need_c = the smallest c that passes, and the rounding-bias means (in
-    bf16 ulps) over the well-conditioned elements."""
-    got, ref, scale = got.double(), ref.double(), scale.double()
-    r = R_BF16 if bf16_out else 0.0
-    err = (got - ref).abs()
-    tol = r * ref.abs() + C_ACC * scale
-    ratio = torch.where(tol > 0, err / tol.clamp_min(1e-300), torch.where(err > 0, torch.inf, 0.0))
-    excess = (err - r * ref.abs()).clamp_min(0)
-    need_c = torch.where(scale > 0, excess / scale.clamp_min(1e-300), torch.where(excess > 0, torch.inf, 0.0))
-    st = {"ratio": float(ratio.max()) if ratio.numel() else 0.0, "need_c": float(need_c.max()) if need_c.numel() else 0.0,
-          "finite": bool(torch.isfinite(got).all()), "n_bias": 0, "mean_ulp": 0.0, "toward_ulp": 0.0}
-    if bf16_out:
-        u = ulp_bf16(ref)
-        well = (ref != 0) & (C_ACC * scale <= u / 16)
-        st["n_bias"] = int(well.sum())
-        if st["n_bias"]:
-            d = ((got - ref) / u)[well]
-            st["mean_ulp"] = float(d.mean())
-            st["toward_ulp"] = float((d * ref.sign()[well]).mean())
-    return st
-
-
-def verdict(st):
-    """Reasons the comparator rejects a result (empty: accepted)."""
-    bad = []
-    if not st["finite"]:
-        bad.append("non-finite output")
-    if not st["ratio"] <= 1.0:
-        bad.append(f"max err/tol {st['ratio']:.3g}")
-    if st["n_bias"] >= BIAS_MIN_ELEMS and (abs(st["mean_ulp"]) >= BIAS_MAX_ULP or abs(st["toward_ulp"]) >= BIAS_MAX_ULP):
-        bad.append(f"rounding bias {st['mean_ulp']:+.3f} / {st['toward_ulp']:+.3f} ulp")
-    return bad
 
 
 # ------------------------------------------------------------------------------------------------ cases

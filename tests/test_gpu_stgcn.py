@@ -274,9 +274,10 @@ def test_serpentine_order_is_bit_identical(monkeypatch, dtype, n, t):
 @pytest.mark.parametrize("n,t", [(1, 1), (1, 2), (2, 11), (1, 12), (2, 13), (3, 25), (7, 33), (2, 61), (1, 65), (2, 95),
                                  (1, 100), (2, 126), (1, 127), (1, 129), (1, 190), (1, 191), (1, 200), (1, 256), (33, 16)])
 def test_bf16_edge_shapes(n, t):
-    """Tile-boundary cases of the specialised kernels: 12 output frames per tile in the fused first block, G row groups
-    of T+2 rows per tile in the halo temporal conv (unsupported above 126 / 190 frames -> per-tap kernels), odd tile
-    counts in the paired 64-channel graph conv, single clips and single frames (tests/tools/shape_sweep.py has the long list)."""
+    """Tile-boundary cases of the specialised kernels: min(T, 13) output frames per tile in the fused first block, G row
+    groups of L+2 rows per tile in the halo temporal conv (long clips cut into segments of L frames, the last one ragged
+    when no divisor of T fits), odd tile counts in the paired 64-channel graph conv, single clips and single frames
+    (tests/tools/shape_sweep.py has the long list; tests/test_gpu_plan_blocks.py checks each block against fp64)."""
     m, sd = _model(dtype="bf16")
     x = synth.make_clips(n, t, seed=1000 * n + t)
     want = sp.regressor_forward(sd, x)["poses"]
