@@ -154,6 +154,29 @@ int tik_body_keypoints(const TikKeypointModel* m, const float* pose_dev, int pos
                        int betas_per_frame, const float* transl_dev, const int32_t* select_host, int n_select,
                        int64_t F, float* out_dev, void* stream);
 
+/* ------------------------------------------------------------------ keypoint fitting
+ * Poses that make tik_body_keypoints hit observed points: per frame f, a few Levenberg-Marquardt steps on
+ *   E(theta, tau) = sum_k w_k |kp_k(theta, beta, tau) - y_k|^2 + prior_weight |theta - theta0|^2
+ * over theta = the axis-angle rotations of joints 0..21 (joints 22..54 stay identity, as pose_J = 22 gives) and, with
+ * fit_transl = 1, the translation tau.  Analytic Jacobian (pose blend of the landmarks included); each iteration solves
+ * (H + mu diag(H)) delta = -g with H = J^T W J + prior_weight I, g = J^T W r + prior_weight (theta - theta0) by
+ * Cholesky and takes the step iff E drops strictly: mu starts at 1e-3, then mu = max(mu/10, 1e-7) on acceptance and
+ * min(mu*10, 1e7) on rejection (a non-positive pivot is a rejection).  n_iter counts solves; E never increases.
+ *   m, betas_dev, betas_per_frame, select_host, n_select: as tik_body_keypoints.
+ *   target_dev (F, n_select, 3): the points y; weights_dev NULL (all 1), (n_select) (weights_per_frame = 0) or
+ *   (F, n_select) (weights_per_frame = 1), non-negative; init_pose_dev (F,22,3): theta0, the start and the prior's
+ *   centre; transl_dev (F,3) or NULL (zero): tau's start (fit_transl = 1) or its fixed value (fit_transl = 0);
+ *   prior_weight > 0 (keeps the system positive definite); n_iter >= 0.
+ *   pose_out_dev (F,22,3); transl_out_dev (F,3) or NULL; cost_dev (F,2) [initial E, final E] or NULL.  A frame whose
+ *   initial E is not finite is returned unchanged with final cost NaN.
+ * fp32, one warp per frame; frames are independent and a frame's result does not depend on the rest of the call.  No
+ * workspace, no host synchronisation, CUDA-graph capturable; F = 0 is a no-op; outputs may not overlap inputs or each
+ * other (checked); nothing outside the outputs is written. */
+int tik_fit_keypoints(const TikKeypointModel* m, const float* target_dev, const float* weights_dev, int weights_per_frame,
+                      const float* init_pose_dev, const float* betas_dev, int betas_per_frame, const float* transl_dev,
+                      int fit_transl, const int32_t* select_host, int n_select, float prior_weight, int n_iter, int64_t F,
+                      float* pose_out_dev, float* transl_out_dev, float* cost_dev, void* stream);
+
 /* ------------------------------------------------------------------ ST-GCN primitives
  * dtype is TIK_F32 (SIMT fp32, 1e-4 parity path) or TIK_BF16 (tcgen05 tensor cores, fp32 accumulate). */
 

@@ -107,6 +107,8 @@ _PROTOS = {
     "tik_lbs": (C.c_int, [C.POINTER(TikLbsModel), C.c_int, vp, vp, vp, C.c_int, vp, i64, vp, i64, vp, vp, C.c_int, vp]),
     "tik_body_keypoints": (C.c_int, [C.POINTER(TikKeypointModel), vp, C.c_int, vp, C.c_int, vp, C.POINTER(i32), C.c_int, i64, vp,
                                      vp]),
+    "tik_fit_keypoints": (C.c_int, [C.POINTER(TikKeypointModel), vp, vp, C.c_int, vp, vp, C.c_int, vp, C.c_int, C.POINTER(i32),
+                                    C.c_int, f32, C.c_int, i64, vp, vp, vp, vp]),
     "tik_stem_gcn": (C.c_int, [C.c_int, vp, vp, vp, vp, vp, vp, vp, vp, vp, C.c_int, i64, C.c_int, C.c_int, C.c_int,
                                C.c_int, C.c_int, C.c_int, vp]),
     "tik_aggregate": (C.c_int, [C.c_int, vp, vp, vp, i64, C.c_int, C.c_int, C.c_int, C.c_int, vp]),

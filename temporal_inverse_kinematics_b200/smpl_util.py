@@ -353,6 +353,87 @@ def keypoints(pose, model, betas=None, transl=None, select="coco"):
     return out
 
 
+FIT_PRIOR_WEIGHT = 1e-3          # 1 rad away from init_pose costs as much as a 3 cm miss of one point at weight 1
+
+
+def fit_keypoints(target, model, init_pose, betas=None, transl=None, select="coco", weights=None,
+                  prior_weight=FIT_PRIOR_WEIGHT, n_iter=10, fit_transl=True):
+    """Body poses whose ``keypoints`` hit ``target``: per frame, ``n_iter`` Levenberg-Marquardt steps (one
+    ``tik_fit_keypoints`` launch, one warp per frame) on
+
+        E = sum_k w_k |keypoints(pose, model, betas, transl, select)[k] - target[k]|^2 + prior_weight |pose - init_pose|^2
+
+    over the rotations of joints 0..21 and, with ``fit_transl``, the translation.  target (F, n, 3) CUDA tensor, n the
+    length of ``select`` ('coco' or names from ``keypoint_names()``); model, betas: as ``keypoints``; init_pose (F, 22, 3)
+    or (F, 66) (``run_inference``'s rows), the start and the prior's centre; transl (F, 3) CUDA tensor or None (zero):
+    the start (``fit_transl``) or the fixed translation; weights None (all 1), n non-negative values for every frame or a
+    CUDA tensor (F, n); prior_weight > 0.  A point that the observation does not really have (e.g. the face points that
+    ``moveai_to_coco`` synthesises from the ears) should get weight 0.  E never increases; a frame whose initial E is not
+    finite comes back unchanged with cost NaN.
+    Returns {"poses": (F, 22, 3), "transl": (F, 3), "cost_init": (F,), "cost": (F,)}, fp32 CUDA tensors."""
+    if not isinstance(model, (SmplxBodyModel, SyntheticBodyModel)):
+        raise TypeError("fit_keypoints needs a SmplxBodyModel or a SyntheticBodyModel(skeleton='full')")
+    model.check_keypoints()
+    sel = keypoint_indices(select)
+    n = len(sel)
+    for name, t in (("target", target), ("init_pose", init_pose), ("transl", transl), ("betas", betas), ("weights", weights)):
+        if torch.is_tensor(t) and not t.is_cuda or (name in ("target", "init_pose") and not torch.is_tensor(t)):
+            raise RuntimeError(f"fit_keypoints: {name} must be a CUDA tensor -- there is no CPU fallback")
+    if transl is not None and not torch.is_tensor(transl):
+        raise RuntimeError("fit_keypoints: transl must be a CUDA tensor -- there is no CPU fallback")
+    if target.dim() != 3 or target.shape[1] != n or target.shape[2] != 3:
+        raise ValueError(f"fit_keypoints: target must be (F, {n}, 3) for the {n} selected points, got {tuple(target.shape)}")
+    F, dev = target.shape[0], target.device
+    if tuple(init_pose.shape) not in ((F, 22, 3), (F, 66)):
+        raise ValueError(f"fit_keypoints: init_pose must be ({F}, 22, 3) or ({F}, 66), got {tuple(init_pose.shape)}")
+    for name, t in (("init_pose", init_pose), ("transl", transl), ("betas", betas), ("weights", weights)):
+        if torch.is_tensor(t) and t.device != dev:
+            raise ValueError(f"fit_keypoints: {name} is on {t.device}, target on {dev}")
+    if transl is not None and tuple(transl.shape) != (F, 3):
+        raise ValueError(f"fit_keypoints: transl must be ({F}, 3), got {tuple(transl.shape)}")
+    prior_weight = float(prior_weight)
+    if not (prior_weight > 0 and np.isfinite(prior_weight)):
+        raise ValueError(f"fit_keypoints: prior_weight must be positive and finite, got {prior_weight}")
+    if int(n_iter) != n_iter or n_iter < 0:
+        raise ValueError(f"fit_keypoints: n_iter must be a non-negative integer, got {n_iter}")
+    w, w_per_frame = None, 0
+    if torch.is_tensor(weights) and weights.dim() == 2:
+        if tuple(weights.shape) != (F, n):
+            raise ValueError(f"fit_keypoints: per-frame weights must be ({F}, {n}), got {tuple(weights.shape)}")
+        w, w_per_frame = _aligned(weights), 1
+    elif weights is not None:
+        v = (weights.detach().float().cpu().numpy() if torch.is_tensor(weights) else np.asarray(weights, dtype=np.float32)).reshape(-1)
+        if v.shape[0] != n:
+            raise ValueError(f"fit_keypoints: weights must have {n} values (one per selected point), got {v.shape[0]}")
+        if not (v >= 0).all():
+            raise ValueError("fit_keypoints: weights must be non-negative")
+        w = torch.from_numpy(np.ascontiguousarray(v)).to(dev)
+    pack = model.keypoint_pack(dev)
+    B = pack.n_betas
+    per_frame, b = 0, None
+    if torch.is_tensor(betas) and betas.dim() == 2:
+        if betas.shape[0] != F or betas.shape[1] > min(SMPLX_NUM_BETAS, B):
+            raise ValueError(f"fit_keypoints: per-frame betas must be ({F}, <= {min(SMPLX_NUM_BETAS, B)}), got {tuple(betas.shape)}")
+        b = _aligned(torch.nn.functional.pad(betas.detach().float(), (0, B - betas.shape[1])))
+        per_frame = 1
+    elif betas is not None:
+        v = (betas.detach().float().cpu().numpy() if torch.is_tensor(betas) else np.asarray(betas, dtype=np.float32)).reshape(-1)
+        if v.shape[0] > min(SMPLX_NUM_BETAS, B):
+            raise ValueError(f"fit_keypoints: at most {min(SMPLX_NUM_BETAS, B)} betas, got {v.shape[0]}")
+        b = torch.from_numpy(np.pad(v, (0, B - v.shape[0]))).to(dev)
+    y, pose0 = _aligned(target), _aligned(init_pose.reshape(F, 22, 3))
+    tr = None if transl is None else _aligned(transl)
+    poses = torch.empty((F, 22, 3), dtype=torch.float32, device=dev)
+    transl_out = torch.empty((F, 3), dtype=torch.float32, device=dev)
+    cost = torch.empty((F, 2), dtype=torch.float32, device=dev)
+    sel_c = (C.c_int32 * n)(*sel)
+    with L.on_device(dev):
+        L.check(L.lib().tik_fit_keypoints(C.byref(pack.c), L.ptr(y), L.ptr(w), w_per_frame, L.ptr(pose0), L.ptr(b), per_frame,
+                                          L.ptr(tr), int(bool(fit_transl)), sel_c, n, prior_weight, int(n_iter), F,
+                                          L.ptr(poses), L.ptr(transl_out), L.ptr(cost), L.stream_ptr(dev)))
+    return {"poses": poses, "transl": transl_out, "cost_init": cost[:, 0], "cost": cost[:, 1]}
+
+
 def run_smpl_keypoints(data, smplx_models, device, apply_trans=True, apply_root_rot=True, apply_shape=True):
     """COCO-17 keypoints (F, 17, 3) numpy of the same ``data`` dict and flags as ``run_smpl_inference``: equal to
     ``smplx_joints_to_coco(run_smpl_inference(...))`` on a full-skeleton model, from one ``keypoints`` launch (the body of
