@@ -177,6 +177,35 @@ int tik_fit_keypoints(const TikKeypointModel* m, const float* target_dev, const 
                       int fit_transl, const int32_t* select_host, int n_select, float prior_weight, int n_iter, int64_t F,
                       float* pose_out_dev, float* transl_out_dev, float* cost_dev, void* stream);
 
+/* One body shape per sequence and a pose per frame: sequences s = 0..n_seqs-1 packed back to back, sequence s the frames
+ * [frame_start[s], frame_start[s+1]), and per sequence Levenberg-Marquardt steps on
+ *   E_s = sum_{f in s} [ sum_k w_fk |kp_k(theta_f, beta_s, tau_f) - y_fk|^2 + prior_weight |theta_f - theta0_f|^2 ]
+ *         + shape_prior_weight |beta_s|^2
+ * over beta_s (the model's B = n_betas >= 1 shape coefficients), theta_f and, with fit_transl = 1, tau_f.  The schedule is
+ * tik_fit_keypoints' applied per sequence: mu_s starts at 1e-3, each iteration solves the damped system of all the
+ * sequence's unknowns, (H + mu diag(H)) delta = -g, by a Schur complement on the betas (frame blocks in fp32, the B x B
+ * system summed and solved in fp64) and takes the step iff E_s drops strictly; a non-positive pivot in any frame block or
+ * in the B x B system is a rejection.  n_iter counts solves; E_s never increases.
+ *   m, target_dev, weights_dev, weights_per_frame, init_pose_dev, transl_dev, fit_transl, select_host, n_select,
+ *   prior_weight, n_iter, F: as tik_fit_keypoints.
+ *   frame_start_dev: n_seqs + 1 int64 DEVICE entries (TikSeqBatch): non-decreasing, [0] = 0, [n_seqs] = F, every sequence
+ *   at least one frame (n_seqs >= 1 iff F >= 1); indices from a malformed table are clamped into the buffers.
+ *   betas_init_dev (n_seqs, B) or NULL (zero): the start of each beta_s; shape_prior_weight > 0 (the prior is centred on
+ *   the mean shape, beta = 0).
+ *   workspace_dev: 256-byte aligned, workspace_bytes >= tik_fit_keypoints_shape_workspace_bytes (~17 KB per frame).
+ *   pose_out_dev (F,22,3); transl_out_dev (F,3) or NULL; betas_out_dev (n_seqs, B); cost_dev (n_seqs, 2) [initial E_s,
+ *   final E_s] or NULL.  A sequence whose initial E_s is not finite is returned unchanged with final cost NaN.
+ * A sequence's results do not depend on the other sequences of the call or on its position.  No host synchronisation,
+ * CUDA-graph capturable; F = 0 is a no-op; outputs may not overlap inputs, the workspace or each other (checked). */
+int tik_fit_keypoints_shape_workspace_bytes(const TikKeypointModel* m, int n_select, int fit_transl, int64_t F,
+                                            int64_t n_seqs, int64_t* bytes);
+int tik_fit_keypoints_shape(const TikKeypointModel* m, const float* target_dev, const float* weights_dev,
+                            int weights_per_frame, const float* init_pose_dev, const float* transl_dev, int fit_transl,
+                            const int64_t* frame_start_dev, int64_t n_seqs, const float* betas_init_dev,
+                            float shape_prior_weight, const int32_t* select_host, int n_select, float prior_weight,
+                            int n_iter, int64_t F, void* workspace_dev, int64_t workspace_bytes, float* pose_out_dev,
+                            float* transl_out_dev, float* betas_out_dev, float* cost_dev, void* stream);
+
 /* ------------------------------------------------------------------ ST-GCN primitives
  * dtype is TIK_F32 (SIMT fp32, 1e-4 parity path) or TIK_BF16 (tcgen05 tensor cores, fp32 accumulate). */
 

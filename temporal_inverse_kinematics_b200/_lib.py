@@ -109,6 +109,10 @@ _PROTOS = {
                                      vp]),
     "tik_fit_keypoints": (C.c_int, [C.POINTER(TikKeypointModel), vp, vp, C.c_int, vp, vp, C.c_int, vp, C.c_int, C.POINTER(i32),
                                     C.c_int, f32, C.c_int, i64, vp, vp, vp, vp]),
+    "tik_fit_keypoints_shape_workspace_bytes": (C.c_int, [C.POINTER(TikKeypointModel), C.c_int, C.c_int, i64, i64,
+                                                          C.POINTER(i64)]),
+    "tik_fit_keypoints_shape": (C.c_int, [C.POINTER(TikKeypointModel), vp, vp, C.c_int, vp, vp, C.c_int, vp, i64, vp, f32,
+                                          C.POINTER(i32), C.c_int, f32, C.c_int, i64, vp, i64, vp, vp, vp, vp, vp]),
     "tik_stem_gcn": (C.c_int, [C.c_int, vp, vp, vp, vp, vp, vp, vp, vp, vp, C.c_int, i64, C.c_int, C.c_int, C.c_int,
                                C.c_int, C.c_int, C.c_int, vp]),
     "tik_aggregate": (C.c_int, [C.c_int, vp, vp, vp, i64, C.c_int, C.c_int, C.c_int, C.c_int, vp]),

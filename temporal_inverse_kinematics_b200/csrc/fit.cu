@@ -17,377 +17,13 @@
 //     rebuilt after every accepted step) and two substitutions; then one forward at the candidate.
 // Every loop and reduction of a frame runs in an order fixed by the frame's own data and lane ids, so a frame's result
 // does not depend on the other frames of the call or on its warp slot.
-#include <math.h>
 #include <string.h>
 
 #include <algorithm>
 
-#include "fk_device.cuh"
+#include "fit_device.cuh"
 
 namespace tik {
-
-constexpr int kFitJ = 55;
-constexpr int kFitBody = 22;                              // joints with unknown rotations (0..21)
-constexpr int kFitPose = 3 * kFitBody;                    // 66
-constexpr int kFitMaxP = kFitPose + 3;                    // + translation
-constexpr int kFitPitch = 72;                             // row pitch of J and length of the x vectors: 18 tiles of 4
-constexpr int kFitTri = kFitMaxP * (kFitMaxP + 1) / 2;    // packed lower triangle of the 69 x 69 system
-constexpr int kFitFeat = (kFitBody - 1) * 9;              // pose-blend features of joints 1..21
-constexpr int kFitMaxWarps = 8;
-constexpr int kFitMaxLevels = 16;
-
-struct FitParams {
-  const float* jt; const float* jd;
-  const float* lm_t; const float* lm_d; const float* lm_pd;
-  const int32_t* skin_idx; const float* skin_w;
-  const float* target; const float* weights; const float* init_pose; const float* betas; const float* transl;
-  float* pose_out; float* transl_out; float* cost;
-  int64_t F;
-  int n_betas, n_lm, kmax, n_sel, weights_per_frame, betas_per_frame, P, n_iter, warps, n_levels;
-  float prior;
-  unsigned long long anc[kFitJ];                          // bit a of anc[j]: joint a is j or an ancestor of j
-  int8_t par[kFitJ];
-  int8_t order[kFitJ];                                    // joints sorted by tree depth
-  int8_t level[kFitMaxLevels + 1];                        // order[level[d] .. level[d+1]) have depth d
-  int8_t sel[TIK_KP_MAX_SELECT];                          // point index of each selected point
-};
-
-// Shared-memory layout in floats, every region 16-byte aligned: CTA tables, then one slice per warp.
-struct FitSmem {
-  int pd, jt, jd, lmt, lmd, w, anc, cta;                  // CTA tables (offsets from 0)
-  int U, H, g, b, x, x0, xc, y, wr, res, beta, rest, psh, p, v, Rl, Rg, t, M, D, warp;   // offsets in a warp slice
-};
-__host__ __device__ inline FitSmem fit_smem(int n_sel, int L, int B, bool has_pd) {
-  auto up = [](int n) { return (n + 3) / 4 * 4; };
-  FitSmem s;
-  int o = 0;
-  s.pd = o;   o += up(has_pd ? 3 * L * kFitFeat : 0);
-  s.jt = o;   o += up(kFitJ * 3);
-  s.jd = o;   o += up(kFitJ * 3 * B);
-  s.lmt = o;  o += up(3 * L);
-  s.lmd = o;  o += up(3 * L * B);
-  s.w = o;    o += up(L * kFitJ);
-  s.anc = o;  o += up(2 * kFitJ);
-  s.cta = o;
-  const int R = 3 * n_sel;
-  o = 0;
-  s.U = o;    o += up(R * kFitPitch > kFitTri ? R * kFitPitch : kFitTri);   // J, then the factor of the damped system
-  s.H = o;    o += up(kFitTri);
-  s.g = o;    o += kFitPitch;
-  s.b = o;    o += kFitPitch;
-  s.x = o;    o += kFitPitch;
-  s.x0 = o;   o += kFitPitch;
-  s.xc = o;   o += kFitPitch;
-  s.y = o;    o += up(R);
-  s.wr = o;   o += up(R);
-  s.res = o;  o += up(R);
-  s.beta = o; o += up(TIK_KP_MAX_BETAS);
-  s.rest = o; o += up(kFitJ * 3);
-  s.psh = o;  o += up(3 * L);
-  s.p = o;    o += up(3 * L);
-  s.v = o;    o += up(3 * L);
-  s.Rl = o;   o += up(kFitBody * 9);
-  s.Rg = o;   o += up(kFitJ * 9);
-  s.t = o;    o += up(kFitJ * 3);
-  s.M = o;    o += up(kFitBody * 9);
-  s.D = o;    o += up(has_pd ? (kFitBody - 1) * 27 : 0);
-  s.warp = o;
-  return s;
-}
-
-struct FitCta { const float *pd, *jt, *jd, *lmt, *lmd, *w; const unsigned long long* anc; };
-struct FitWarp { float *U, *H, *g, *b, *x, *x0, *xc, *y, *wr, *res, *beta, *rest, *psh, *p, *v, *Rl, *Rg, *t, *M, *D; };
-
-__device__ __forceinline__ float fit_warp_sum(float v) {
-  // xor butterfly: every lane ends with the same bits (each step adds the same two partial sums on both sides)
-#pragma unroll
-  for (int o = 16; o; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-  return v;
-}
-__device__ __forceinline__ int tri(int i) { return i * (i + 1) / 2; }
-
-// Keypoints of the pose xv (theta, tau), residuals and cost; leaves the frame's FK state (Rl, Rg, t, p) in shared memory.
-__device__ float fit_forward(const FitParams& p, const FitCta& c, const FitWarp& s, const float* xv, int lane) {
-  const int L = p.n_lm, R = 3 * p.n_sel;
-  if (lane < kFitBody) {
-    float Rm[9];
-    rodrigues_q_fast(xv[lane * 3], xv[lane * 3 + 1], xv[lane * 3 + 2], Rm);
-#pragma unroll
-    for (int e = 0; e < 9; ++e) s.Rl[lane * 9 + e] = Rm[e];
-  }
-  __syncwarp();
-  for (int d = 0; d < p.n_levels; ++d) {
-    for (int i = p.level[d] + lane; i < p.level[d + 1]; i += 32) {
-      const int j = p.order[i], par = p.par[j];
-      float* G = s.Rg + j * 9;
-      float* tj = s.t + j * 3;
-      if (par < 0) {
-#pragma unroll
-        for (int e = 0; e < 9; ++e) G[e] = s.Rl[j * 9 + e];
-        tj[0] = s.rest[j * 3]; tj[1] = s.rest[j * 3 + 1]; tj[2] = s.rest[j * 3 + 2];
-      } else {
-        const float* GP = s.Rg + par * 9;
-        const float* tp = s.t + par * 3;
-        const float d0 = s.rest[j * 3] - s.rest[par * 3], d1 = s.rest[j * 3 + 1] - s.rest[par * 3 + 1],
-                    d2 = s.rest[j * 3 + 2] - s.rest[par * 3 + 2];
-#pragma unroll
-        for (int r = 0; r < 3; ++r) {
-          if (j < kFitBody) {
-            const float* Rm = s.Rl + j * 9;
-#pragma unroll
-            for (int cc = 0; cc < 3; ++cc)
-              G[r * 3 + cc] = GP[r * 3] * Rm[cc] + GP[r * 3 + 1] * Rm[3 + cc] + GP[r * 3 + 2] * Rm[6 + cc];
-          } else {
-            G[r * 3] = GP[r * 3]; G[r * 3 + 1] = GP[r * 3 + 1]; G[r * 3 + 2] = GP[r * 3 + 2];
-          }
-          tj[r] = GP[r * 3] * d0 + GP[r * 3 + 1] * d1 + GP[r * 3 + 2] * d2 + tp[r];
-        }
-      }
-    }
-    __syncwarp();
-  }
-  if (lane < 3 * L) {                                      // landmark rest positions: shape + pose blend
-    float acc = 0.f;
-    if (c.pd != nullptr) {
-      const float* row = c.pd + lane * kFitFeat;
-      for (int j = 1; j < kFitBody; ++j)
-#pragma unroll
-        for (int e = 0; e < 9; ++e)
-          acc = fmaf(row[(j - 1) * 9 + e], s.Rl[j * 9 + e] - (e % 4 == 0 ? 1.f : 0.f), acc);
-    }
-    s.p[lane] = s.psh[lane] + acc;
-  }
-  __syncwarp();
-  if (lane < 3 * L) {                                      // skinning: v_l = sum_m w_lm (Rg_m (p_l - rest_m) + t_m)
-    const int l = lane / 3, cc = lane % 3;
-    float v = 0.f;
-    for (int m = 0; m < kFitJ; ++m) {
-      const float w = c.w[l * kFitJ + m];
-      if (w != 0.f) {
-        const float qx = s.p[l * 3] - s.rest[m * 3], qy = s.p[l * 3 + 1] - s.rest[m * 3 + 1],
-                    qz = s.p[l * 3 + 2] - s.rest[m * 3 + 2];
-        const float* G = s.Rg + m * 9 + cc * 3;
-        v = fmaf(w, fmaf(G[0], qx, fmaf(G[1], qy, fmaf(G[2], qz, s.t[m * 3 + cc]))), v);
-      }
-    }
-    s.v[lane] = v;
-  }
-  __syncwarp();
-  float e = 0.f, pr = 0.f;
-  for (int i = lane; i < R; i += 32) {
-    const int k = i / 3, cc = i % 3, q = p.sel[k];
-    const float kp = (q < kFitJ ? s.t[q * 3 + cc] : s.v[(q - kFitJ) * 3 + cc]) + xv[kFitPose + cc];
-    const float r = kp - s.y[i];
-    s.res[i] = r;
-    e = fmaf(s.wr[i] * r, r, e);
-  }
-  for (int i = lane; i < kFitPose; i += 32) {
-    const float dl = xv[i] - s.x0[i];
-    pr = fmaf(dl, dl, pr);
-  }
-  const float E = fit_warp_sum(e) + p.prior * fit_warp_sum(pr);
-  __syncwarp();
-  return E;
-}
-
-// J at the point of the last forward (x), then H (packed, lambda on the pose diagonal) and g.
-__device__ void fit_normal_equations(const FitParams& p, const FitCta& c, const FitWarp& s, int lane) {
-  const int n = p.n_sel, R = 3 * n, P = p.P;
-  const bool has_pd = c.pd != nullptr;
-  if (lane < kFitBody) {
-    // right Jacobian of the exponential map at theta_j, M_j = Rg_j Jr, and D_j,a = R_j [Jr e_a]x for the pose blend
-    const float a0 = s.x[lane * 3], a1 = s.x[lane * 3 + 1], a2 = s.x[lane * 3 + 2];
-    const float phi2 = a0 * a0 + a1 * a1 + a2 * a2;
-    float ca, cb;                                          // Jr = I - ca [a]x + cb [a]x^2
-    if (phi2 < 0.04f) {
-      ca = 0.5f - phi2 * (1.f / 24.f - phi2 * (1.f / 720.f));
-      cb = 1.f / 6.f - phi2 * (1.f / 120.f - phi2 * (1.f / 5040.f));
-    } else {
-      const float phi = sqrtf(phi2), sh = sinf(0.5f * phi);
-      ca = 2.f * sh * sh / phi2;
-      cb = (phi - sinf(phi)) / (phi2 * phi);
-    }
-    const float K[9] = {0.f, -a2, a1, a2, 0.f, -a0, -a1, a0, 0.f};
-    float Jr[9];
-#pragma unroll
-    for (int r = 0; r < 3; ++r)
-#pragma unroll
-      for (int cc = 0; cc < 3; ++cc) {
-        const float k2 = K[r * 3] * K[cc] + K[r * 3 + 1] * K[3 + cc] + K[r * 3 + 2] * K[6 + cc];
-        Jr[r * 3 + cc] = (r == cc ? 1.f : 0.f) - ca * K[r * 3 + cc] + cb * k2;
-      }
-    const float* G = s.Rg + lane * 9;
-#pragma unroll
-    for (int r = 0; r < 3; ++r)
-#pragma unroll
-      for (int cc = 0; cc < 3; ++cc)
-        s.M[lane * 9 + r * 3 + cc] = G[r * 3] * Jr[cc] + G[r * 3 + 1] * Jr[3 + cc] + G[r * 3 + 2] * Jr[6 + cc];
-    if (has_pd && lane >= 1) {
-      const float* Rm = s.Rl + lane * 9;
-#pragma unroll
-      for (int a = 0; a < 3; ++a) {
-        const float u0 = Jr[a], u1 = Jr[3 + a], u2 = Jr[6 + a];
-        const float S[9] = {0.f, -u2, u1, u2, 0.f, -u0, -u1, u0, 0.f};
-#pragma unroll
-        for (int r = 0; r < 3; ++r)
-#pragma unroll
-          for (int cc = 0; cc < 3; ++cc)
-            s.D[(lane - 1) * 27 + a * 9 + r * 3 + cc] = Rm[r * 3] * S[cc] + Rm[r * 3 + 1] * S[3 + cc] + Rm[r * 3 + 2] * S[6 + cc];
-      }
-    }
-  }
-  float4* U4 = reinterpret_cast<float4*>(s.U);
-  for (int i = lane; i < R * (kFitPitch / 4); i += 32) U4[i] = make_float4(0.f, 0.f, 0.f, 0.f);
-  __syncwarp();
-  for (int pi = lane; pi < n * kFitBody; pi += 32) {
-    const int k = pi / kFitBody, j = pi % kFitBody, q = p.sel[k];
-    const float* Mj = s.M + j * 9;
-    float blk[9];
-    bool nz = false;
-    if (q < kFitJ) {
-      if (q != j && ((c.anc[q] >> j) & 1ull)) {            // joint point below j: rotation about t_j
-        const float d0 = s.t[q * 3] - s.t[j * 3], d1 = s.t[q * 3 + 1] - s.t[j * 3 + 1], d2 = s.t[q * 3 + 2] - s.t[j * 3 + 2];
-#pragma unroll
-        for (int a = 0; a < 3; ++a) {                      // column a: M_a x d
-          const float m0 = Mj[a], m1 = Mj[3 + a], m2 = Mj[6 + a];
-          blk[a] = m1 * d2 - m2 * d1; blk[3 + a] = m2 * d0 - m0 * d2; blk[6 + a] = m0 * d1 - m1 * d0;
-        }
-        nz = true;
-      }
-    } else {
-      const int l = q - kFitJ;
-      float s0 = 0.f, s1 = 0.f, s2 = 0.f, A[9] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
-      const float* pl = s.p + l * 3;
-      for (int m = 0; m < kFitJ; ++m) {
-        const float w = c.w[l * kFitJ + m];
-        if (w == 0.f) continue;
-        const float* G = s.Rg + m * 9;
-        if (has_pd)
-#pragma unroll
-          for (int e = 0; e < 9; ++e) A[e] = fmaf(w, G[e], A[e]);
-        if ((c.anc[m] >> j) & 1ull) {                      // x_lm - t_j for every skinning joint m below (or at) j
-          const float qx = pl[0] - s.rest[m * 3], qy = pl[1] - s.rest[m * 3 + 1], qz = pl[2] - s.rest[m * 3 + 2];
-          s0 = fmaf(w, fmaf(G[0], qx, fmaf(G[1], qy, fmaf(G[2], qz, s.t[m * 3]))) - s.t[j * 3], s0);
-          s1 = fmaf(w, fmaf(G[3], qx, fmaf(G[4], qy, fmaf(G[5], qz, s.t[m * 3 + 1]))) - s.t[j * 3 + 1], s1);
-          s2 = fmaf(w, fmaf(G[6], qx, fmaf(G[7], qy, fmaf(G[8], qz, s.t[m * 3 + 2]))) - s.t[j * 3 + 2], s2);
-        }
-      }
-#pragma unroll
-      for (int a = 0; a < 3; ++a) {
-        const float m0 = Mj[a], m1 = Mj[3 + a], m2 = Mj[6 + a];
-        blk[a] = m1 * s2 - m2 * s1; blk[3 + a] = m2 * s0 - m0 * s2; blk[6 + a] = m0 * s1 - m1 * s0;
-      }
-      if (has_pd && j >= 1) {                              // (sum_m w_lm Rg_m) . d offset_l / d theta_j
-        const float* D = s.D + (j - 1) * 27;
-        float dp[9];
-#pragma unroll
-        for (int cc = 0; cc < 3; ++cc) {
-          const float* row = c.pd + (l * 3 + cc) * kFitFeat + (j - 1) * 9;
-#pragma unroll
-          for (int a = 0; a < 3; ++a) {
-            float v = 0.f;
-#pragma unroll
-            for (int e = 0; e < 9; ++e) v = fmaf(row[e], D[a * 9 + e], v);
-            dp[cc * 3 + a] = v;
-          }
-        }
-#pragma unroll
-        for (int r = 0; r < 3; ++r)
-#pragma unroll
-          for (int a = 0; a < 3; ++a)
-            blk[r * 3 + a] += A[r * 3] * dp[a] + A[r * 3 + 1] * dp[3 + a] + A[r * 3 + 2] * dp[6 + a];
-      }
-      nz = true;
-    }
-    if (nz)
-#pragma unroll
-      for (int r = 0; r < 3; ++r)
-#pragma unroll
-        for (int a = 0; a < 3; ++a) s.U[(3 * k + r) * kFitPitch + 3 * j + a] = blk[r * 3 + a];
-  }
-  if (P > kFitPose)
-    for (int i = lane; i < R; i += 32) s.U[i * kFitPitch + kFitPose + i % 3] = 1.f;
-  __syncwarp();
-
-  // H: lanes over the 4x4 tiles of the lower triangle, rows in order
-  const int nt = (P + 3) / 4, ntiles = nt * (nt + 1) / 2;
-  for (int ti = lane; ti < ntiles; ti += 32) {
-    int I = 0;
-    while (tri(I + 1) <= ti) ++I;
-    const int Jc = ti - tri(I);
-    float acc[16];
-#pragma unroll
-    for (int e = 0; e < 16; ++e) acc[e] = 0.f;
-    for (int r = 0; r < R; ++r) {
-      const float wr = s.wr[r];
-      const float4 a4 = *reinterpret_cast<const float4*>(s.U + r * kFitPitch + 4 * I);
-      const float4 b4 = *reinterpret_cast<const float4*>(s.U + r * kFitPitch + 4 * Jc);
-      const float wa[4] = {wr * a4.x, wr * a4.y, wr * a4.z, wr * a4.w}, bb[4] = {b4.x, b4.y, b4.z, b4.w};
-#pragma unroll
-      for (int u = 0; u < 4; ++u)
-#pragma unroll
-        for (int v = 0; v < 4; ++v) acc[u * 4 + v] = fmaf(wa[u], bb[v], acc[u * 4 + v]);
-    }
-#pragma unroll
-    for (int u = 0; u < 4; ++u)
-#pragma unroll
-      for (int v = 0; v < 4; ++v) {
-        const int i = 4 * I + u, j = 4 * Jc + v;
-        if (j <= i && i < P) s.H[tri(i) + j] = acc[u * 4 + v] + (i == j && i < kFitPose ? p.prior : 0.f);
-      }
-  }
-  for (int a = lane; a < P; a += 32) {
-    float acc = 0.f;
-    for (int r = 0; r < R; ++r) acc = fmaf(s.wr[r] * s.U[r * kFitPitch + a], s.res[r], acc);
-    s.g[a] = acc + (a < kFitPose ? p.prior * (s.x[a] - s.x0[a]) : 0.f);
-  }
-  __syncwarp();
-}
-
-// (H + mu diag(H)) delta = -g by Cholesky in U; delta in b.  false: a pivot was not positive (or not finite).
-__device__ bool fit_solve(const FitParams& p, const FitWarp& s, float mu, int lane) {
-  const int P = p.P;
-  float* A = s.U;
-  for (int i = lane; i < tri(P); i += 32) A[i] = s.H[i];
-  for (int i = lane; i < P; i += 32) s.b[i] = -s.g[i];
-  __syncwarp();
-  for (int i = lane; i < P; i += 32) A[tri(i) + i] = fmaf(mu, s.H[tri(i) + i], s.H[tri(i) + i]);
-  __syncwarp();
-  for (int k = 0; k < P; ++k) {
-    const float d = A[tri(k) + k];
-    if (!(d > 0.f) || !(d < INFINITY)) return false;      // same value in every lane: the warp leaves together
-    const float lk = sqrtf(d);
-    __syncwarp();
-    for (int i = k + 1 + lane; i < P; i += 32) A[tri(i) + k] /= lk;
-    if (lane == 0) A[tri(k) + k] = lk;
-    __syncwarp();
-    for (int i = k + 1 + lane; i < P; i += 32) {
-      const float lik = A[tri(i) + k];
-      float* row = A + tri(i);
-      int jk = tri(k + 1) + k;
-      for (int j = k + 1; j <= i; ++j) {
-        row[j] = fmaf(-lik, A[jk], row[j]);
-        jk += j + 1;
-      }
-    }
-    __syncwarp();
-  }
-  for (int k = 0; k < P; ++k) {                            // L y = -g
-    const float yk = s.b[k] / A[tri(k) + k];
-    __syncwarp();
-    for (int i = k + 1 + lane; i < P; i += 32) s.b[i] = fmaf(-A[tri(i) + k], yk, s.b[i]);
-    if (lane == 0) s.b[k] = yk;
-    __syncwarp();
-  }
-  for (int k = P - 1; k >= 0; --k) {                       // L^T delta = y
-    const float dk = s.b[k] / A[tri(k) + k];
-    __syncwarp();
-    for (int i = lane; i < k; i += 32) s.b[i] = fmaf(-A[tri(k) + i], dk, s.b[i]);
-    if (lane == 0) s.b[k] = dk;
-    __syncwarp();
-  }
-  return true;
-}
 
 __global__ void __launch_bounds__(kFitMaxWarps * 32)
 fit_keypoints_kernel(const __grid_constant__ FitParams p) {
@@ -489,12 +125,6 @@ fit_keypoints_kernel(const __grid_constant__ FitParams p) {
   }
 }
 
-static bool fit_overlap(const void* a, int64_t na, const void* b, int64_t nb) {
-  if (a == nullptr || b == nullptr || na <= 0 || nb <= 0) return false;
-  const uintptr_t x = (uintptr_t)a, y = (uintptr_t)b;
-  return x < y + (uintptr_t)nb * 4 && y < x + (uintptr_t)na * 4;
-}
-
 }  // namespace tik
 
 extern "C" int tik_fit_keypoints(const TikKeypointModel* m, const float* target_dev, const float* weights_dev,
@@ -503,37 +133,16 @@ extern "C" int tik_fit_keypoints(const TikKeypointModel* m, const float* target_
                                  int n_select, float prior_weight, int n_iter, int64_t F, float* pose_out_dev,
                                  float* transl_out_dev, float* cost_dev, void* stream) {
   using namespace tik;
-  TIK_CHECK_ARG(m != nullptr, "fit_keypoints: null model");
+  const char* fn = "fit_keypoints";
+  TIK_CHECK_ARG(m != nullptr, "%s: null model", fn);
   const int B = m->n_betas, L = m->n_landmarks;
-  TIK_CHECK_ARG(B >= 0 && B <= TIK_KP_MAX_BETAS, "fit_keypoints: n_betas=%d outside [0,%d]", B, TIK_KP_MAX_BETAS);
-  TIK_CHECK_ARG(L >= 0 && L <= TIK_LBS_MAX_LANDMARKS, "fit_keypoints: n_landmarks=%d outside [0,%d]", L, TIK_LBS_MAX_LANDMARKS);
-  TIK_CHECK_ARG(m->joint_template_dev != nullptr && (m->joint_dirs_dev != nullptr) == (B > 0),
-                "fit_keypoints: joint_template_dev must be set and joint_dirs_dev set iff n_betas > 0");
-  if (L > 0) {
-    TIK_CHECK_ARG(m->kmax >= 1 && m->kmax <= kFitJ, "fit_keypoints: kmax=%d outside [1,%d]", m->kmax, kFitJ);
-    TIK_CHECK_ARG(m->lm_template_dev && m->lm_skin_idx_dev && m->lm_skin_w_dev && (m->lm_dirs_dev != nullptr) == (B > 0),
-                  "fit_keypoints: landmark arrays missing (lm_dirs_dev must be set iff n_betas > 0)");
-  }
-  TIK_CHECK_ARG(weights_per_frame == 0 || weights_per_frame == 1, "fit_keypoints: weights_per_frame=%d must be 0 or 1",
-                weights_per_frame);
-  TIK_CHECK_ARG(!(weights_per_frame && weights_dev == nullptr), "fit_keypoints: per-frame weights need weights_dev");
+  if (int rc = fit_check_model(m, fn)) return rc;
+  if (int rc = fit_check_weights(weights_dev, weights_per_frame, fn)) return rc;
   TIK_CHECK_ARG(betas_per_frame == 0 || betas_per_frame == 1, "fit_keypoints: betas_per_frame=%d must be 0 or 1", betas_per_frame);
   TIK_CHECK_ARG(!(betas_per_frame && betas_dev == nullptr && B > 0), "fit_keypoints: per-frame betas need betas_dev");
-  TIK_CHECK_ARG(fit_transl == 0 || fit_transl == 1, "fit_keypoints: fit_transl=%d must be 0 or 1", fit_transl);
-  TIK_CHECK_ARG(n_select >= 1 && n_select <= TIK_KP_MAX_SELECT, "fit_keypoints: n_select=%d outside [1,%d]", n_select,
-                TIK_KP_MAX_SELECT);
-  TIK_CHECK_ARG(select_host != nullptr, "fit_keypoints: null select_host");
-  TIK_CHECK_ARG(prior_weight > 0.f && prior_weight < INFINITY, "fit_keypoints: prior_weight=%g must be positive and finite",
-                (double)prior_weight);
-  TIK_CHECK_ARG(n_iter >= 0, "fit_keypoints: n_iter=%d must be >= 0", n_iter);
-  TIK_CHECK_ARG(F >= 0, "fit_keypoints: negative frame count");
   FitParams p;
   memset(&p, 0, sizeof(p));
-  for (int s = 0; s < n_select; ++s) {
-    const int q = select_host[s];
-    TIK_CHECK_ARG(q >= 0 && q < kFitJ + L, "fit_keypoints: select[%d]=%d outside [0,%d)", s, q, kFitJ + L);
-    p.sel[s] = (int8_t)q;
-  }
+  if (int rc = fit_check_solver(m, fit_transl, select_host, n_select, prior_weight, n_iter, F, &p, fn)) return rc;
   if (F == 0) return TIK_OK;
   TIK_CHECK_ARG(target_dev != nullptr && init_pose_dev != nullptr && pose_out_dev != nullptr, "fit_keypoints: null pointer");
   const bool use_betas = B > 0 && betas_dev != nullptr;
@@ -550,36 +159,14 @@ extern "C" int tik_fit_keypoints(const TikKeypointModel* m, const float* target_
       TIK_CHECK_ARG(!fit_overlap(outs[o], out_n[o], outs[o2], out_n[o2]), "fit_keypoints: outputs %d and %d overlap", o, o2);
   }
 
-  p.jt = m->joint_template_dev; p.jd = m->joint_dirs_dev;
-  p.lm_t = m->lm_template_dev; p.lm_d = m->lm_dirs_dev; p.lm_pd = m->lm_posedirs_dev;
-  p.skin_idx = m->lm_skin_idx_dev; p.skin_w = m->lm_skin_w_dev;
+  fit_model_params(m, &p);
   p.target = target_dev; p.weights = weights_dev; p.init_pose = init_pose_dev;
   p.betas = use_betas ? betas_dev : nullptr; p.transl = transl_dev;
   p.pose_out = pose_out_dev; p.transl_out = transl_out_dev; p.cost = cost_dev;
   p.F = F;
   p.n_betas = use_betas ? B : 0;          // no betas: the shape directions are not read at all
-  p.n_lm = L; p.kmax = L > 0 ? m->kmax : 0; p.n_sel = n_select;
   p.weights_per_frame = weights_dev != nullptr ? weights_per_frame : 0;
   p.betas_per_frame = use_betas ? betas_per_frame : 0;
-  p.P = fit_transl ? kFitMaxP : kFitPose;
-  p.n_iter = n_iter; p.prior = prior_weight;
-  // tree tables: ancestors (parents precede children), depth order
-  int depth[kFitJ], maxd = 0;
-  for (int j = 0; j < kFitJ; ++j) {
-    const int par = f60_parent(j);
-    p.par[j] = (int8_t)par;
-    p.anc[j] = (par < 0 ? 0ull : p.anc[par]) | (1ull << j);
-    depth[j] = par < 0 ? 0 : depth[par] + 1;
-    maxd = std::max(maxd, depth[j]);
-  }
-  p.n_levels = maxd + 1;
-  int o = 0;
-  for (int d = 0; d <= maxd; ++d) {
-    p.level[d] = (int8_t)o;
-    for (int j = 0; j < kFitJ; ++j)
-      if (depth[j] == d) p.order[o++] = (int8_t)j;
-  }
-  p.level[maxd + 1] = (int8_t)o;
 
   // The model tables never need more than B = 16 directions; size the launch by the call's own shapes.
   const bool has_pd = p.lm_pd != nullptr && L > 0;

@@ -260,7 +260,7 @@ static int run_impl(TikPlan* P, const float* x, const TikWindowing& win, const W
 
 extern "C" {
 
-int tik_version(void) { return 103; }
+int tik_version(void) { return 104; }
 const char* tik_last_error(void) { return tik::g_err; }
 
 int tik_check_device(void) {

@@ -356,6 +356,61 @@ def keypoints(pose, model, betas=None, transl=None, select="coco"):
 FIT_PRIOR_WEIGHT = 1e-3          # 1 rad away from init_pose costs as much as a 3 cm miss of one point at weight 1
 
 
+def _fit_args(fn, target, model, init_pose, transl, weights, prior_weight, n_iter, select, **tensors):
+    """The argument checks that fit_keypoints and fit_keypoints_shape share (``fn`` names the caller in the messages;
+    ``tensors`` are further optional inputs that must be CUDA tensors on target's device when they are tensors).
+    Returns the selection, the frame count, the device, the keypoint pack and the device inputs."""
+    if not isinstance(model, (SmplxBodyModel, SyntheticBodyModel)):
+        raise TypeError(f"{fn} needs a SmplxBodyModel or a SyntheticBodyModel(skeleton='full')")
+    model.check_keypoints()
+    sel = keypoint_indices(select)
+    n = len(sel)
+    opt = [("transl", transl), *tensors.items(), ("weights", weights)]
+    for name, t in [("target", target), ("init_pose", init_pose), *opt]:
+        if torch.is_tensor(t) and not t.is_cuda or (name in ("target", "init_pose") and not torch.is_tensor(t)):
+            raise RuntimeError(f"{fn}: {name} must be a CUDA tensor -- there is no CPU fallback")
+    if transl is not None and not torch.is_tensor(transl):
+        raise RuntimeError(f"{fn}: transl must be a CUDA tensor -- there is no CPU fallback")
+    if target.dim() != 3 or target.shape[1] != n or target.shape[2] != 3:
+        raise ValueError(f"{fn}: target must be (F, {n}, 3) for the {n} selected points, got {tuple(target.shape)}")
+    F, dev = target.shape[0], target.device
+    if tuple(init_pose.shape) not in ((F, 22, 3), (F, 66)):
+        raise ValueError(f"{fn}: init_pose must be ({F}, 22, 3) or ({F}, 66), got {tuple(init_pose.shape)}")
+    for name, t in [("init_pose", init_pose), *opt]:
+        if torch.is_tensor(t) and t.device != dev:
+            raise ValueError(f"{fn}: {name} is on {t.device}, target on {dev}")
+    if transl is not None and tuple(transl.shape) != (F, 3):
+        raise ValueError(f"{fn}: transl must be ({F}, 3), got {tuple(transl.shape)}")
+    prior_weight = float(prior_weight)
+    if not (prior_weight > 0 and np.isfinite(prior_weight)):
+        raise ValueError(f"{fn}: prior_weight must be positive and finite, got {prior_weight}")
+    if int(n_iter) != n_iter or n_iter < 0:
+        raise ValueError(f"{fn}: n_iter must be a non-negative integer, got {n_iter}")
+    w, w_per_frame = None, 0
+    if torch.is_tensor(weights) and weights.dim() == 2:
+        if tuple(weights.shape) != (F, n):
+            raise ValueError(f"{fn}: per-frame weights must be ({F}, {n}), got {tuple(weights.shape)}")
+        w, w_per_frame = _aligned(weights), 1
+    elif weights is not None:
+        v = (weights.detach().float().cpu().numpy() if torch.is_tensor(weights) else np.asarray(weights, dtype=np.float32)).reshape(-1)
+        if v.shape[0] != n:
+            raise ValueError(f"{fn}: weights must have {n} values (one per selected point), got {v.shape[0]}")
+        if not (v >= 0).all():
+            raise ValueError(f"{fn}: weights must be non-negative")
+        w = torch.from_numpy(np.ascontiguousarray(v)).to(dev)
+    return dict(sel=sel, n=n, F=F, dev=dev, pack=model.keypoint_pack(dev), w=w, w_per_frame=w_per_frame,
+                y=_aligned(target), pose0=_aligned(init_pose.reshape(F, 22, 3)),
+                tr=None if transl is None else _aligned(transl), prior_weight=prior_weight)
+
+
+def _betas_vector(fn, betas, B, dev):
+    """One beta vector (at most min(10, B) values) -> (B,) fp32 on dev, zero-padded."""
+    v = (betas.detach().float().cpu().numpy() if torch.is_tensor(betas) else np.asarray(betas, dtype=np.float32)).reshape(-1)
+    if v.shape[0] > min(SMPLX_NUM_BETAS, B):
+        raise ValueError(f"{fn}: at most {min(SMPLX_NUM_BETAS, B)} betas, got {v.shape[0]}")
+    return torch.from_numpy(np.pad(v, (0, B - v.shape[0]))).to(dev)
+
+
 def fit_keypoints(target, model, init_pose, betas=None, transl=None, select="coco", weights=None,
                   prior_weight=FIT_PRIOR_WEIGHT, n_iter=10, fit_transl=True):
     """Body poses whose ``keypoints`` hit ``target``: per frame, ``n_iter`` Levenberg-Marquardt steps (one
@@ -371,44 +426,9 @@ def fit_keypoints(target, model, init_pose, betas=None, transl=None, select="coc
     ``moveai_to_coco`` synthesises from the ears) should get weight 0.  E never increases; a frame whose initial E is not
     finite comes back unchanged with cost NaN.
     Returns {"poses": (F, 22, 3), "transl": (F, 3), "cost_init": (F,), "cost": (F,)}, fp32 CUDA tensors."""
-    if not isinstance(model, (SmplxBodyModel, SyntheticBodyModel)):
-        raise TypeError("fit_keypoints needs a SmplxBodyModel or a SyntheticBodyModel(skeleton='full')")
-    model.check_keypoints()
-    sel = keypoint_indices(select)
-    n = len(sel)
-    for name, t in (("target", target), ("init_pose", init_pose), ("transl", transl), ("betas", betas), ("weights", weights)):
-        if torch.is_tensor(t) and not t.is_cuda or (name in ("target", "init_pose") and not torch.is_tensor(t)):
-            raise RuntimeError(f"fit_keypoints: {name} must be a CUDA tensor -- there is no CPU fallback")
-    if transl is not None and not torch.is_tensor(transl):
-        raise RuntimeError("fit_keypoints: transl must be a CUDA tensor -- there is no CPU fallback")
-    if target.dim() != 3 or target.shape[1] != n or target.shape[2] != 3:
-        raise ValueError(f"fit_keypoints: target must be (F, {n}, 3) for the {n} selected points, got {tuple(target.shape)}")
-    F, dev = target.shape[0], target.device
-    if tuple(init_pose.shape) not in ((F, 22, 3), (F, 66)):
-        raise ValueError(f"fit_keypoints: init_pose must be ({F}, 22, 3) or ({F}, 66), got {tuple(init_pose.shape)}")
-    for name, t in (("init_pose", init_pose), ("transl", transl), ("betas", betas), ("weights", weights)):
-        if torch.is_tensor(t) and t.device != dev:
-            raise ValueError(f"fit_keypoints: {name} is on {t.device}, target on {dev}")
-    if transl is not None and tuple(transl.shape) != (F, 3):
-        raise ValueError(f"fit_keypoints: transl must be ({F}, 3), got {tuple(transl.shape)}")
-    prior_weight = float(prior_weight)
-    if not (prior_weight > 0 and np.isfinite(prior_weight)):
-        raise ValueError(f"fit_keypoints: prior_weight must be positive and finite, got {prior_weight}")
-    if int(n_iter) != n_iter or n_iter < 0:
-        raise ValueError(f"fit_keypoints: n_iter must be a non-negative integer, got {n_iter}")
-    w, w_per_frame = None, 0
-    if torch.is_tensor(weights) and weights.dim() == 2:
-        if tuple(weights.shape) != (F, n):
-            raise ValueError(f"fit_keypoints: per-frame weights must be ({F}, {n}), got {tuple(weights.shape)}")
-        w, w_per_frame = _aligned(weights), 1
-    elif weights is not None:
-        v = (weights.detach().float().cpu().numpy() if torch.is_tensor(weights) else np.asarray(weights, dtype=np.float32)).reshape(-1)
-        if v.shape[0] != n:
-            raise ValueError(f"fit_keypoints: weights must have {n} values (one per selected point), got {v.shape[0]}")
-        if not (v >= 0).all():
-            raise ValueError("fit_keypoints: weights must be non-negative")
-        w = torch.from_numpy(np.ascontiguousarray(v)).to(dev)
-    pack = model.keypoint_pack(dev)
+    a = _fit_args("fit_keypoints", target, model, init_pose, transl, weights, prior_weight, n_iter, select, betas=betas)
+    sel, n, F, dev, pack = a["sel"], a["n"], a["F"], a["dev"], a["pack"]
+    w, w_per_frame, y, pose0, tr, prior_weight = a["w"], a["w_per_frame"], a["y"], a["pose0"], a["tr"], a["prior_weight"]
     B = pack.n_betas
     per_frame, b = 0, None
     if torch.is_tensor(betas) and betas.dim() == 2:
@@ -417,12 +437,7 @@ def fit_keypoints(target, model, init_pose, betas=None, transl=None, select="coc
         b = _aligned(torch.nn.functional.pad(betas.detach().float(), (0, B - betas.shape[1])))
         per_frame = 1
     elif betas is not None:
-        v = (betas.detach().float().cpu().numpy() if torch.is_tensor(betas) else np.asarray(betas, dtype=np.float32)).reshape(-1)
-        if v.shape[0] > min(SMPLX_NUM_BETAS, B):
-            raise ValueError(f"fit_keypoints: at most {min(SMPLX_NUM_BETAS, B)} betas, got {v.shape[0]}")
-        b = torch.from_numpy(np.pad(v, (0, B - v.shape[0]))).to(dev)
-    y, pose0 = _aligned(target), _aligned(init_pose.reshape(F, 22, 3))
-    tr = None if transl is None else _aligned(transl)
+        b = _betas_vector("fit_keypoints", betas, B, dev)
     poses = torch.empty((F, 22, 3), dtype=torch.float32, device=dev)
     transl_out = torch.empty((F, 3), dtype=torch.float32, device=dev)
     cost = torch.empty((F, 2), dtype=torch.float32, device=dev)
@@ -432,6 +447,79 @@ def fit_keypoints(target, model, init_pose, betas=None, transl=None, select="coc
                                           L.ptr(tr), int(bool(fit_transl)), sel_c, n, prior_weight, int(n_iter), F,
                                           L.ptr(poses), L.ptr(transl_out), L.ptr(cost), L.stream_ptr(dev)))
     return {"poses": poses, "transl": transl_out, "cost_init": cost[:, 0], "cost": cost[:, 1]}
+
+
+# Weight of |beta|^2 in fit_keypoints_shape.  Betas are whitened PCA coefficients (unit variance over the population), so
+# this is a Gaussian prior on the shape.  At 1e-3 a shape 1 sigma from the mean costs as much as a 3 cm miss of one point
+# in one frame (as FIT_PRIOR_WEIGHT does for 1 rad of pose): over a clip of hundreds of frames the data decides the shape,
+# and on a clip of a few frames the prior still keeps directions the keypoints do not see near the mean.
+FIT_SHAPE_PRIOR_WEIGHT = 1e-3
+
+
+def fit_keypoints_shape(target, model, init_pose, lengths=None, betas=None, transl=None, select="coco", weights=None,
+                        prior_weight=FIT_PRIOR_WEIGHT, shape_prior_weight=FIT_SHAPE_PRIOR_WEIGHT, n_iter=10,
+                        fit_transl=True):
+    """One body shape per sequence and a pose per frame whose ``keypoints`` hit ``target``: per sequence s,
+    ``n_iter`` Levenberg-Marquardt steps (``tik_fit_keypoints_shape``) on
+
+        E_s = sum_{f in s} [ sum_k w_k |keypoints(pose_f, model, beta_s, transl_f)[k] - target_f[k]|^2
+                             + prior_weight |pose_f - init_pose_f|^2 ] + shape_prior_weight |beta_s|^2
+
+    over beta_s (the model's shape coefficients, 10 for both model kinds), the rotations of joints 0..21 of every frame and,
+    with ``fit_transl``, the translations.  target, model, init_pose, transl, select, weights, prior_weight, n_iter: as
+    ``fit_keypoints`` (frames of every sequence packed back to back); lengths: host ints, the frame count of each sequence
+    (sum = F), None for one sequence; betas: the start of the shape -- None (the mean shape, 0), one vector for every
+    sequence or a CUDA tensor (S, <= 10); shape_prior_weight > 0, the weight of the prior centred on the mean shape.  E_s
+    never increases; a sequence whose initial E_s is not finite comes back unchanged with cost NaN.  A sequence's results
+    do not depend on the other sequences of the call.
+    Returns {"poses": (F, 22, 3), "transl": (F, 3), "betas": (S, B), "cost_init": (S,), "cost": (S,)}, fp32 CUDA
+    tensors."""
+    from .inference import sequence_tables
+    a = _fit_args("fit_keypoints_shape", target, model, init_pose, transl, weights, prior_weight, n_iter, select,
+                  betas=betas)
+    sel, n, F, dev, pack = a["sel"], a["n"], a["F"], a["dev"], a["pack"]
+    B = pack.n_betas
+    shape_prior_weight = float(shape_prior_weight)
+    if not (shape_prior_weight > 0 and np.isfinite(shape_prior_weight)):
+        raise ValueError(f"fit_keypoints_shape: shape_prior_weight must be positive and finite, got {shape_prior_weight}")
+    if lengths is None:
+        lengths = [F] if F > 0 else []
+    lengths = [int(k) for k in lengths]
+    if F == 0 and not lengths:
+        fs = np.zeros(1, dtype=np.int64)
+    else:
+        fs = sequence_tables(lengths, 1, -1, 1)[0]
+    S = len(lengths)
+    if int(fs[-1]) != F:
+        raise ValueError(f"fit_keypoints_shape: lengths sum to {int(fs[-1])}, target has {F} frames")
+    if torch.is_tensor(betas) and betas.dim() == 2:
+        if betas.shape[0] != S or betas.shape[1] > min(SMPLX_NUM_BETAS, B):
+            raise ValueError(f"fit_keypoints_shape: per-sequence betas must be ({S}, <= {min(SMPLX_NUM_BETAS, B)}), "
+                             f"got {tuple(betas.shape)}")
+        b = _aligned(torch.nn.functional.pad(betas.detach().float(), (0, B - betas.shape[1])))
+    elif betas is not None:
+        b = _betas_vector("fit_keypoints_shape", betas, B, dev).expand(S, B).contiguous()
+    else:
+        b = None
+    poses = torch.empty((F, 22, 3), dtype=torch.float32, device=dev)
+    transl_out = torch.empty((F, 3), dtype=torch.float32, device=dev)
+    betas_out = torch.empty((S, B), dtype=torch.float32, device=dev)
+    cost = torch.empty((S, 2), dtype=torch.float32, device=dev)
+    if F == 0:
+        return {"poses": poses, "transl": transl_out, "betas": betas_out, "cost_init": cost[:, 0], "cost": cost[:, 1]}
+    frame_start = torch.from_numpy(fs).to(dev)
+    sel_c = (C.c_int32 * n)(*sel)
+    nbytes = C.c_int64()
+    L.check(L.lib().tik_fit_keypoints_shape_workspace_bytes(C.byref(pack.c), n, int(bool(fit_transl)), F, S,
+                                                             C.byref(nbytes)))
+    ws = torch.empty(max(1, nbytes.value), dtype=torch.uint8, device=dev)
+    with L.on_device(dev):
+        L.check(L.lib().tik_fit_keypoints_shape(
+            C.byref(pack.c), L.ptr(a["y"]), L.ptr(a["w"]), a["w_per_frame"], L.ptr(a["pose0"]), L.ptr(a["tr"]),
+            int(bool(fit_transl)), L.ptr(frame_start), S, L.ptr(b), shape_prior_weight, sel_c, n, a["prior_weight"],
+            int(n_iter), F, L.ptr(ws), nbytes.value, L.ptr(poses), L.ptr(transl_out), L.ptr(betas_out), L.ptr(cost),
+            L.stream_ptr(dev)))
+    return {"poses": poses, "transl": transl_out, "betas": betas_out, "cost_init": cost[:, 0], "cost": cost[:, 1]}
 
 
 def run_smpl_keypoints(data, smplx_models, device, apply_trans=True, apply_root_rot=True, apply_shape=True):
